@@ -9,9 +9,15 @@ BASELINE.json's metric has two halves, both measured here on that configuration:
 The default line also carries the other half as a first-class block (`demos`, with its own roofline, cpu_baseline and
 e2e).  See DESIGN.md "Measurement".
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--metric steps|demos]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--metric steps|demos] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  For N>1 launch with torch.distributed.run.
+
+--dump-outputs DIR writes what the last timed step returned, as DIR/<name>.npy in float32: the step's (slab, flags, nnz)
+(--metric steps) or the generator's (tape, slab, flags) (--metric demos).  The inputs are seeded, so the same arguments
+give the same arrays on every run and two builds can be compared file by file.  Arrays larger than the dump budget keep
+the games of one fixed, seeded sample, the same games in every array.  At N > 1 rank 0 writes its shard, which holds the
+same games as a one-GPU run.
 """
 from __future__ import annotations
 
@@ -33,6 +39,8 @@ FALLBACK_HBM_GBS = 6650.0  # B200_PROFILING.md fallback
 VALUES5, PROBS5 = (-2, -1, 0, 1, 2), (0.05, 0.10, 0.70, 0.10, 0.05)  # P(0) = 0.7 as in the reference (datasets.py:31)
 VALUES3, PROBS3 = (-1, 0, 1), (0.15, 0.7, 0.15)                      # the reference's defaults (datasets.py:30-31)
 REF_DIR = ROOT / "baseline" / "_ref"  # verbatim copy of the reference's scripts (scripts/install_ref.sh), if installed
+DUMP_BYTES = 60_000_000  # --dump-outputs budget: under 64 MB with the .npy headers
+DUMP_NAMES = ("slab", "flags", "nnz", "tape")  # the files --dump-outputs writes: steps (slab, flags, nnz), demos (tape, slab, flags)
 
 
 def demo_bytes(S: int, R: int) -> int:
@@ -54,7 +62,14 @@ def parse() -> argparse.Namespace:
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--ctas-per-sm", type=int, default=0, help="tuning sweep only (TG_TUNING=1 build)")
     ap.add_argument("--variant", type=int, default=0, help="tuning sweep only (TG_TUNING=1 build)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", type=Path, default=None, metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times CPU code)")
+    return args
 
 
 def workload_config(metric: str, S: int, B: int, shift: int, world: int) -> dict:
@@ -135,6 +150,37 @@ def _time_ms(fn, iters: int, torch) -> float:
     e1.record()
     torch.cuda.synchronize()
     return e0.elapsed_time(e1) / iters
+
+
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+def sample_outputs(outputs: dict, B: int) -> dict:
+    """Host float32 copies of device outputs, each given as (tensor, dimension indexing the B games).  Over the
+    DUMP_BYTES budget every array keeps the same fixed, seeded, sorted sample of games."""
+    import numpy as np
+    import torch
+
+    per_game = sum(t.numel() // B for t, _ in outputs.values()) * 4
+    n = min(B, DUMP_BYTES // per_game)
+    idx = None if n == B else torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, n, replace=False)))
+    host = {}
+    for name, (t, dim) in outputs.items():
+        if idx is not None:
+            t = t.index_select(dim, idx.to(t.device))
+        host[name] = t.cpu().numpy().astype(np.float32)
+    return host
+
+
+def write_outputs(out_dir: Path, host: dict) -> None:
+    """DIR/<name>.npy for every array; a file another run left under one of the names either metric writes is removed
+    first, so that DIR holds exactly this run's outputs."""
+    import numpy as np
+
+    assert set(host) <= set(DUMP_NAMES), sorted(host)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name in DUMP_NAMES:
+        (out_dir / f"{name}.npy").unlink(missing_ok=True)
+    for name, a in host.items():
+        np.save(out_dir / f"{name}.npy", a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU legs
@@ -332,9 +378,10 @@ def max_over_ranks(x: float, torch, dist, dev, world: int) -> float:
 
 # ------------------------------------------------------------------------------------------------ demos block
 def measure_demos(env, torch, dist, dev, S, B, R, values, probs, shift, world, rank, local, barrier, K, with_e2e, with_cpu,
-                  tape=None, slab=None) -> dict:
+                  tape=None, slab=None, dump=False) -> dict:
     """Synthetic demos/s (the other half of BASELINE.json's metric) as a first-class measurement: device-timed value,
-    roofline of the generator kernel, end to end into pinned host memory (tg_demo_gen_host), CPU baselines."""
+    roofline of the generator kernel, end to end into pinned host memory (tg_demo_gen_host), CPU baselines.  With
+    `dump`, out["outputs"] holds host copies of the last timed launch's (tape, slab, flags)."""
     lay = env.layout(S)
     peak, peak_kind = hbm_peak()
     if tape is None:
@@ -352,6 +399,7 @@ def measure_demos(env, torch, dist, dev, S, B, R, values, probs, shift, world, r
         _, _, dflags = gen(i)
     e1.record()
     barrier()
+    outputs = sample_outputs({"tape": (tape, 1), "slab": (slab, 0), "flags": (dflags, 0)}, B) if dump else None
     ms = max_over_ranks(e0.elapsed_time(e1) / K, torch, dist, dev, world)
     algo = demo_bytes(S, R)
     achieved = B * algo / (ms * 1e-3) / 1e9
@@ -391,6 +439,8 @@ def measure_demos(env, torch, dist, dev, S, B, R, values, probs, shift, world, r
         real = cpu_demo_reference(S, R, shift, values, probs, 4.0)
         if real is not None:
             out["cpu_reference"] = {"value": real[0], "unit": "demos/s", "cores": real[1], "kind": "reference", "sample": real[2]}
+    if dump:
+        out["outputs"] = outputs
     return out
 
 
@@ -634,9 +684,12 @@ def main() -> None:
         torch.cuda.synchronize()
 
     peak, peak_kind = hbm_peak()
+    dump = args.dump_outputs is not None and rank == 0
     if args.metric == "demos":
         blk = measure_demos(env, torch, dist, dev, S, B, R, VALUES5, PROBS5, shift, world, rank, local, barrier, K,
-                            not args.no_e2e, not args.no_cpu)
+                            not args.no_e2e, not args.no_cpu, dump=dump)
+        if dump:
+            write_outputs(args.dump_outputs, blk.pop("outputs"))
         if rank == 0:
             line = {"metric": blk["metric"], "value": blk["value"], "unit": blk["unit"], "n_gpus": world, "steps": K, "warmup": 3,
                     "ms_per_step": blk["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -658,9 +711,9 @@ def main() -> None:
     flags = torch.empty(B, dtype=torch.uint8, device=dev)
     nnz = torch.empty(B, dtype=torch.int32, device=dev)
 
-    def one_step(i: int) -> None:
+    def one_step(i: int):
         src, dst = (slab_a, slab_b) if i % 2 == 0 else (slab_b, slab_a)
-        env.step_batch(src, tape3[(R - 1 - i) % R], S, shift, out=dst, flags=flags, nnz=nnz)
+        return env.step_batch(src, tape3[(R - 1 - i) % R], S, shift, out=dst, flags=flags, nnz=nnz)
 
     for i in range(W):
         one_step(i)
@@ -672,10 +725,12 @@ def main() -> None:
     barrier()
     ev0.record()
     for i in range(K):
-        one_step(W + i)
+        last = one_step(W + i)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
+    # copied before the loads below overwrite the buffers
+    outputs = sample_outputs({"slab": (last[0], 0), "flags": (last[1], 0), "nnz": (last[2], 0)}, B) if dump else None
     # keep the clock sampler under the same load for ~1 s (its period is 200 ms); results are discarded
     t_end = time.perf_counter() + max(0.0, 1.0 - ms / 1e3)
     i = 0
@@ -790,6 +845,8 @@ def main() -> None:
             real = cpu_step_reference(S, 5.0)
             if real is not None:
                 line["cpu_reference"] = {"value": real[0], "unit": "steps/s", "cores": real[1], "kind": "reference", "sample": real[2]}
+        if dump:
+            write_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
