@@ -26,14 +26,19 @@
  *     throws.  There is no CPU fallback: without a CUDA device every compute
  *     entry point returns TG_E_CUDA.
  *
- * Device formats (S = dim_3d in {4, 9, 16}; see DESIGN.md "Data layout")
+ * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
+ * K1-K4, K6-K8, parity mode, host buffers).  The change of basis (K5) stays
+ * {4, 9, 16} and tg_demo_accumulate_tc 16; at 25 tg_demo_gen_philox keeps
+ * contract v1 for every alphabet (tg_demo_alias_tables returns TG_E_ARG).
+ *
+ * Device formats (see DESIGN.md "Data layout")
  *   slab   int8  [B][GP]   residual tensors, entry (i,j,k) at i*RP + j*S + k,
  *                          RP = roundup4(S*S), GP = roundup16(S*RP); padding
  *                          bytes are zero.  (S=4: 16/64, S=9: 84/768,
- *                          S=16: 256/4096.)  Values must stay in [-64, 63]
+ *                          S=16: 256/4096, S=25: 628/15712.)  Values must stay in [-64, 63]
  *                          for the next step to be guaranteed (TG_FLAG_RANGE).
  *   tape   uint8 [B][TP]   action tokens cat(u,v,w)+shift in bytes [0,3S),
- *                          TP = roundup16(3S) (16/32/48), padding zero.
+ *                          TP = roundup16(3S) (16/32/48/80), padding zero.
  *                          Token bound: every token is <= 2*shift (|coefficient|
  *                          <= shift <= 4) for the shift handed to the same call;
  *                          tg_step, tg_rollout, tg_replay and tg_expand_children
@@ -159,7 +164,7 @@ int tg_demo_gen_philox(uint64_t seed, uint64_t first_demo, int64_t N, int R, int
                        int8_t *slab, uint8_t *flags, void *stream);
 /* HOST function: the alias tables of contract v2 as uint16 [8][128] -- [0] the plain distribution of a group of three
  * entries, [1] of a single entry, [2 + g] the tilted table of group g; bucket = 9-bit threshold | alias outcome << 9.
- * TG_E_ARG where v2 does not apply. */
+ * TG_E_ARG where v2 does not apply (also at S = 25: nine groups per factor, the tables hold six). */
 int tg_demo_alias_tables(const int8_t *values, const double *probs, int n_values, int S, uint16_t *tables_host);
 /* slab[n] = sum_r rank1(tape[r][n]) -- the target tensor of a given action
  * list (utils.py:40-53 uvw_to_demo, utils.py:232, datasets.py:141). */
@@ -234,7 +239,7 @@ int tg_slice_rank(const int8_t *slab, int32_t *ranks, int64_t B, int S, void *st
  * which is how tg_expand_children keys a child without a pass over it.  (TG_VERSION 200 changed the constants.) */
 int tg_state_key(const int8_t *slab, uint64_t *keys, int64_t B, int S, void *stream);
 
-/* ---- K5: change-of-basis augmentation ------------------------------------- */
+/* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,
  * "Change of basis"): T'[i][j][k] = sum_abc A[i][a] B[j][b] C[k][c] T[a][b][c].
  * mats: int8 [N or 1][3][S][S] = (A, B, C) row-major, one triple per game

@@ -55,7 +55,7 @@ __device__ __forceinline__ void split_index(long long id, int R, long long &demo
 // once (the step-major tape puts each record of a demo in a different DRAM page; read one after the other inside the
 // replay loop they serialise into R - a round trips per sample, which is what bounded this kernel).
 template <int S, bool PACK16, bool STAGE>
-__global__ void __launch_bounds__(128, PACK16 ? (S == 16 ? 6 : 8) : 1)
+__global__ void __launch_bounds__(128, PACK16 ? (S == 16 ? 6 : (S == 25 ? 3 : 8)) : 1)
     demo_sample_kernel(const uint8_t *__restrict__ tape, long long tape_step_stride,
                                    const int8_t *__restrict__ slab, long long N, int R, int dim_t, int replay_shift,
                                    const long long *__restrict__ idx, long long nb, float *__restrict__ states,
@@ -137,12 +137,11 @@ __global__ void __launch_bounds__(128, PACK16 ? (S == 16 ? 6 : 8) : 1)
                 const int w0 = rec[L.off_w[0]], w1 = rec[L.off_w[1]], w2 = rec[L.off_w[2]], w3 = rec[L.off_w[3]];
                 const int np0 = (inA0 ? nvA : nvB) * w0 + ((inA1 ? nvA : nvB) * w1) * 65536;
                 const int np1 = (inA2 ? nvA : nvB) * w2 + ((inA3 ? nvA : nvB) * w3) * 65536;
-                uint32_t uq[4];
+                uint32_t uq[UW<S>];
                 if constexpr (S <= 4) {
                     uq[0] = *reinterpret_cast<const uint32_t *>(rec);
                 } else {
-                    const uint4 q4 = *reinterpret_cast<const uint4 *>(rec);
-                    uq[0] = q4.x, uq[1] = q4.y, uq[2] = q4.z, uq[3] = q4.w;
+                    load_u<S>(reinterpret_cast<const uint8_t *>(rec), uq);
                 }
 #pragma unroll
                 for (int i = 0; i < S; i++) {
@@ -467,6 +466,152 @@ __global__ void __launch_bounds__(SampleCfg<S>::NT)
     } else {
         for (size_t e = tid; e < bytes / 4; e += NT) dst[e] = s_tile[e];
     }
+}
+
+// ------------------------------------------------------------------ K4 at 25x25x25, demo-major store
+// One 25x25x25 state slot is 62.5 KB of float32, so the shared-memory image of whole samples that demo_sample_dm_kernel
+// builds does not fit from dim_t = 4 on.  Here a CTA serves one sample: its records a .. R-1 (one contiguous run of the
+// demo-major store) arrive with one bulk copy, thread c (one of the 157 word columns) keeps the four entries
+// (i, 4c .. 4c+3) of every row of the head in registers -- exact int32 entries, or two 16-bit lanes per register under the
+// same bound as above -- and every state slot leaves straight from the registers with the widest stores each address
+// allows (store_run), so states may start at any float.
+template <bool TGT16, bool PACK16>
+__global__ void __launch_bounds__(160, PACK16 ? 3 : 1)
+    demo_sample_dm25_kernel(const uint8_t *__restrict__ tape_dm, const uint8_t *__restrict__ targets, long long N, int R, int dim_t,
+                            int replay_shift, const long long *__restrict__ idx, float *__restrict__ states,
+                            float *__restrict__ scalars, long long *__restrict__ actions, float *__restrict__ rewards) {
+    constexpr int S = 25;
+    using G = Geo<S>;
+    extern __shared__ __align__(16) uint8_t s_rec[]; // [R][TP]: record a raw, records a+1 .. R-1 as int8 coefficients
+    __shared__ uint64_t s_bar;
+    const int tid = threadIdx.x;
+    const long long b = blockIdx.x;
+    long long demo = -1;
+    int a = 0;
+    const long long id = idx[b];
+    if (id >= 0) split_index(id, R, demo, a);
+    const bool worker = tid < G::WR;
+    Lane<S> L;
+    L.init(worker ? tid : 0);
+    const int nv = min(4, G::S2 - 4 * L.c);
+    float *st = states + b * (long long)dim_t * G::S3;
+    if (demo < 0 || demo >= N) { // bad index: zero states, nothing else written
+        if (worker)
+            for (int s = 0; s < dim_t; s++)
+#pragma unroll
+                for (int i = 0; i < S; i++) store_run<S>(st + (size_t)s * G::S3 + i * G::S2 + 4 * L.c, nv, 0.f, 0.f, 0.f, 0.f);
+        return;
+    }
+    if (tid == 0) {
+        mbar_init(&s_bar, 1);
+        mbar_fence_init();
+    }
+    __syncthreads();
+    if (tid == 0) {
+        const uint32_t rb = (uint32_t)(R - a) * G::TP;
+        mbar_expect_tx(&s_bar, rb);
+        bulk_g2s(s_rec + (size_t)a * G::TP, tape_dm + ((size_t)demo * R + a) * G::TP, rb, &s_bar);
+    }
+    // the target words of this word column are in flight while the records land
+    int acc[S][PACK16 ? 2 : 4];
+    if (worker) {
+#pragma unroll
+        for (int i = 0; i < S; i++) {
+            int e[4];
+            if constexpr (TGT16) {
+                const uint2 p = __ldg(reinterpret_cast<const uint2 *>(targets + ((size_t)demo * G::GP + i * G::RP + 4 * L.c) * 2));
+                e[0] = (int)(short)(p.x & 0xFFFFu), e[1] = (int)p.x >> 16, e[2] = (int)(short)(p.y & 0xFFFFu), e[3] = (int)p.y >> 16;
+            } else {
+                const uint32_t w = __ldg(reinterpret_cast<const uint32_t *>(targets + (size_t)demo * G::GP + i * G::RP + 4 * L.c));
+                e[0] = sext_byte<0>(w), e[1] = sext_byte<1>(w), e[2] = sext_byte<2>(w), e[3] = sext_byte<3>(w);
+            }
+            if constexpr (PACK16) {
+                acc[i][0] = e[0] + e[1] * 65536, acc[i][1] = e[2] + e[3] * 65536;
+            } else {
+                acc[i][0] = e[0], acc[i][1] = e[1], acc[i][2] = e[2], acc[i][3] = e[3];
+            }
+        }
+    }
+    mbar_wait(&s_bar, 0);
+    {   // records that are only replayed become int8 coefficients in place (no borrow between bytes: token | 0x80 > shift)
+        const uint32_t sh4 = (uint32_t)replay_shift * ONES4;
+        uint32_t *rw = reinterpret_cast<uint32_t *>(s_rec + (size_t)(a + 1) * G::TP);
+        for (int w = tid; w < (R - a - 1) * (G::TP / 4); w += 160) rw[w] = ((rw[w] | H4) - sh4) ^ H4;
+    }
+    __syncthreads();
+    if (!worker) return;
+    // entries outside the row (last word column) take v_B; they are never stored, and a 16-bit lane never reads the one above it
+    const bool inA[4] = {(L.maskA & 0x1u) != 0, (L.maskA & 0x100u) != 0, (L.maskA & 0x10000u) != 0, (L.maskA & 0x1000000u) != 0};
+    const int8_t *rec0 = reinterpret_cast<const int8_t *>(s_rec);
+#pragma unroll 2
+    for (int j = a + 1; j < R; j++) {
+        const int8_t *rec = rec0 + (size_t)j * G::TP;
+        const int nvA = -(int)rec[L.off_vA], nvB = -(int)rec[L.off_vB];
+        int p[4];
+#pragma unroll
+        for (int q = 0; q < 4; q++) p[q] = (inA[q] ? nvA : nvB) * (int)rec[L.off_w[q]];
+        uint32_t uq[UW<S>];
+        load_u<S>(reinterpret_cast<const uint8_t *>(rec), uq);
+        const int np0 = p[0] + p[1] * 65536, np1 = p[2] + p[3] * 65536;
+#pragma unroll
+        for (int i = 0; i < S; i++) {
+            int u;
+            switch (i & 3) {
+            case 0: u = sext_byte<0>(uq[i >> 2]); break;
+            case 1: u = sext_byte<1>(uq[i >> 2]); break;
+            case 2: u = sext_byte<2>(uq[i >> 2]); break;
+            default: u = sext_byte<3>(uq[i >> 2]); break;
+            }
+            if constexpr (PACK16) {
+                acc[i][0] += u * np0, acc[i][1] += u * np1;
+            } else {
+                acc[i][0] += u * p[0], acc[i][1] += u * p[1], acc[i][2] += u * p[2], acc[i][3] += u * p[3];
+            }
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < S; i++) {
+        float f[4];
+        if constexpr (PACK16) {
+#pragma unroll
+            for (int h = 0; h < 2; h++) {
+                const int x = acc[i][h];
+                const int lo = (int)(short)(x & 0xFFFF);
+                f[2 * h] = (float)lo, f[2 * h + 1] = (float)((x - lo) >> 16);
+            }
+        } else {
+#pragma unroll
+            for (int q = 0; q < 4; q++) f[q] = (float)acc[i][q];
+        }
+        store_run<S>(st + i * G::S2 + 4 * L.c, nv, f[0], f[1], f[2], f[3]);
+    }
+    // history slots: rank-1 tensors of the next actions, latest first
+    const int hi = min(a + dim_t, R);
+    for (int s = 1; s < dim_t; s++) {
+        const int j = hi - s;
+        float *ss = st + (size_t)s * G::S3;
+        if (j >= a + 1) {
+            const int8_t *hr = rec0 + (size_t)j * G::TP;
+            const int vA = (int)hr[L.off_vA], vB = (int)hr[L.off_vB];
+            float pf[4];
+#pragma unroll
+            for (int q = 0; q < 4; q++) pf[q] = (float)((inA[q] ? vA : vB) * (int)hr[L.off_w[q]]);
+#pragma unroll
+            for (int i = 0; i < S; i++) {
+                const float uf = (float)(int)hr[i];
+                store_run<S>(ss + i * G::S2 + 4 * L.c, nv, uf * pf[0], uf * pf[1], uf * pf[2], uf * pf[3]);
+            }
+        } else {
+#pragma unroll
+            for (int i = 0; i < S; i++) store_run<S>(ss + i * G::S2 + 4 * L.c, nv, 0.f, 0.f, 0.f, 0.f);
+        }
+    }
+    if (tid == 0) {
+        scalars[b] = (float)(R - a);
+        rewards[b] = -(float)(a + 1);
+    }
+    const uint8_t *ta = s_rec + (size_t)a * G::TP; // the sample's own action: raw tokens
+    for (int q = tid; q < 3 * S; q += G::WR) actions[b * 3 * S + q] = (long long)ta[q];
 }
 
 // ------------------------------------------------------------------ K4r: 9x9x9, one thread per (sample, row i)
@@ -1004,6 +1149,15 @@ __global__ void __launch_bounds__(256) state_key_kernel(const int8_t *__restrict
                 for (int x = 0; x < G::WR; x++) k += s_ph[tid * G::WR + x];
                 keys[g0 + tid] = k;
             }
+        } else if constexpr (G::WR > 64) { // S = 25: one game per pass (157 partial sums), reduced by warp 0
+            static_assert(TG == 1, "one game per pass");
+            if (tid < 32 && g0 < B) {
+                unsigned long long k = 0;
+                for (int x = tid; x < G::WR; x += 32) k += s_ph[x];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) k += __shfl_xor_sync(0xFFFFFFFFu, k, o);
+                if (tid == 0) keys[g0] = k;
+            }
         } else { // S = 16: 64 partial sums per game, one warp per game
             static_assert(G::WR <= 32 || (G::WR == 64 && TG <= 8), "warp-per-game reduction");
             const int wp = tid >> 5, ln = tid & 31;
@@ -1025,6 +1179,7 @@ __global__ void __launch_bounds__(256) state_key_kernel(const int8_t *__restrict
     case 4: { constexpr int kS = 4; __VA_ARGS__; } break;   \
     case 9: { constexpr int kS = 9; __VA_ARGS__; } break;   \
     case 16: { constexpr int kS = 16; __VA_ARGS__; } break; \
+    case 25: { constexpr int kS = 25; __VA_ARGS__; } break; \
     default: return TG_E_ARG; \
     }
 
@@ -1180,11 +1335,37 @@ int tg_demo_sample_dm(const uint8_t *tape_dm, const void *targets, int targets_i
         TG_CUDA(cudaGetLastError());
         return TG_OK;
     }
-    TG_SWITCH_S(S, {
-        const int rc = tg::launch_demo_sample_dm<kS>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
-                                                     (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
-        if (rc != TG_OK) return rc;
-    });
+    if (S == 25) { // one CTA per sample, states straight from the registers
+        const long long smem = (long long)R * tg::Geo<25>::TP;
+        if (smem > 227 * 1024 || nb > 0x7FFFFFFFLL) return TG_E_ARG;
+#define TG_DM25(T16, P16)                                                                                                     \
+    {                                                                                                                         \
+        auto kern = tg::demo_sample_dm25_kernel<T16, P16>;                                                                    \
+        TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                          \
+        kern<<<(unsigned)nb, 160, (size_t)smem, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift, (const long long *)idx, \
+                                                     states, scalars, (long long *)actions, rewards);                         \
+    }
+        if (targets_i16) {
+            if (pack16) TG_DM25(true, true) else TG_DM25(true, false)
+        } else {
+            if (pack16) TG_DM25(false, true) else TG_DM25(false, false)
+        }
+#undef TG_DM25
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    }
+    switch (S) {
+    case 4: { const int rc = tg::launch_demo_sample_dm<4>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
+                                                          (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
+              if (rc != TG_OK) return rc; } break;
+    case 9: { const int rc = tg::launch_demo_sample_dm<9>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
+                                                          (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
+              if (rc != TG_OK) return rc; } break;
+    case 16: { const int rc = tg::launch_demo_sample_dm<16>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
+                                                            (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
+               if (rc != TG_OK) return rc; } break;
+    default: return TG_E_ARG;
+    }
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }

@@ -807,7 +807,7 @@ __global__ void __launch_bounds__(128)
 // int8 slab in; int8 slab out (out16 == 0) or int16 slab out
 static int change_of_basis_impl(const int8_t *slab_in, const int8_t *mats, int per_game, void *slab_out, int out16, uint8_t *flags,
                                 int64_t N, int S, void *stream) {
-    if (!tg::supported_S(S) || N < 0) return TG_E_ARG;
+    if (!tg::basis_supported_S(S) || N < 0) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!slab_in || !mats || !slab_out || (const void *)slab_in == (const void *)slab_out) return TG_E_ARG;
     if (((uintptr_t)slab_in | (uintptr_t)slab_out) & 15) return TG_E_ARG;
@@ -894,7 +894,7 @@ int tg_change_of_basis_i16(const int8_t *slab_in, const int8_t *mats, int per_ga
 int tg_change_of_basis_factors(const uint8_t *tape_in, int64_t in_step_stride, int shift_in, const int8_t *mats, int per_game,
                                uint8_t *tape_out, int64_t out_step_stride, int shift_out, uint8_t *flags, int64_t N, int R,
                                int S, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || shift_in < 0 || shift_out < 1 || shift_out > 127) return TG_E_ARG;
+    if (!tg::basis_supported_S(S) || N < 0 || R < 1 || shift_in < 0 || shift_out < 1 || shift_out > 127) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!tape_in || !mats || !tape_out || !flags) return TG_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
@@ -918,7 +918,7 @@ int tg_change_of_basis_factors(const uint8_t *tape_in, int64_t in_step_stride, i
 }
 
 int tg_sample_unimodular(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, int8_t *mats, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || !(p_nonzero >= 0.0) || p_nonzero > 1.0) return TG_E_ARG;
+    if (!tg::basis_supported_S(S) || N < 0 || !(p_nonzero >= 0.0) || p_nonzero > 1.0) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!mats) return TG_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;

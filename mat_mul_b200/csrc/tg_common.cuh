@@ -22,7 +22,10 @@ struct Geo {
     static constexpr bool STRADDLE = (S % 4) != 0; // a word can span two j
 };
 
-__host__ __device__ constexpr bool supported_S(int S) { return S == 4 || S == 9 || S == 16; }
+// the game path (layout, conversions, step, expansion, rollout, keys, ranks, demos, samples, host buffers)
+__host__ __device__ constexpr bool supported_S(int S) { return S == 4 || S == 9 || S == 16 || S == 25; }
+// change of basis (tg_change_of_basis*, tg_sample_unimodular): kernels specialised per size, not built for 25x25x25
+__host__ __device__ constexpr bool basis_supported_S(int S) { return S == 4 || S == 9 || S == 16; }
 
 extern int g_last_cuda_error;
 

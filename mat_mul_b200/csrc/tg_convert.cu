@@ -100,6 +100,7 @@ static inline int grid_for(long long total, int block) {
     case 4: { constexpr int kS = 4; CALL; } break;   \
     case 9: { constexpr int kS = 9; CALL; } break;   \
     case 16: { constexpr int kS = 16; CALL; } break; \
+    case 25: { constexpr int kS = 25; CALL; } break; \
     default: return TG_E_ARG;  \
     }
 

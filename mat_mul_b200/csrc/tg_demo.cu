@@ -967,7 +967,8 @@ static void vose128(const double *P, int count, uint16_t *out) {
 
 // contract v2 applies to alphabets of at most five values whose P(0) leaves a non-zero factor reachable
 static bool alias_applies(const int8_t *values, const double *probs, int n, int S) {
-    if (n < 1 || n > 5 || !supported_S(S)) return false;
+    // AliasParams has room for the tilted tables of six groups (factors of up to 18 entries): 25x25x25 keeps contract v1
+    if (n < 1 || n > 5 || !supported_S(S) || (S + 2) / 3 > 6) return false;
     double total = 0, p0 = 0;
     for (int i = 0; i < n; i++) total += probs[i];
     for (int i = 0; i < n; i++)
@@ -1109,6 +1110,105 @@ static int dispatch_demo16_mma(unsigned long long first, long long N, int R, int
     return launch_demo16_mma<NTHR, 128, 2, 4>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
 }
 
+// ---- 25x25x25.  Phase B of demo_kernel (thread j holds the S x KW packed words of its runs (i, j, .)) would need 175
+// accumulator registers here.  Instead the sampler runs alone (MMA = -1: phase A writes the tape and the EXHAUSTED flags)
+// and demo_acc_cols_kernel sums the targets from the tape: thread (demo, word column c) holds the four entries
+// (i, 4c .. 4c+3) of every row as plain int32 (100 registers, exact for any tape), the CTA stages its demo's R records in
+// shared memory first.  Stored bytes are the entries modulo 256 and TG_FLAG_RANGE marks an entry outside [-64, 63] -- the
+// contract of the packed kernels.  or_flags: OR into flags (after the sampler) instead of overwriting them.
+template <int S>
+__global__ void __launch_bounds__(160)
+    demo_acc_cols_kernel(const uint8_t *__restrict__ tape, long long tape_step_stride, long long N, int R, int shift,
+                         int8_t *__restrict__ slab, uint8_t *__restrict__ flags, int or_flags) {
+    using G = Geo<S>;
+    static_assert(G::WR <= 160, "one demo per CTA");
+    extern __shared__ __align__(16) uint8_t s_tok[]; // [R][TP]
+    __shared__ uint32_t s_bad;
+    const int tid = threadIdx.x;
+    const long long n = blockIdx.x;
+    if (tid == 0) s_bad = 0;
+    for (int w = tid; w < R * (G::TP / 16); w += 160) {
+        const int r = w / (G::TP / 16), q = w - r * (G::TP / 16);
+        reinterpret_cast<uint4 *>(s_tok)[w] = __ldg(reinterpret_cast<const uint4 *>(tape + (size_t)r * tape_step_stride + n * G::TP) + q);
+    }
+    __syncthreads();
+    if (tid < G::WR) {
+        Lane<S> L;
+        L.init(tid);
+        int acc[S][4];
+#pragma unroll
+        for (int i = 0; i < S; i++)
+#pragma unroll
+            for (int q = 0; q < 4; q++) acc[i][q] = 0;
+#pragma unroll 1
+        for (int r = 0; r < R; r++) {
+            const uint8_t *tok = s_tok + (size_t)r * G::TP;
+            const int vA = (int)tok[L.off_vA] - shift, vB = (int)tok[L.off_vB] - shift;
+            int vw[4];
+#pragma unroll
+            for (int b = 0; b < 4; b++) {
+                const bool inA = (L.maskA >> (8 * b)) & 1u, inB = (L.maskB >> (8 * b)) & 1u;
+                vw[b] = inA ? vA * ((int)tok[L.off_w[b]] - shift) : (inB ? vB * ((int)tok[L.off_w[b]] - shift) : 0);
+            }
+#pragma unroll
+            for (int i = 0; i < S; i++) {
+                const int u = (int)tok[i] - shift;
+#pragma unroll
+                for (int q = 0; q < 4; q++) acc[i][q] += u * vw[q];
+            }
+        }
+        bool bad = false;
+        uint32_t *dst = reinterpret_cast<uint32_t *>(slab + n * G::GP) + L.c;
+#pragma unroll
+        for (int i = 0; i < S; i++) {
+            uint32_t word = 0;
+#pragma unroll
+            for (int q = 0; q < 4; q++) {
+                bad |= acc[i][q] < -64 || acc[i][q] > 63;
+                word |= ((uint32_t)acc[i][q] & 0xFFu) << (8 * q);
+            }
+            dst[i * G::WR] = word;
+        }
+        if constexpr (G::GP != S * G::RP) {
+            if (L.c == 0)
+                for (int x = S * G::RP; x < G::GP; x += 4) *reinterpret_cast<uint32_t *>(slab + n * G::GP + x) = 0u;
+        }
+        if (bad) atomicOr(&s_bad, (uint32_t)TG_FLAG_RANGE);
+    }
+    __syncthreads();
+    if (flags && tid == 0) flags[n] = (uint8_t)((or_flags ? flags[n] : 0) | s_bad);
+}
+
+template <int S>
+static int launch_demo_acc_cols(const uint8_t *tape, long long stride, long long N, int R, int shift, int8_t *slab, uint8_t *flags,
+                                int or_flags, cudaStream_t st) {
+    const long long smem = (long long)R * Geo<S>::TP;
+    if (smem > 227 * 1024 || N > 0x7FFFFFFFLL) return TG_E_ARG;
+    auto kern = demo_acc_cols_kernel<S>;
+    TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(unsigned)N, 160, (size_t)smem, st>>>(tape, stride, N, R, shift, slab, flags, or_flags);
+    TG_CUDA(cudaGetLastError());
+    return TG_OK;
+}
+
+// 25x25x25 throughput mode (contract v1): the sampler alone, then the column sum from the tape
+template <int NTHR>
+static int launch_demo25(unsigned long long first, long long N, int R, int shift, const Categorical &cat, int max_tries, uint8_t *tape,
+                         long long stride, int8_t *slab, uint8_t *flags, cudaStream_t st) {
+    constexpr int NT = 128;
+    using C = DemoCfg<25, NT, 1>;
+    const int smem = C::FLAG_BYTES + 16 + 2 * NT * 4;
+    if (R > 65535 || (long long)C::TG * R >= (1LL << 16)) return TG_E_ARG;
+    const uint32_t magic = R == 1 ? 0u : (uint32_t)((0x100000000ULL + (unsigned)R - 1) / (unsigned)R);
+    const long long grid = (N + C::TG - 1) / C::TG;
+    if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
+    static const AliasDev no_alias = {};
+    demo_kernel<25, NT, 1, true, NTHR, false, -1><<<(int)grid, NT, smem, st>>>(first, N, R, magic, shift, cat, max_tries, tape, stride,
+                                                                              nullptr, flags, no_alias);
+    TG_CUDA(cudaGetLastError());
+    return launch_demo_acc_cols<25>(tape, stride, N, R, shift, slab, flags, 1, st);
+}
+
 template <bool SAMPLE, int NTHR>
 static int dispatch_demo(unsigned long long first, long long N, int R, int S, int shift, const Categorical &cat,
                          int max_tries, uint8_t *tape, long long stride, int8_t *slab, uint8_t *flags, cudaStream_t st) {
@@ -1223,6 +1323,11 @@ int tg_demo_gen_philox(uint64_t seed, uint64_t first_demo, int64_t N, int R, int
 #else
     constexpr int use_mma = 1;
 #endif
+    if (S == 25) {
+        if (n_values <= 3) return tg::launch_demo25<2>(first_demo, N, R, shift, cat, max_tries, tape, tape_step_stride, slab, flags, st);
+        if (n_values <= 5) return tg::launch_demo25<4>(first_demo, N, R, shift, cat, max_tries, tape, tape_step_stride, slab, flags, st);
+        return tg::launch_demo25<7>(first_demo, N, R, shift, cat, max_tries, tape, tape_step_stride, slab, flags, st);
+    }
     if (S == 16 && use_mma && tg::demo_acc16_mma_applies(R)) {
         if (n_values <= 3) return tg::dispatch_demo16_mma<2>(first_demo, N, R, shift, cat, max_tries, tape, tape_step_stride, slab, flags, st);
         if (n_values <= 5) return tg::dispatch_demo16_mma<4>(first_demo, N, R, shift, cat, max_tries, tape, tape_step_stride, slab, flags, st);
@@ -1258,6 +1363,7 @@ int tg_demo_accumulate(const uint8_t *tape, int64_t tape_step_stride, int64_t N,
 #else
     constexpr int use_mma = 1;
 #endif
+    if (S == 25) return tg::launch_demo_acc_cols<25>(tape, tape_step_stride, N, R, shift, slab, flags, 0, (cudaStream_t)stream);
     if (S == 16 && use_mma && tg::demo_acc16_mma_applies(R))
         return tg::launch_demo_acc16_mma(tape, tape_step_stride, N, R, shift, slab, flags, 0, (cudaStream_t)stream);
     if (S == 4 && (long long)R * shift * shift * shift <= 191 && R <= 65535 && N <= 0x7FFFFFFFLL * 128) { // one thread per demo

@@ -146,8 +146,8 @@ __global__ void __launch_bounds__(NT)
         if (active) {
             const uint8_t *tok = s_tok + ((size_t)g * k + c) * G::TP;
             const int32_t vw = pack_vw<S>(tok, L, shift);
-            const uint4 ut = *reinterpret_cast<const uint4 *>(tok);
-            const uint32_t uw[4] = {ut.x, ut.y, ut.z, ut.w};
+            uint32_t uw[UW<S>];
+            load_u<S>(tok, uw);
             const uint32_t nvw = (uint32_t)(-vw);
             uint32_t cnt = 0, rng = 0;
             int uany = 0;
@@ -330,6 +330,7 @@ extern "C" int tg_expand_children(const int8_t *parents, const uint8_t *tape, in
     }
     case 9: return tg::launch_expand<9, 128>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
     case 16: return tg::launch_expand<16, 128>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
+    case 25: return tg::launch_expand<25, 160>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st); // one parent per CTA
     }
     return TG_E_ARG;
 }

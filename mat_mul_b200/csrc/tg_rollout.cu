@@ -122,8 +122,8 @@ __global__ void __launch_bounds__(NT + 32)
             if (alive) {
                 const uint8_t *tok = tok0 + st * C::TOK_BYTES;
                 const int32_t vw = pack_vw<S>(tok, L, shift);
-                const uint4 ut = *reinterpret_cast<const uint4 *>(tok);
-                const uint32_t uw[4] = {ut.x, ut.y, ut.z, ut.w};
+                uint32_t uw[UW<S>];
+                load_u<S>(tok, uw);
                 uint32_t any = 0;
                 const uint32_t nvw = (uint32_t)(-vw);
 #pragma unroll
@@ -355,6 +355,8 @@ static int rollout_dispatch(const int8_t *slab_in, const uint8_t *tape, int64_t 
             return tg::launch_rollout<16, 256, 4>(slab_in, tape, tape_step_stride, K, slab_out, flags, nnz, steps, B, shift, freeze, st);
 #endif
         return tg::launch_rollout_rows(slab_in, tape, tape_step_stride, K, slab_out, flags, nnz, steps, B, 16, shift, freeze, st);
+    case 25: // the word-column kernel: 25 row words per thread, two games (314 of 320 compute threads) per CTA
+        return tg::launch_rollout<25, 320, 4>(slab_in, tape, tape_step_stride, K, slab_out, flags, nnz, steps, B, shift, freeze, st);
     }
     return TG_E_ARG;
 }

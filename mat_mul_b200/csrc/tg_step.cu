@@ -233,6 +233,9 @@ int tg_step(const int8_t *slab_in, const uint8_t *tape, int8_t *slab_out, uint8_
     case 4: return tg::launch_step<4, 256, 4, 2>(slab_in, tape, slab_out, flags, nnz, B, shift, 32, st);
     case 9: return tg::launch_step<9, 256, 2, 2>(slab_in, tape, slab_out, flags, nnz, B, shift, 32, st);
     case 16: return tg::launch_step<16, 256, 1, 2>(slab_in, tape, slab_out, flags, nnz, B, shift, 32, st);
+    // 25x25x25: 157 word columns per game, so five compute warps hold one game with three threads idle (256 would leave 99);
+    // shared memory (two 15.8 KB stages) allows seven such CTAs per SM
+    case 25: return tg::launch_step<25, 160, 1, 2>(slab_in, tape, slab_out, flags, nnz, B, shift, 32, st);
     }
     return TG_E_ARG;
 }

@@ -91,14 +91,36 @@ __device__ __forceinline__ bool tokens_out_of_range(const uint8_t *tok, const La
     return ((((x & 0x7F7F7F7Fu) + (uint32_t)(0x7F - 2 * shift) * ONES4) | x) & H4) != 0;
 }
 
+// The u tokens of a record (bytes 0 .. S-1) as UW<S> words: one 16-byte shared-memory load per 16 tokens (records are
+// 16-byte aligned and TP >= 16 * ceil(S / 16) bytes long); words beyond byte S - 1 hold v tokens and are never indexed.
+template <int S>
+constexpr int UW = 4 * ((S + 15) / 16);
+template <int S>
+__device__ __forceinline__ void load_u(const uint8_t *tok, uint32_t (&uw)[UW<S>]) {
+    static_assert(UW<S> * 4 <= Geo<S>::TP, "u words inside the token record");
+#pragma unroll
+    for (int q = 0; q < UW<S> / 4; q++) {
+        const uint4 ut = reinterpret_cast<const uint4 *>(tok)[q];
+        uw[4 * q] = ut.x, uw[4 * q + 1] = ut.y, uw[4 * q + 2] = ut.z, uw[4 * q + 3] = ut.w;
+    }
+}
+
 // coefficient u_i = token_i - shift from the packed u tokens: one dp4a against a one-hot byte vector
-__device__ __forceinline__ int coef_u(const uint32_t uw[4], int i, int shift) {
+__device__ __forceinline__ int coef_u(const uint32_t *uw, int i, int shift) {
     return (int)__dp4a(uw[i >> 2], 1u << (8 * (i & 3)), (uint32_t)(-shift));
 }
 
 // Partial result word of one thread for one game; summing it over the WR
 // threads of a game gives nnz (bits 0-15), #threads whose update was non-zero
 // (bits 16-23) and #threads that saw an entry outside [-64,63] (bits 24-31).
+// The fields cannot carry into each other while S^3 < 2^16 and WR < 2^8 (25x25x25: 15625 entries, 157 threads).
+template <int S>
+struct PartialFits {
+    static constexpr bool value = Geo<S>::S3 < (1 << 16) && Geo<S>::WR < (1 << 8);
+};
+static_assert(PartialFits<4>::value && PartialFits<9>::value && PartialFits<16>::value && PartialFits<25>::value,
+              "partial result word fields");
+static_assert(Geo<25>::WR >= Geo<25>::TP / 4, "25x25x25: the threads of a game cover its token record");
 __device__ __forceinline__ uint32_t make_partial(uint32_t nnz, bool changed, bool range) {
     return nnz | (changed ? 1u << 16 : 0u) | (range ? 1u << 24 : 0u);
 }
@@ -113,8 +135,8 @@ template <int S, int SIGN>
 __device__ __forceinline__ uint32_t rank1_update(uint8_t *game, const uint8_t *tok, const Lane<S> &L, int shift) {
     using G = Geo<S>;
     const int32_t vw = pack_vw<S>(tok, L, shift);
-    const uint4 ut = *reinterpret_cast<const uint4 *>(tok); // u tokens (first min(S,16) bytes)
-    const uint32_t uw[4] = {ut.x, ut.y, ut.z, ut.w};
+    uint32_t uw[UW<S>];
+    load_u<S>(tok, uw);
     uint32_t cnt = 0, rng = 0;
     int uany = 0;
     uint32_t *col = reinterpret_cast<uint32_t *>(game) + L.c;

@@ -121,6 +121,7 @@ __global__ void pack_f32_i16_kernel(const float *__restrict__ src, long long src
     case 4: { constexpr int kS = 4; __VA_ARGS__; } break;   \
     case 9: { constexpr int kS = 9; __VA_ARGS__; } break;   \
     case 16: { constexpr int kS = 16; __VA_ARGS__; } break; \
+    case 25: { constexpr int kS = 25; __VA_ARGS__; } break; \
     default: return TG_E_ARG;                               \
     }
 

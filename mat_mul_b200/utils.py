@@ -5,7 +5,7 @@ path -- inputs living on the CPU are moved to the CUDA device, processed there
 and the result is returned on the caller's device, as the reference would.
 
 Star-import surface (the reference has no __all__): torch, Categorical, List,
-Tuple and every function below.  Sizes: dim_3d in {4, 9, 16}; factor
+Tuple and every function below.  Sizes: dim_3d in {4, 9, 16, 25}; factor
 coefficients in [-4, 4] (the game's alphabet is {-2..2}).
 """
 from typing import List, Tuple  # noqa: F401  (part of the reference's star-import surface)
