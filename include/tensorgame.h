@@ -170,8 +170,8 @@ int tg_demo_alias_tables(const int8_t *values, const double *probs, int n_values
  * list (utils.py:40-53 uvw_to_demo, utils.py:232, datasets.py:141). */
 int tg_demo_accumulate(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift, int8_t *slab,
                        uint8_t *flags, void *stream);
-/* the same sum into an int16 slab [N][GP] of int16 (plain int32 arithmetic per entry: exact for every tape and any
- * shift in [0,127]; TG_FLAG_RANGE = an entry does not fit int16).  The reference accumulates targets in float32
+/* the same sum into an int16 slab [N][GP] of int16 (exact for every tape and any shift in [0,127]: int32 arithmetic per
+ * entry while R * max(shift, 255 - shift)^3 fits int32, 64-bit beyond; TG_FLAG_RANGE = an entry does not fit int16).  The reference accumulates targets in float32
  * without limit (utils.py:218-232); this is where targets beyond the int8 slab's zone go. */
 int tg_demo_accumulate_i16(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift, int16_t *slab16,
                            uint8_t *flags, void *stream);
@@ -225,8 +225,9 @@ int tg_tape_to_demo_major(const uint8_t *tape, int64_t tape_step_stride, uint8_t
 
 /* ---- K6: rank reward ------------------------------------------------------ */
 /* ranks[b] = sum_i rank(T_b[i,:,:]) -- get_rank (utils.py:134-140), the
- * terminal reward -get_rank of act.py:59,214.  Exact rank over GF(2^31-1)
- * instead of the reference's float32 SVD. */
+ * terminal reward -get_rank of act.py:59,214.  Exact rank over Q for every
+ * int8 slab (over GF(2^31-1), and over further 31-bit primes where a slice's
+ * Hadamard bound exceeds the first) instead of the reference's float32 SVD. */
 int tg_slice_rank(const int8_t *slab, int32_t *ranks, int64_t B, int S, void *stream);
 
 /* ---- K7: state keys ------------------------------------------------------- */
@@ -245,7 +246,8 @@ int tg_state_key(const int8_t *slab, uint64_t *keys, int64_t B, int S, void *str
  * mats: int8 [N or 1][3][S][S] = (A, B, C) row-major, one triple per game
  * (per_game != 0) or one shared triple.  slab_out must differ from slab_in.
  * flags (may be NULL): TG_FLAG_RANGE if an entry of T' left [-64,63] (the
- * int8 slab's guaranteed zone; intermediates are int32 and exact). */
+ * int8 slab's guaranteed zone; the test is on the exact value, which for int8
+ * input and int8 matrices can reach 2^40; the stored byte is its low byte). */
 int tg_change_of_basis(const int8_t *slab_in, const int8_t *mats, int per_game, int8_t *slab_out, uint8_t *flags, int64_t N,
                        int S, void *stream);
 /* The same contraction with the result as an int16 slab [N][GP] of int16 (entry (i,j,k) at element i*RP + j*S + k) --

@@ -1018,40 +1018,24 @@ __global__ void tape_to_demo_major_kernel(const uint4 *__restrict__ src, long lo
 }
 
 // ------------------------------------------------------------------ K6
-// get_rank (utils.py:134-140): sum over the S slices T[i,:,:] of the matrix
-// rank.  The reference takes a float32 SVD; here the rank is computed exactly
-// over GF(p), p = 2^31-1, by fraction-free elimination (row <- row*piv -
-// row[c]*pivrow), one matrix per group of S lanes, lane = matrix row.  rank_p
-// <= rank_Q with equality unless p divides a pivot minor (probability ~S/p per
-// matrix); the small integer matrices of the game are far from that.
-__device__ __forceinline__ uint32_t mulmod31(uint32_t a, uint32_t b) {
-    const unsigned long long z = (unsigned long long)a * b;
-    uint32_t r = (uint32_t)(z & 0x7FFFFFFFu) + (uint32_t)(z >> 31);
-    r = (r & 0x7FFFFFFFu) + (r >> 31);
-    return r >= 0x7FFFFFFFu ? r - 0x7FFFFFFFu : r;
-}
+// get_rank (utils.py:134-140): sum over the S slices T[i,:,:] of the matrix rank.  The reference takes a float32 SVD;
+// here the rank over Q is computed exactly: fraction-free elimination (row <- row*piv - row[c]*pivrow) over GF(p), one
+// matrix per group of S lanes, lane = matrix row.  rank_p <= rank_Q.  With r the largest rank_p over primes p_1 .. p_k,
+// rank_Q > r needs a non-zero (r+1) x (r+1) minor divisible by every p_j, i.e. one of size >= p_1 ... p_k > 2^(30 k)
+// (primes 2^31 - c).  By Hadamard a minor is at most the product of the norms of its rows; a lane bounds its row's
+// |row|^2 by 2^e (e = ceil(log2 |row|^2) <= 19), so once the r+1 largest e of the slice sum to at most 60 k -- or r is the
+// slice's count of non-zero rows -- r = rank_Q.  Until then the slice is eliminated again mod the next prime: one prime
+// for the few-unit entries of most game states, up to eight for int8 extremes at 25x25x25.
+__constant__ uint32_t c_rank_c[8] = {1, 19, 61, 69, 85, 99, 105, 151}; // p = 2^31 - c, all prime
 
 template <int S>
-__global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__restrict__ ranks, long long B) {
-    using G = Geo<S>;
-    constexpr int LG = S;       // lanes per matrix: 4 / 9 / 16 (the shuffles address absolute lanes, so any group size works)
-    constexpr int MPW = 32 / LG; // matrices per warp: 8 / 3 (lanes 27..31 idle; two per warp with groups of 16 was 1.5x slower) / 2
-    constexpr uint32_t P = 0x7FFFFFFFu;
-    const int lane = threadIdx.x & 31;
-    const int sub = lane / LG, r = lane % LG;
-    const long long warp = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
-    const long long mat = warp * MPW + sub; // matrix index = game * S + slice
-    const long long game = mat / S;
-    const int slice = (int)(mat - game * S);
-    const bool live = sub < MPW && game < B && r < S;
+__device__ __forceinline__ int rank_mod_p(const int8_t *__restrict__ src, bool live, int lane, uint32_t gmask, uint32_t P, uint32_t C) {
     uint32_t row[S];
 #pragma unroll
     for (int c = 0; c < S; c++) {
-        int v = 0;
-        if (live) v = slab[game * G::GP + slice * G::RP + r * S + c];
+        const int v = live ? src[c] : 0;
         row[c] = v >= 0 ? (uint32_t)v : P - (uint32_t)(-v);
     }
-    const uint32_t gmask = sub < MPW ? (((1u << LG) - 1u) << (sub * LG)) : 0u;
     bool used = !live;
     int rank = 0;
 #pragma unroll
@@ -1069,14 +1053,62 @@ __global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__re
         for (int k = c + 1; k < S; k++) {
             const uint32_t pk = __shfl_sync(0xFFFFFFFFu, row[k], pl);
             if (elim) {
+                // 2^31 = C (mod P): fold the bits above 31 twice, then one conditional subtraction (C <= 151)
                 const unsigned long long z = (unsigned long long)row[k] * pv + (unsigned long long)nmine * pk; // < 2^63
-                unsigned long long r = (z & 0x7FFFFFFFull) + (z >> 31);                                        // < 2^33
-                uint32_t q = (uint32_t)(r & 0x7FFFFFFFull) + (uint32_t)(r >> 31);
+                unsigned long long r = (z & 0x7FFFFFFFull) + (z >> 31) * C;                                    // < 2^40
+                uint32_t q = (uint32_t)(r & 0x7FFFFFFFull) + (uint32_t)(r >> 31) * C;                          // < P + 2^18
                 row[k] = q >= P ? q - P : q;
             }
         }
         if (has && lane == pl) used = true;
         rank += has ? 1 : 0;
+    }
+    return rank;
+}
+
+template <int S>
+__global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__restrict__ ranks, long long B) {
+    using G = Geo<S>;
+    constexpr int LG = S;       // lanes per matrix: 4 / 9 / 16 (the shuffles address absolute lanes, so any group size works)
+    constexpr int MPW = 32 / LG; // matrices per warp: 8 / 3 (lanes 27..31 idle; two per warp with groups of 16 was 1.5x slower) / 2
+    const int lane = threadIdx.x & 31;
+    const int sub = lane / LG, r = lane % LG;
+    const long long warp = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const long long mat = warp * MPW + sub; // matrix index = game * S + slice
+    const long long game = mat / S;
+    const int slice = (int)(mat - game * S);
+    const bool live = sub < MPW && game < B && r < S;
+    const int8_t *src = slab + (live ? game * G::GP + slice * G::RP + r * S : 0);
+    const uint32_t gmask = sub < MPW ? (((1u << LG) - 1u) << (sub * LG)) : 0u;
+    int rank = rank_mod_p<S>(src, live, lane, gmask, 0x7FFFFFFFu, 1u);
+    uint32_t n2 = 0; // |row|^2 <= 25 * 128^2 < 2^19
+#pragma unroll
+    for (int c = 0; c < S; c++) {
+        const int v = live ? src[c] : 0;
+        n2 += (uint32_t)(v * v);
+    }
+    const int e = n2 <= 1 ? 0 : 32 - __clz(n2 - 1); // |row|^2 <= 2^e
+    const int emax = (int)__reduce_max_sync(0xFFFFFFFFu, (unsigned)e);
+    const int nzrows = __popc(__ballot_sync(0xFFFFFFFFu, n2 != 0) & gmask);
+    // sum of the m largest e of the group (sum over t of min(m, #{e >= t})): an m x m minor is at most 2^(that / 2)
+    auto top_e = [&](int m) {
+        int E = 0;
+        for (int t = 1; t <= emax; t++) E += min(m, __popc(__ballot_sync(0xFFFFFFFFu, e >= t) & gmask));
+        return E;
+    };
+    // rank_Q > r (the largest rank_p so far) needs a non-zero (r+1) x (r+1) minor that every prime so far divides: none
+    // exists once the product of the primes (> 2^(30 j)) exceeds the minor's Hadamard bound, or once r = nzrows
+    bool fin = rank == nzrows;
+    if (!__all_sync(0xFFFFFFFFu, fin)) {
+        const int E = top_e(rank + 1);
+        fin = fin || E <= 60;
+    }
+#pragma unroll 1
+    for (int j = 1; j < 8 && !__all_sync(0xFFFFFFFFu, fin); j++) { // every lane runs the shuffles
+        const int rj = rank_mod_p<S>(src, live, lane, gmask, 0x80000000u - c_rank_c[j], c_rank_c[j]);
+        if (!fin) rank = max(rank, rj);
+        const int E = top_e(rank + 1);
+        fin = fin || rank == nzrows || E <= 60 * (j + 1);
     }
     // every lane of a group counted the same pivots; add the slices of a game
     if (live && r == 0) atomicAdd(&ranks[game], rank);

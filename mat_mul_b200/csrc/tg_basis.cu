@@ -26,10 +26,11 @@
 //     X[b][c][i] = sum_a A[i][a] T[a][b][c]
 //     Y[c][i][j] = sum_b B[j][b] X[b][c][i]
 //     Z[i][j][k] = sum_c C[k][c] Y[c][i][j]
-// Intermediates live in shared memory as int32 (exact for any int8 input and
-// int8 matrices); a thread owns one column of the contracted axis in registers
-// and produces its S outputs.  TG_FLAG_RANGE marks games whose T' leaves the
-// int8 slab's guaranteed zone [-64,63].
+// X and Y live in shared memory as int32 (|Y| <= S^2 * 2^21 <= 2^29 for int8
+// input and int8 matrices); the last pass accumulates in 64 bit, because |T'|
+// reaches S^3 * 2^28 = 2^34 .. 2^40.  A thread owns one column of the
+// contracted axis in registers and produces its S outputs.  TG_FLAG_RANGE marks
+// games whose T' leaves the int8 slab's guaranteed zone [-64,63].
 #include "tg_common.cuh"
 
 namespace tg {
@@ -42,23 +43,27 @@ struct BasisCfg {
     static constexpr int SMEM_BYTES = G::GP + 2 * S3 * 4 + 3 * S2 * 4 + 16;
 };
 
-// out[rest][a'] = sum_a M[a'][a] in[a][rest]; `rest` has S*S entries.
-template <int S, int NT>
+// out[rest][a'] = sum_a M[a'][a] in[a][rest]; `rest` has S*S entries.  Acc = long long: the sums are formed in 64 bit,
+// stored as their low 32 bits, and TG_FLAG_RANGE is OR-ed into *s_flag where one does not fit int32.
+template <int S, int NT, typename Acc = int32_t>
 __device__ __forceinline__ void mode_pass(const int32_t *__restrict__ in, int32_t *__restrict__ out,
-                                          const int32_t *__restrict__ M) {
+                                          const int32_t *__restrict__ M, uint32_t *s_flag = nullptr) {
     constexpr int S2 = S * S;
+    bool wide = false;
     for (int r = threadIdx.x; r < S2; r += NT) {
         int32_t col[S];
 #pragma unroll
         for (int a = 0; a < S; a++) col[a] = in[a * S2 + r];
 #pragma unroll
         for (int ap = 0; ap < S; ap++) {
-            int32_t acc = 0;
+            Acc acc = 0;
 #pragma unroll
-            for (int a = 0; a < S; a++) acc += M[ap * S + a] * col[a];
-            out[r * S + ap] = acc;
+            for (int a = 0; a < S; a++) acc += (Acc)M[ap * S + a] * col[a];
+            out[r * S + ap] = (int32_t)acc;
+            if constexpr (sizeof(Acc) > 4) wide |= acc != (Acc)(int32_t)acc;
         }
     }
+    if (wide) atomicOr(s_flag, (uint32_t)TG_FLAG_RANGE);
 }
 
 
@@ -113,7 +118,7 @@ __global__ void __launch_bounds__(BasisCfg<S>::NT)
     __syncthreads();
     mode_pass<S, NT>(s_b, s_a, s_m + C::S2); // contract b with B
     __syncthreads();
-    mode_pass<S, NT>(s_a, s_b, s_m + 2 * C::S2); // contract c with C -> Z[i][j][k]
+    mode_pass<S, NT, long long>(s_a, s_b, s_m + 2 * C::S2, s_flag); // contract c with C -> Z[i][j][k]
     __syncthreads();
     uint32_t bad = 0;
     if constexpr (OUT16) {
@@ -704,13 +709,34 @@ __global__ void __launch_bounds__(64)
 }
 
 // ------------------------------------------------------------------ 4x4x4: one THREAD per game
-// A 4x4x4 game is 64 bytes and its three matrices 48: the whole change of basis fits the registers of one thread, exact in
-// int32 (the same ring arithmetic as basis_kernel, so the same results for any int8 input): contract c with DP4A on the
+// A 4x4x4 game is 64 bytes and its three matrices 48: the whole change of basis fits the registers of one thread, in int32
+// ring arithmetic (the stored low bytes are those of the true T' for any int8 input): contract c with DP4A on the
 // packed input words (Y[a][b][k'] = dp4a(T[a][b][.], C[k'][.])), then b and a with scalar matrix entries -- 64 DP4A + 512
 // IMAD per game, no CTA barrier (the packed-lane kernel above needs three CTA barriers per 64 games and spends its time
 // in them: 5.9 G games/s, 0.21 of HBM).  The 32 results of a warp are one contiguous block of the output slab: they go
 // through a warp-private stage in shared memory (thread-major in, linear out) so that every store instruction writes 512
 // contiguous bytes instead of 16-byte pieces of 32 different lines.
+// |T'| <= 128 * nA * nB * nC (n = largest absolute row sum of a matrix).  Where that bound passes 2^31 - 1 an int32 result
+// may have wrapped into the range it is tested against, so such a game's range test is redone here in 64 bit, one entry
+// at a time from global memory (matrices whose row sums multiply to more than 2^24: never those of a game).
+template <bool OUT16>
+__device__ __noinline__ bool basis4_out_of_range_wide(const int8_t *__restrict__ game, const int8_t *__restrict__ m) {
+    const long long lo = OUT16 ? -32768 : -64, hi = OUT16 ? 32767 : 63;
+    bool bad = false;
+#pragma unroll 1
+    for (int e = 0; e < 64; e++) {
+        const int i = e >> 4, j = (e >> 2) & 3, k = e & 3;
+        long long v = 0;
+#pragma unroll 1
+        for (int abc = 0; abc < 64; abc++) {
+            const int a = abc >> 4, b = (abc >> 2) & 3, c = abc & 3;
+            v += (long long)(m[4 * i + a] * m[16 + 4 * j + b]) * (m[32 + 4 * k + c] * game[abc]);
+        }
+        bad |= v < lo || v > hi;
+    }
+    return bad;
+}
+
 template <bool OUT16>
 __global__ void __launch_bounds__(128)
     basis4_thread_kernel(const int8_t *__restrict__ slab_in, const int8_t *__restrict__ mats, long long mat_stride,
@@ -795,7 +821,17 @@ __global__ void __launch_bounds__(128)
         }
         bad >>= 7;
     }
-    if (flags && nw0 + lane < N) flags[n] = bad ? (uint8_t)TG_FLAG_RANGE : (uint8_t)0;
+    if (flags && nw0 + lane < N) {
+        uint32_t na = 0, nb = 0, nc = 0; // largest absolute row sums (|-128| counts 128: unsigned bytes of __vabs4)
+#pragma unroll
+        for (int r = 0; r < 4; r++) {
+            na = max(na, __dp4a(__vabs4(rA[r]), 0x01010101u, 0u));
+            nb = max(nb, __dp4a(__vabs4(rB[r]), 0x01010101u, 0u));
+            nc = max(nc, __dp4a(__vabs4(rC[r]), 0x01010101u, 0u));
+        }
+        if (128ull * na * nb * nc > 0x7FFFFFFFull && basis4_out_of_range_wide<OUT16>(slab_in + n * 64, mats + n * mat_stride)) bad = 1;
+        flags[n] = bad ? (uint8_t)TG_FLAG_RANGE : (uint8_t)0;
+    }
     __syncwarp();
     const int total = (int)min(32LL, N - nw0) * IPG;
     uint4 *out = reinterpret_cast<uint4 *>(reinterpret_cast<uint8_t *>(slab_out) + nw0 * (IPG * 16));

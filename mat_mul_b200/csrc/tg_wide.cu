@@ -11,7 +11,8 @@
 
 namespace tg {
 
-// slab16[n] = sum_r rank1(tape[r][n]) in plain int32 arithmetic per entry (exact for every tape), stored as int16.
+// slab16[n] = sum_r rank1(tape[r][n]) in plain int32 arithmetic per entry, stored as int16.  Exact while R * cmax^3 fits
+// int32 (cmax = max(shift, 255 - shift), the largest |token - shift| of a byte); longer tapes go to the kernel below.
 // Thread (demo, word column c) owns the entries (i, 4c .. 4c+3) of every row; the CTA stages the records of its demos for
 // one step at a time in shared memory.
 template <int S>
@@ -79,6 +80,27 @@ __global__ void __launch_bounds__(256)
     if (flags && tid < ng) flags[g0 + tid] = (uint8_t)s_bad[tid];
 }
 
+// The same sum in 64 bit, one thread per entry: for tapes whose terms could carry an int32 sum past 2^31 (R >= 130 at
+// shift 0, R >= 1024 at shift 127).
+template <int S>
+__global__ void __launch_bounds__(256)
+    demo_accumulate_i16_wide_kernel(const uint8_t *__restrict__ tape, long long tape_step_stride, long long N, int R, int shift,
+                                    int16_t *__restrict__ slab16, uint8_t *__restrict__ flags) {
+    using G = Geo<S>;
+    for (long long x = blockIdx.x * (long long)blockDim.x + threadIdx.x; x < N * G::GP; x += (long long)gridDim.x * blockDim.x) {
+        const long long n = x / G::GP;
+        const int e = (int)(x % G::GP), i = e / G::RP, jk = e % G::RP, j = jk / S, k = jk % S;
+        long long v = 0;
+        if (i < S && jk < G::S2) {
+            const uint8_t *tok = tape + n * G::TP;
+            for (int r = 0; r < R; r++, tok += tape_step_stride)
+                v += (long long)(((int)__ldg(tok + i) - shift) * ((int)__ldg(tok + S + j) - shift)) * ((int)__ldg(tok + 2 * S + k) - shift);
+        }
+        slab16[x] = (int16_t)v;
+        if (flags && (v < -32768 || v > 32767)) flags[n] = (uint8_t)TG_FLAG_RANGE; // same value from every writer
+    }
+}
+
 // slab16 -> float32 dense (S,S,S) at dst + b*dst_stride; one thread per pair of entries
 template <int S>
 __global__ void expand_f32_i16_kernel(const int16_t *__restrict__ slab16, float *__restrict__ dst, long long dst_stride, long long B) {
@@ -134,6 +156,17 @@ int tg_demo_accumulate_i16(const uint8_t *tape, int64_t tape_step_stride, int64_
     if (!tape || !slab16) return TG_E_ARG;
     if (((uintptr_t)tape | (uintptr_t)slab16 | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
+    const long long cmax = shift > 255 - shift ? shift : 255 - shift;
+    if ((long long)R * cmax * cmax * cmax > 0x7FFFFFFFLL) {
+        if (flags) TG_CUDA(cudaMemsetAsync(flags, 0, (size_t)N, st));
+        TG_SWITCH_S(S, {
+            const long long blocks = (N * tg::Geo<kS>::GP + 255) / 256;
+            tg::demo_accumulate_i16_wide_kernel<kS><<<(unsigned)(blocks < 148 * 32 ? blocks : 148 * 32), 256, 0, st>>>(
+                tape, tape_step_stride, N, R, shift, slab16, flags);
+        });
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    }
     TG_SWITCH_S(S, {
         constexpr int DPC = 256 / tg::Geo<kS>::WR;
         const long long grid = (N + DPC - 1) / DPC;
