@@ -60,7 +60,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 200
+#define TG_VERSION 201
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -69,7 +69,7 @@ extern "C" {
 
 #define TG_FLAG_TERMINAL 1u /* new head all zero: utils.py:181-188 on the head (act.py:177) */
 #define TG_FLAG_NULL 2u     /* rank-1 update all zero: utils.py:191-194 */
-#define TG_FLAG_RANGE 4u    /* a residual entry left [-64, 63] (int8 slab no longer guaranteed) or a token exceeded 2*shift */
+#define TG_FLAG_RANGE 4u    /* a residual entry left the guaranteed zone ([-64, 63] int8, [-16384, 16383] int16) or a token exceeded 2*shift */
 #define TG_FLAG_EXHAUSTED 8u /* demo generation: a term hit max_tries and was forced to a unit triple */
 #define TG_FLAG_TOKEN_RANGE 16u /* change of basis: a transformed factor entry left [-shift_out, shift_out] */
 #define TG_FLAG_PATH_PLANES 32u /* change of basis, informational: 16x16x16 game computed on int8 byte planes (not f16) */
@@ -239,6 +239,35 @@ int tg_slice_rank(const int8_t *slab, int32_t *ranks, int64_t B, int S, void *st
  * odd vectors: linear in T, and the key of a rank-1 action u (x) v (x) w is (sum u_i A_i)(sum v_j B_j)(sum w_k C_k),
  * which is how tg_expand_children keys a child without a pass over it.  (TG_VERSION 200 changed the constants.) */
 int tg_state_key(const int8_t *slab, uint64_t *keys, int64_t B, int S, void *stream);
+
+/* ---- int16 game path: K1, K8, K2, K7, K6 on int16 slabs (S in {4, 9, 16, 25}) ----------------------------------- */
+/* The int16 twins of tg_step, tg_expand_children, tg_rollout, tg_replay, tg_state_key and tg_slice_rank, for residuals
+ * the int8 slab cannot hold (tg_change_of_basis_i16 outputs, tg_demo_accumulate_i16 targets, start tensors with large
+ * entries).  Same arguments, checks and outputs as the int8 twin, with int16 slabs [B][GP] of int16: entry (i,j,k) at
+ * element i*RP + j*S + k, padding elements zero, 16-byte aligned.
+ *   - Tokens: the same token bound (every token <= 2*shift, shift in [1,4], so |u v w| <= 64 per step); a record that
+ *     breaks it raises TG_FLAG_RANGE (the game's result is then unspecified).
+ *   - Zone: entries are guaranteed while they stay in [-16384, 16383] (the top two bits of a 16-bit lane are equal).
+ *     A step whose result leaves the zone raises TG_FLAG_RANGE and is still exact; the next one is not guaranteed.
+ *     tg_rollout_i16 / tg_replay_i16 test the zone after every applied step: RANGE = the start state or the state after
+ *     an applied step had an entry outside the zone, or an applied step's record broke the token bound.
+ *   - TG_FLAG_TERMINAL, TG_FLAG_NULL, nnz and steps mean what they mean on int8.
+ *   - tg_state_key_i16 is tg_state_key's trilinear form over the int16 values: a state whose values fit int8 has the
+ *     same key in both formats, so int8 and int16 nodes share one MCTS tree.  tg_expand_children_i16 keys its children
+ *     by the same parent-minus-action rule as tg_expand_children.
+ *   - tg_slice_rank_i16: exact rank over Q for every int16 slab (no zone), with up to fifteen 31-bit primes.
+ * tg_expand_children_i16 holds a CTA's k records in shared memory and returns TG_E_ARG when they do not fit
+ * (k above about 1200 at 25x25x25, more at the smaller sizes). */
+int tg_step_i16(const int16_t *slab_in, const uint8_t *tape, int16_t *slab_out, uint8_t *flags, int32_t *nnz, int64_t B, int S,
+                int shift, void *stream);
+int tg_expand_children_i16(const int16_t *parents, const uint8_t *tape, int k, int16_t *children, uint8_t *flags, int32_t *nnz,
+                           uint64_t *keys, int64_t B, int S, int shift, void *stream);
+int tg_rollout_i16(const int16_t *slab_in, const uint8_t *tape, int64_t tape_step_stride, int K, int16_t *slab_out, uint8_t *flags,
+                   int32_t *nnz, int32_t *steps, int64_t B, int S, int shift, void *stream);
+int tg_replay_i16(const int16_t *slab_in, const uint8_t *tape, int64_t tape_step_stride, int K, int16_t *slab_out, uint8_t *flags,
+                  int32_t *nnz, int64_t B, int S, int shift, void *stream);
+int tg_state_key_i16(const int16_t *slab16, uint64_t *keys, int64_t B, int S, void *stream);
+int tg_slice_rank_i16(const int16_t *slab16, int32_t *ranks, int64_t B, int S, void *stream);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

@@ -120,6 +120,12 @@ _SIGNATURES = {
     "tg_demo_accumulate_i16": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
     "tg_pack_f32_i16": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, _vp, _vp]),
     "tg_expand_f32_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
+    "tg_step_i16": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_expand_children_i16": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_rollout_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_replay_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_state_key_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_slice_rank_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
     "tg_change_of_basis_factors": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp, C.c_int64,
                                              C.c_int, C.c_int, _vp]),
     "tg_sample_unimodular": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),

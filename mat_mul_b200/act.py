@@ -24,7 +24,7 @@ except ImportError:  # pragma: no cover - model.py is not part of this package
 
 from mat_mul_b200 import env as _env
 from mat_mul_b200.utils import *  # noqa: F401,F403
-from mat_mul_b200.utils import _COEF_SHIFT, ChildStates, _device, _heads_to_slab
+from mat_mul_b200.utils import _COEF_SHIFT, ChildStates, _device, _heads_to_slab, _slab_to_heads
 
 _MAX_EXPANSION_TRIES = 1000  # the reference loops forever when every sampled child is null or known (SURVEY Q11)
 
@@ -42,18 +42,20 @@ def get_child_states(state: torch.Tensor, actions: torch.Tensor, vec_cardinality
     bs, k = actions.shape[:2]
     S = state.shape[-1]
     dev = _device()
-    head = _heads_to_slab(state[:, 0], S)                                   # (bs, GP)
+    head = _heads_to_slab(state[:, 0], S)                                   # (bs, GP), int8 or int16
     # the reference's coefficient is token - 1 whatever the alphabet (action_to_tensor, SURVEY Q1): re-based to the
     # kernels' widest alphabet (token + 3, shift 4) so that the token bound of the packed arithmetic holds
     tape = _env.pack_actions(actions.reshape(bs * k, -1).to(dev).to(torch.int64).contiguous(), S,
                              rebase=_COEF_SHIFT - 1).reshape(bs, k, -1)
     # one launch: the k children of every state, their null / terminal flags, non-zero counts and state keys (K8)
     out, flags, nnz, keys = _env.expand_children(head, tape, S, _COEF_SHIFT)
+    if head.dtype == torch.int8 and bool((flags & _env.FLAG_RANGE).any()):
+        # the reference computes in float32 and never wraps: children the int8 slab cannot hold are made from the int16
+        # slab of the same values (same element layout)
+        out, flags, nnz, keys = _env.expand_children(head.to(torch.int16), tape, S, _COEF_SHIFT)
     if bool((flags & _env.FLAG_RANGE).any()):
-        # the reference computes in float32 and never wraps; the int8 slab cannot hold these children
-        raise _env.TensorGameError("get_child_states: a child state left the int8 slab's guaranteed range [-64, 63]")
-    out = out.reshape(bs * k, -1)
-    new_heads = _env.expand_states(out, S).reshape(bs, k, S, S, S).to(device=state.device, dtype=state.dtype)
+        raise _env.TensorGameError("get_child_states: a child state left the int16 slab's guaranteed range [-16384, 16383]")
+    new_heads = _slab_to_heads(out.reshape(bs * k, -1), S, (bs, k), state.dtype, state.device)
     children = ChildStates(torch.cat([new_heads[:, i : i + 1], state[:, :-1]], dim=1) for i in range(k))
     f = flags.reshape(bs, k)
     children.parent = state

@@ -18,7 +18,7 @@ from torch.utils.data import Dataset
 
 from mat_mul_b200 import env as _env
 from mat_mul_b200.utils import *  # noqa: F401,F403
-from mat_mul_b200.utils import _device, _COEF_SHIFT, TensorGameError
+from mat_mul_b200.utils import _device, _COEF_SHIFT, TensorGameError, _heads_to_slab, _slab_to_heads
 
 SAVE_DIR_SYNTH_DEMOS = Path("data_unversioned/synthetic_demos")
 SAVE_DIR_VAL = Path("data_unversioned/synthetic_demos_val")
@@ -153,11 +153,14 @@ class SyntheticDemoDataset(Dataset):
         # coefficient = token - 1 (action_to_tensor's fixed shift, SURVEY Q1), re-based to (token + 3, shift 4) so that
         # the kernels' token bound holds for every alphabet the reference's datasets use
         tape = _env.pack_actions(tokens, S, rebase=_COEF_SHIFT - 1).unsqueeze(1)
-        slab = _env.pack_states(target_tensor.reshape(1, S, S, S).to(dev).float().contiguous(), S)
+        slab = _heads_to_slab(target_tensor.reshape(1, S, S, S), S)  # int8, or int16 for targets beyond it
         out, flags, _ = _env.replay(slab, tape, S, _COEF_SHIFT)
+        if slab.dtype == torch.int8 and bool((flags & _env.FLAG_RANGE).any()):
+            # the reference computes in float32 and never wraps: replay the int16 slab of the same values
+            out, flags, _ = _env.replay(slab.to(torch.int16), tape, S, _COEF_SHIFT)
         if bool((flags & _env.FLAG_RANGE).any()):
-            raise TensorGameError("_take_actions left the int8 slab's guaranteed range [-64, 63]")
-        return _env.expand_states(out, S)[0].to(target_tensor.device)
+            raise TensorGameError("_take_actions left the int16 slab's guaranteed range [-16384, 16383]")
+        return _slab_to_heads(out, S, (), torch.float32, target_tensor.device)
 
     def _factor_sample(self):
         """datasets.py:155-158"""

@@ -82,6 +82,14 @@ def _p(t: torch.Tensor | None) -> C.c_void_p:
     return C.c_void_p(0 if t is None else t.data_ptr())
 
 
+def _game_slab(slab: torch.Tensor, name: str = "slab") -> str:
+    """Checks a residual slab, int8 or int16 (include/tensorgame.h "int16 game path"), and returns the suffix of the
+    entry points for its dtype: "" or "_i16"."""
+    wide = isinstance(slab, torch.Tensor) and slab.dtype == torch.int16
+    _need_cuda(slab, name, torch.int16 if wide else torch.int8)
+    return "_i16" if wide else ""
+
+
 # ---------------------------------------------------------------- formats
 def new_slab(B: int, S: int, device) -> torch.Tensor:
     """Zeroed residual slab, int8 (B, GP)."""
@@ -190,10 +198,10 @@ def step_batch(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: 
                flags: torch.Tensor | None = None, nnz: torch.Tensor | None = None):
     """One transition for every game: out = slab - u(x)v(x)w.  Returns (out, flags, nnz).
 
-    flags uint8 (B,): FLAG_TERMINAL | FLAG_NULL | FLAG_RANGE; nnz int32 (B,).
-    Reference: act.py:266-275, training.py:253-267, utils.py:181-194.
+    slab int8 or int16 (tg_step_i16); out has its dtype.  flags uint8 (B,): FLAG_TERMINAL | FLAG_NULL | FLAG_RANGE;
+    nnz int32 (B,).  Reference: act.py:266-275, training.py:253-267, utils.py:181-194.
     """
-    _need_cuda(slab, "slab", torch.int8)
+    sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
     B = slab.shape[0]
     lay = layout(S)
@@ -202,7 +210,7 @@ def step_batch(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: 
     out = torch.empty_like(slab) if out is None else out
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device) if flags is None else flags
     nnz = torch.empty(B, dtype=torch.int32, device=slab.device) if nnz is None else nnz
-    _call("tg_step", (slab, tape, out, flags, nnz,), _p(slab), _p(tape), _p(out), _p(flags), _p(nnz), B, S, shift)
+    _call("tg_step" + sfx, (slab, tape, out, flags, nnz,), _p(slab), _p(tape), _p(out), _p(flags), _p(nnz), B, S, shift)
     return out, flags, nnz
 
 
@@ -210,10 +218,10 @@ def step_batch(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: 
 def expand_children(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, with_keys: bool = True):
     """Batched leaf expansion (tg_expand_children): children[b, c] = slab[b] - rank1(tape[b, c]).
 
-    slab int8 (B, GP), tape uint8 (B, k, TP).  Returns (children (B, k, GP), flags (B, k), nnz (B, k), keys (B, k) or
-    None).  Reference: act.py:266-275 get_child_states + the null / terminal / already-in-tree tests of extend_tree
-    (act.py:177-195), for B states at once."""
-    _need_cuda(slab, "slab", torch.int8)
+    slab int8 or int16 (B, GP) (tg_expand_children_i16), tape uint8 (B, k, TP).  Returns (children (B, k, GP) of the
+    slab's dtype, flags (B, k), nnz (B, k), keys (B, k) or None).  Reference: act.py:266-275 get_child_states + the
+    null / terminal / already-in-tree tests of extend_tree (act.py:177-195), for B states at once."""
+    sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
     lay = layout(S)
     B = slab.shape[0]
@@ -221,18 +229,19 @@ def expand_children(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, 
         raise TensorGameError(f"expected slab (B,{lay.game_pitch}) and tape (B,k,{lay.token_pitch})")
     k = tape.shape[1]
     dev = slab.device
-    children = torch.empty((B, k, lay.game_pitch), dtype=torch.int8, device=dev)
+    children = torch.empty((B, k, lay.game_pitch), dtype=slab.dtype, device=dev)
     flags = torch.empty((B, k), dtype=torch.uint8, device=dev)
     nnz = torch.empty((B, k), dtype=torch.int32, device=dev)
     keys = torch.empty((B, k), dtype=torch.int64, device=dev) if with_keys else None
-    _call("tg_expand_children", (slab, tape, children, flags, nnz, keys,), _p(slab), _p(tape), k, _p(children), _p(flags), _p(nnz), _p(keys), B, S, shift)
+    _call("tg_expand_children" + sfx, (slab, tape, children, flags, nnz, keys,), _p(slab), _p(tape), k, _p(children), _p(flags), _p(nnz), _p(keys), B, S, shift)
     return children, flags, nnz, keys
 
 
 def rollout(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torch.Tensor | None = None):
     """Apply a step-major tape (K, B, TP) to every game, freezing solved games.
-    Returns (out, flags, nnz, steps).  Reference: datasets.py:144-153, training.py:336-342, act.py:49."""
-    _need_cuda(slab, "slab", torch.int8)
+    slab int8 or int16 (tg_rollout_i16).  Returns (out, flags, nnz, steps).  Reference: datasets.py:144-153,
+    training.py:336-342, act.py:49."""
+    sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
     lay = layout(S)
     B = slab.shape[0]
@@ -243,13 +252,14 @@ def rollout(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: tor
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device)
     nnz = torch.empty(B, dtype=torch.int32, device=slab.device)
     steps = torch.empty(B, dtype=torch.int32, device=slab.device)
-    _call("tg_rollout", (slab, tape, out, flags, nnz, steps,), _p(slab), _p(tape), B * lay.token_pitch, K, _p(out), _p(flags), _p(nnz), _p(steps), B, S, shift)
+    _call("tg_rollout" + sfx, (slab, tape, out, flags, nnz, steps,), _p(slab), _p(tape), B * lay.token_pitch, K, _p(out), _p(flags), _p(nnz), _p(steps), B, S, shift)
     return out, flags, nnz, steps
 
 
 def replay(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torch.Tensor | None = None):
-    """All K actions of a step-major tape applied without freezing (datasets.py:144-153).  Returns (out, flags, nnz)."""
-    _need_cuda(slab, "slab", torch.int8)
+    """All K actions of a step-major tape applied without freezing (datasets.py:144-153); slab int8 or int16
+    (tg_replay_i16).  Returns (out, flags, nnz)."""
+    sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
     lay = layout(S)
     B, K = slab.shape[0], tape.shape[0]
@@ -258,7 +268,7 @@ def replay(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torc
     out = torch.empty_like(slab) if out is None else out
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device)
     nnz = torch.empty(B, dtype=torch.int32, device=slab.device)
-    _call("tg_replay", (slab, tape, out, flags, nnz,), _p(slab), _p(tape), B * lay.token_pitch, K, _p(out), _p(flags), _p(nnz), B, S, shift)
+    _call("tg_replay" + sfx, (slab, tape, out, flags, nnz,), _p(slab), _p(tape), B * lay.token_pitch, K, _p(out), _p(flags), _p(nnz), B, S, shift)
     return out, flags, nnz
 
 
@@ -484,10 +494,10 @@ class DemoStore:
 
 
 def slice_rank(slab: torch.Tensor, S: int) -> torch.Tensor:
-    """get_rank per game (utils.py:134-140): int32 (B,)."""
-    _need_cuda(slab, "slab", torch.int8)
+    """get_rank per game (utils.py:134-140) of an int8 or int16 slab (tg_slice_rank_i16): int32 (B,)."""
+    sfx = _game_slab(slab)
     ranks = torch.empty(slab.shape[0], dtype=torch.int32, device=slab.device)
-    _call("tg_slice_rank", (slab, ranks,), _p(slab), _p(ranks), slab.shape[0], S)
+    _call("tg_slice_rank" + sfx, (slab, ranks,), _p(slab), _p(ranks), slab.shape[0], S)
     return ranks
 
 
@@ -507,10 +517,11 @@ def episode_returns(final_slab: torch.Tensor, steps: torch.Tensor, S: int, max_l
 
 
 def state_keys(slab: torch.Tensor, S: int) -> torch.Tensor:
-    """64-bit state keys (as int64 bit patterns), replacing utils.state_to_str dict keys."""
-    _need_cuda(slab, "slab", torch.int8)
+    """64-bit state keys (as int64 bit patterns), replacing utils.state_to_str dict keys.  An int16 slab
+    (tg_state_key_i16) gives the same key as an int8 slab of the same values."""
+    sfx = _game_slab(slab)
     keys = torch.empty(slab.shape[0], dtype=torch.int64, device=slab.device)
-    _call("tg_state_key", (slab, keys,), _p(slab), _p(keys), slab.shape[0], S)
+    _call("tg_state_key" + sfx, (slab, keys,), _p(slab), _p(keys), slab.shape[0], S)
     return keys
 
 

@@ -28,13 +28,18 @@ def _device() -> torch.device:
 
 
 def _heads_to_slab(heads: torch.Tensor, S: int) -> torch.Tensor:
-    """(..., S, S, S) tensor of any dtype/device -> slab int8 (N, GP) on the CUDA device."""
+    """(..., S, S, S) tensor of any dtype/device -> slab (N, GP) on the CUDA device: int8 whenever every value is an
+    integer in [-128, 127], int16 otherwise (the reference computes in float32 and has no such limit).  Raises if a
+    value is not an integer in [-32768, 32767].  The one place the mirrors choose a slab format."""
     h = heads.reshape(-1, S, S, S).to(device=_device(), dtype=torch.float32).contiguous()
-    return _env.pack_states(h, S)
+    try:
+        return _env.pack_states(h, S)
+    except TensorGameError:
+        return _env.pack_states16(h, S)
 
 
 def _slab_to_heads(slab: torch.Tensor, S: int, shape, dtype, device) -> torch.Tensor:
-    out = _env.expand_states(slab, S)
+    out = _env.expand_states16(slab, S) if slab.dtype == torch.int16 else _env.expand_states(slab, S)
     return out.reshape(*shape, S, S, S).to(device=device, dtype=dtype)
 
 
@@ -42,7 +47,8 @@ class ChildStates(list):
     """The list get_child_states returns, carrying what the step kernel already knows about every child."""
 
     parent = None       # the state tensor the children were expanded from
-    range_flags = None  # bool (k,): the child left the int8 slab's guaranteed zone (always False: expansion raises)
+    range_flags = None  # bool (k,): the child left the guaranteed zone of the slab it was computed in (always False: a
+    #                     child that leaves the int8 zone is recomputed on an int16 slab, and leaving the int16 zone raises)
     null_flags = None   # bool (k,): child head == parent head (utils.py:191-194)
     terminal = None     # bool (k,): child head all zero
     nnz = None          # int32 (k,)
