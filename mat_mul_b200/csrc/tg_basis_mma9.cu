@@ -115,7 +115,16 @@ __global__ void __launch_bounds__(32 * WARPS)
         const int8_t *rp = mats + n * mat_stride + 9 * lane;
         const uint32_t o = (uint32_t)(reinterpret_cast<uintptr_t>(rp) & 3);
         const uint32_t *w = reinterpret_cast<const uint32_t *>(rp - o);
-        mraw[0] = __ldg(w), mraw[1] = __ldg(w + 1), mraw[2] = __ldg(w + 2);
+        mraw[0] = __ldg(w), mraw[1] = __ldg(w + 1);
+        if (lane == 26 && (mat_stride == 0 || n == N - 1)) {
+            // the last row of the last triple: its third word can reach up to 3 bytes past the triple, which may be the
+            // end of the allocation; only the row's bytes of that word (0 .. o) are read
+            const uint8_t *b = reinterpret_cast<const uint8_t *>(w + 2);
+            mraw[2] = __ldg(b);
+            for (uint32_t e = 1; e <= o; e++) mraw[2] |= (uint32_t)__ldg(b + e) << (8 * e);
+        } else {
+            mraw[2] = __ldg(w + 2);
+        }
         msh = 8 * o;
     }
     const uint32_t *gw = reinterpret_cast<const uint32_t *>(slab_in + n * 768);
