@@ -27,7 +27,7 @@
  *     entry point returns TG_E_CUDA.
  *
  * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
- * K1-K4, K6-K8, parity mode, host buffers).  The change of basis (K5) stays
+ * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths).  The change of basis (K5) stays
  * {4, 9, 16} and tg_demo_accumulate_tc 16; at 25 tg_demo_gen_philox keeps
  * contract v1 for every alphabet (tg_demo_alias_tables returns TG_E_ARG).
  *
@@ -60,7 +60,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 201
+#define TG_VERSION 202
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -268,6 +268,44 @@ int tg_replay_i16(const int16_t *slab_in, const uint8_t *tape, int64_t tape_step
                   int32_t *nnz, int64_t B, int S, int shift, void *stream);
 int tg_state_key_i16(const int16_t *slab16, uint64_t *keys, int64_t B, int S, void *stream);
 int tg_slice_rank_i16(const int16_t *slab16, int32_t *ranks, int64_t B, int S, void *stream);
+
+/* ---- mod-2 game path: K1, K8, K2, K7, K6 on bit slabs (S in {4, 9, 16, 25}) ------------------------------------- */
+/* The game over Z_2 (the AlphaTensor paper's "modular" arithmetic): T' = T xor (u (x) v (x) w mod 2).
+ *   bit slab  uint32 [B][GB/4]  row i of a game is the S^2 bits (j,k) in RW = ceil(S^2/32) little-endian words: entry
+ *                          (i,j,k) is bit (j*S+k) % 32 of word i*RW + (j*S+k)/32; padding bits and words are zero; games
+ *                          are 16-byte aligned at GB = roundup16(4*S*RW) bytes (S=4: 1/16, S=9: 3/112, S=16: 8/512,
+ *                          S=25: 20/2000 words per row / bytes per game).  In torch an int32 tensor [B][GB/4].
+ *   Tapes are unchanged: token t stands for the coefficient t - shift (shift in [1,4], checked as on int8), whose residue
+ *   is (t - shift) & 1.  Every byte is a valid token, so TG_FLAG_RANGE is never raised.
+ *   Each entry point takes its int8 twin's arguments, checks and aliasing rules (in place allowed for step, rollout and
+ *   replay), with bit slabs for slabs:
+ *   - tg_step_gf2: TERMINAL = T' all zero; NULL = the term vanishes mod 2 (u, v or w has only even coefficients; then
+ *     T' = T); nnz = popcount of T'.
+ *   - tg_expand_children_gf2: k children per parent as tg_expand_children, keys optional.
+ *   - tg_rollout_gf2 / tg_replay_gf2: tg_rollout / tg_replay (freeze at solved, steps, tape step stride); flags TERMINAL.
+ *   - tg_state_key_gf2: tg_state_key of the 0/1 unpacking (the trilinear form over the values 0 and 1), so a mod-2 state
+ *     and the int8 slab of its 0/1 values share a key.  tg_expand_children_gf2 keys its children the same way, from the
+ *     child itself (parent-minus-action does not hold under xor).
+ *   - tg_slice_rank_gf2: sum_i rank over GF(2) of T[i,:,:], the slices of tg_slice_rank.
+ * Conversions: tg_pack_gf2 (int8 slab) and tg_pack_gf2_i16 (int16 slab) keep the low bit of each two's-complement entry
+ * (-1 -> 1); tg_unpack_gf2 writes the int8 slab of 0/1 values (to float32 through tg_expand_f32).  tg_demo_accumulate
+ * and tg_demo_gen_philox store the low byte of each entry and tg_demo_accumulate_i16 its int16 value, so packing their
+ * targets gives the mod-2 sum of the tape, RANGE-flagged targets included (tg_demo_accumulate_tc saturates instead: its
+ * targets keep their parity only where they fit int8). */
+int tg_layout_gf2(int S, int *row_words, int *game_bytes);
+int tg_pack_gf2(const int8_t *slab, uint32_t *bits, int64_t B, int S, void *stream);
+int tg_pack_gf2_i16(const int16_t *slab16, uint32_t *bits, int64_t B, int S, void *stream);
+int tg_unpack_gf2(const uint32_t *bits, int8_t *slab, int64_t B, int S, void *stream);
+int tg_step_gf2(const uint32_t *bits_in, const uint8_t *tape, uint32_t *bits_out, uint8_t *flags, int32_t *nnz, int64_t B, int S,
+                int shift, void *stream);
+int tg_expand_children_gf2(const uint32_t *parents, const uint8_t *tape, int k, uint32_t *children, uint8_t *flags, int32_t *nnz,
+                           uint64_t *keys, int64_t B, int S, int shift, void *stream);
+int tg_rollout_gf2(const uint32_t *bits_in, const uint8_t *tape, int64_t tape_step_stride, int K, uint32_t *bits_out, uint8_t *flags,
+                   int32_t *nnz, int32_t *steps, int64_t B, int S, int shift, void *stream);
+int tg_replay_gf2(const uint32_t *bits_in, const uint8_t *tape, int64_t tape_step_stride, int K, uint32_t *bits_out, uint8_t *flags,
+                  int32_t *nnz, int64_t B, int S, int shift, void *stream);
+int tg_state_key_gf2(const uint32_t *bits, uint64_t *keys, int64_t B, int S, void *stream);
+int tg_slice_rank_gf2(const uint32_t *bits, int32_t *ranks, int64_t B, int S, void *stream);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

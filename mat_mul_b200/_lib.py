@@ -126,6 +126,16 @@ _SIGNATURES = {
     "tg_replay_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
     "tg_state_key_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
     "tg_slice_rank_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_layout_gf2": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "tg_pack_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_pack_gf2_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_unpack_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_step_gf2": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_expand_children_gf2": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_rollout_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_replay_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
+    "tg_state_key_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
+    "tg_slice_rank_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
     "tg_change_of_basis_factors": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp, C.c_int64,
                                              C.c_int, C.c_int, _vp]),
     "tg_sample_unimodular": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),

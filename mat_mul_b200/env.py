@@ -82,12 +82,20 @@ def _p(t: torch.Tensor | None) -> C.c_void_p:
     return C.c_void_p(0 if t is None else t.data_ptr())
 
 
+_SLAB_SUFFIX = {torch.int16: "_i16", torch.int32: "_gf2"}
+
+
 def _game_slab(slab: torch.Tensor, name: str = "slab") -> str:
-    """Checks a residual slab, int8 or int16 (include/tensorgame.h "int16 game path"), and returns the suffix of the
-    entry points for its dtype: "" or "_i16"."""
-    wide = isinstance(slab, torch.Tensor) and slab.dtype == torch.int16
-    _need_cuda(slab, name, torch.int16 if wide else torch.int8)
-    return "_i16" if wide else ""
+    """Checks a residual slab, int8, int16 (include/tensorgame.h "int16 game path") or an int32 bit slab ("mod-2 game
+    path"), and returns the suffix of the entry points for its dtype: "", "_i16" or "_gf2"."""
+    sfx = _SLAB_SUFFIX.get(slab.dtype, "") if isinstance(slab, torch.Tensor) else ""
+    _need_cuda(slab, name, {"": torch.int8, "_i16": torch.int16, "_gf2": torch.int32}[sfx])
+    return sfx
+
+
+def _game_pitch(sfx: str, S: int) -> int:
+    """Elements per game of a slab of the format `sfx` selects."""
+    return layout_gf2(S).game_words if sfx == "_gf2" else layout(S).game_pitch
 
 
 # ---------------------------------------------------------------- formats
@@ -193,20 +201,63 @@ def unpack_actions(tape: torch.Tensor, S: int) -> torch.Tensor:
     return out
 
 
+# ---------------------------------------------------------------- mod-2 bit slabs
+@dataclass(frozen=True)
+class LayoutGF2:
+    S: int
+    row_words: int   # RW: 32-bit words per i-row (S^2 bits)
+    game_bytes: int  # GB: bytes per game in a bit slab
+
+    @property
+    def game_words(self) -> int:
+        return self.game_bytes // 4
+
+
+def layout_gf2(S: int) -> LayoutGF2:
+    rw, gb = C.c_int(), C.c_int()
+    check(_lib.lib().tg_layout_gf2(S, C.byref(rw), C.byref(gb)), f"tg_layout_gf2(S={S})")
+    return LayoutGF2(S, rw.value, gb.value)
+
+
+def pack_gf2(slab: torch.Tensor, S: int) -> torch.Tensor:
+    """int8 or int16 slab -> bit slab int32 (B, GB/4) of the residues mod 2 (tg_pack_gf2 / tg_pack_gf2_i16: the low bit
+    of each two's-complement entry)."""
+    sfx = _game_slab(slab)
+    if sfx == "_gf2":
+        raise TensorGameError("pack_gf2 takes an int8 or int16 slab")
+    if slab.dim() != 2 or slab.shape[1] != layout(S).game_pitch:
+        raise TensorGameError(f"expected slab (B,{layout(S).game_pitch})")
+    B = slab.shape[0]
+    bits = torch.empty((B, layout_gf2(S).game_words), dtype=torch.int32, device=slab.device)
+    _call("tg_pack_gf2" + sfx, (slab, bits), _p(slab), _p(bits), B, S)
+    return bits
+
+
+def unpack_gf2(bits: torch.Tensor, S: int) -> torch.Tensor:
+    """bit slab -> int8 slab of 0/1 values (tg_unpack_gf2); expand_states takes it on to float32."""
+    _need_cuda(bits, "bits", torch.int32)
+    if bits.dim() != 2 or bits.shape[1] != layout_gf2(S).game_words:
+        raise TensorGameError(f"expected bits (B,{layout_gf2(S).game_words})")
+    B = bits.shape[0]
+    slab = torch.empty((B, layout(S).game_pitch), dtype=torch.int8, device=bits.device)
+    _call("tg_unpack_gf2", (bits, slab), _p(bits), _p(slab), B, S)
+    return slab
+
+
 # ---------------------------------------------------------------- K1
 def step_batch(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torch.Tensor | None = None,
                flags: torch.Tensor | None = None, nnz: torch.Tensor | None = None):
     """One transition for every game: out = slab - u(x)v(x)w.  Returns (out, flags, nnz).
 
-    slab int8 or int16 (tg_step_i16); out has its dtype.  flags uint8 (B,): FLAG_TERMINAL | FLAG_NULL | FLAG_RANGE;
+    slab int8, int16 (tg_step_i16) or an int32 bit slab (tg_step_gf2: out = slab xor rank1 mod 2); out has its dtype.  flags uint8 (B,): FLAG_TERMINAL | FLAG_NULL | FLAG_RANGE;
     nnz int32 (B,).  Reference: act.py:266-275, training.py:253-267, utils.py:181-194.
     """
     sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
     B = slab.shape[0]
-    lay = layout(S)
-    if slab.shape != (B, lay.game_pitch) or tape.shape != (B, lay.token_pitch):
-        raise TensorGameError(f"expected slab (B,{lay.game_pitch}) and tape (B,{lay.token_pitch})")
+    lay, gp = layout(S), _game_pitch(sfx, S)
+    if slab.shape != (B, gp) or tape.shape != (B, lay.token_pitch):
+        raise TensorGameError(f"expected slab (B,{gp}) and tape (B,{lay.token_pitch})")
     out = torch.empty_like(slab) if out is None else out
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device) if flags is None else flags
     nnz = torch.empty(B, dtype=torch.int32, device=slab.device) if nnz is None else nnz
@@ -218,18 +269,18 @@ def step_batch(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: 
 def expand_children(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, with_keys: bool = True):
     """Batched leaf expansion (tg_expand_children): children[b, c] = slab[b] - rank1(tape[b, c]).
 
-    slab int8 or int16 (B, GP) (tg_expand_children_i16), tape uint8 (B, k, TP).  Returns (children (B, k, GP) of the
+    slab int8 or int16 (B, GP) (tg_expand_children_i16) or a bit slab (tg_expand_children_gf2), tape uint8 (B, k, TP).  Returns (children (B, k, GP) of the
     slab's dtype, flags (B, k), nnz (B, k), keys (B, k) or None).  Reference: act.py:266-275 get_child_states + the
     null / terminal / already-in-tree tests of extend_tree (act.py:177-195), for B states at once."""
     sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
-    lay = layout(S)
+    lay, gp = layout(S), _game_pitch(sfx, S)
     B = slab.shape[0]
-    if tape.dim() != 3 or tape.shape[0] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != lay.game_pitch:
-        raise TensorGameError(f"expected slab (B,{lay.game_pitch}) and tape (B,k,{lay.token_pitch})")
+    if tape.dim() != 3 or tape.shape[0] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != gp:
+        raise TensorGameError(f"expected slab (B,{gp}) and tape (B,k,{lay.token_pitch})")
     k = tape.shape[1]
     dev = slab.device
-    children = torch.empty((B, k, lay.game_pitch), dtype=slab.dtype, device=dev)
+    children = torch.empty((B, k, gp), dtype=slab.dtype, device=dev)
     flags = torch.empty((B, k), dtype=torch.uint8, device=dev)
     nnz = torch.empty((B, k), dtype=torch.int32, device=dev)
     keys = torch.empty((B, k), dtype=torch.int64, device=dev) if with_keys else None
@@ -239,14 +290,14 @@ def expand_children(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, 
 
 def rollout(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torch.Tensor | None = None):
     """Apply a step-major tape (K, B, TP) to every game, freezing solved games.
-    slab int8 or int16 (tg_rollout_i16).  Returns (out, flags, nnz, steps).  Reference: datasets.py:144-153,
+    slab int8, int16 (tg_rollout_i16) or a bit slab (tg_rollout_gf2).  Returns (out, flags, nnz, steps).  Reference: datasets.py:144-153,
     training.py:336-342, act.py:49."""
     sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
-    lay = layout(S)
+    lay, gp = layout(S), _game_pitch(sfx, S)
     B = slab.shape[0]
-    if tape.dim() != 3 or tape.shape[1] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != lay.game_pitch:
-        raise TensorGameError(f"expected slab (B,{lay.game_pitch}) and tape (K,B,{lay.token_pitch})")
+    if tape.dim() != 3 or tape.shape[1] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != gp:
+        raise TensorGameError(f"expected slab (B,{gp}) and tape (K,B,{lay.token_pitch})")
     K = tape.shape[0]
     out = torch.empty_like(slab) if out is None else out
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device)
@@ -257,14 +308,14 @@ def rollout(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: tor
 
 
 def replay(slab: torch.Tensor, tape: torch.Tensor, S: int, shift: int, out: torch.Tensor | None = None):
-    """All K actions of a step-major tape applied without freezing (datasets.py:144-153); slab int8 or int16
-    (tg_replay_i16).  Returns (out, flags, nnz)."""
+    """All K actions of a step-major tape applied without freezing (datasets.py:144-153); slab int8, int16
+    (tg_replay_i16) or a bit slab (tg_replay_gf2).  Returns (out, flags, nnz)."""
     sfx = _game_slab(slab)
     _need_cuda(tape, "tape", torch.uint8)
-    lay = layout(S)
+    lay, gp = layout(S), _game_pitch(sfx, S)
     B, K = slab.shape[0], tape.shape[0]
-    if tape.dim() != 3 or tape.shape[1] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != lay.game_pitch:
-        raise TensorGameError(f"expected slab (B,{lay.game_pitch}) and tape (K,B,{lay.token_pitch})")
+    if tape.dim() != 3 or tape.shape[1] != B or tape.shape[2] != lay.token_pitch or slab.shape[1] != gp:
+        raise TensorGameError(f"expected slab (B,{gp}) and tape (K,B,{lay.token_pitch})")
     out = torch.empty_like(slab) if out is None else out
     flags = torch.empty(B, dtype=torch.uint8, device=slab.device)
     nnz = torch.empty(B, dtype=torch.int32, device=slab.device)
@@ -494,7 +545,8 @@ class DemoStore:
 
 
 def slice_rank(slab: torch.Tensor, S: int) -> torch.Tensor:
-    """get_rank per game (utils.py:134-140) of an int8 or int16 slab (tg_slice_rank_i16): int32 (B,)."""
+    """get_rank per game (utils.py:134-140) of an int8 or int16 slab (tg_slice_rank_i16): int32 (B,).  Of a bit slab
+    (tg_slice_rank_gf2): the sum of the slices' ranks over GF(2)."""
     sfx = _game_slab(slab)
     ranks = torch.empty(slab.shape[0], dtype=torch.int32, device=slab.device)
     _call("tg_slice_rank" + sfx, (slab, ranks,), _p(slab), _p(ranks), slab.shape[0], S)
@@ -518,7 +570,8 @@ def episode_returns(final_slab: torch.Tensor, steps: torch.Tensor, S: int, max_l
 
 def state_keys(slab: torch.Tensor, S: int) -> torch.Tensor:
     """64-bit state keys (as int64 bit patterns), replacing utils.state_to_str dict keys.  An int16 slab
-    (tg_state_key_i16) gives the same key as an int8 slab of the same values."""
+    (tg_state_key_i16) gives the same key as an int8 slab of the same values, a bit slab (tg_state_key_gf2) the key of
+    its 0/1 values."""
     sfx = _game_slab(slab)
     keys = torch.empty(slab.shape[0], dtype=torch.int64, device=slab.device)
     _call("tg_state_key" + sfx, (slab, keys,), _p(slab), _p(keys), slab.shape[0], S)
