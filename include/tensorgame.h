@@ -25,6 +25,15 @@
  *   - return value: 0 on success, a negative TG_E_* code otherwise; nothing
  *     throws.  There is no CPU fallback: without a CUDA device every compute
  *     entry point returns TG_E_CUDA.
+ *   - argument rules of the game path (tg_step, tg_expand_children,
+ *     tg_rollout, tg_replay, tg_state_key, tg_slice_rank and the conversions,
+ *     for every slab format), checked in this order: a bad scalar (S, B < 0,
+ *     shift outside [1, 4], k < 1, K < 0) returns TG_E_ARG; an empty batch
+ *     (B == 0) returns TG_OK before any pointer is looked at; a null pointer
+ *     the call needs returns TG_E_ARG; a misaligned buffer returns TG_E_ARG.
+ *     Slabs of every format, tapes and tape_step_stride are 16-byte aligned,
+ *     float32 arrays 4-byte and int64 token arrays 8-byte aligned; flags, nnz,
+ *     steps, keys and ranks are naturally aligned arrays (not checked).
  *
  * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
  * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths).  The change of basis (K5) stays

@@ -1204,19 +1204,6 @@ __global__ void __launch_bounds__(256) state_key_kernel(const int8_t *__restrict
     }
 }
 
-} // namespace tg
-
-#define TG_SWITCH_S(S, ...) \
-    switch (S) {            \
-    case 4: { constexpr int kS = 4; __VA_ARGS__; } break;   \
-    case 9: { constexpr int kS = 9; __VA_ARGS__; } break;   \
-    case 16: { constexpr int kS = 16; __VA_ARGS__; } break; \
-    case 25: { constexpr int kS = 25; __VA_ARGS__; } break; \
-    default: return TG_E_ARG; \
-    }
-
-namespace tg {
-
 template <int S, bool P16, bool STG>
 static int launch_demo_sample_variant(unsigned grid, size_t smem, const uint8_t *tape, long long tape_step_stride, const int8_t *slab,
                                       long long N, int R, int dim_t, int replay_shift, const long long *idx, long long nb,
@@ -1308,13 +1295,14 @@ int tg_demo_sample(const uint8_t *tape, int64_t tape_step_stride, const int8_t *
     // 127 + R * cmax^3 fits an int16 lane
     const long long cmax = replay_shift > 8 - replay_shift ? replay_shift : 8 - replay_shift;
     const bool pack16 = replay_shift >= 0 && replay_shift <= 8 && 127 + (long long)R * cmax * cmax * cmax <= 32767;
-    TG_SWITCH_S(S, {
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
         const int rc = tg::launch_demo_sample<kS>(tape, tape_step_stride, slab, N, R, dim_t, replay_shift, (const long long *)idx, nb,
                                                   states, scalars, (long long *)actions, rewards, pack16, st);
         if (rc != TG_OK) return rc;
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 int tg_demo_sample_dm(const uint8_t *tape_dm, const void *targets, int targets_i16, int target_bound, int64_t N, int R, int S,
@@ -1417,31 +1405,28 @@ int tg_tape_to_demo_major(const uint8_t *tape, int64_t tape_step_stride, uint8_t
 }
 
 int tg_slice_rank(const int8_t *slab, int32_t *ranks, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab || !ranks) return TG_E_ARG;
+    if (const int rc = tg::check_pair(S, B, slab, 16, ranks, 1); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     TG_CUDA(cudaMemsetAsync(ranks, 0, (size_t)B * 4, st));
-    TG_SWITCH_S(S, {
-        constexpr int LG = kS;
-        const long long warps = (B * kS + (32 / LG) - 1) / (32 / LG);
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        const long long warps = (B * kS + (32 / kS) - 1) / (32 / kS);
         tg::slice_rank_kernel<kS><<<(unsigned)((warps * 32 + 127) / 128), 128, 0, st>>>(slab, ranks, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 int tg_state_key(const int8_t *slab, uint64_t *keys, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab || !keys) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_SWITCH_S(S, {
+    if (const int rc = tg::check_pair(S, B, slab, 16, keys, 1); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
         const long long tiles = (B + (256 / tg::Geo<kS>::WR) - 1) / (256 / tg::Geo<kS>::WR);
-        tg::state_key_kernel<kS><<<(unsigned)(tiles < 148 * 16 ? tiles : 148 * 16), 256, 0, st>>>(slab, (unsigned long long *)keys, B);
+        tg::state_key_kernel<kS><<<(unsigned)(tiles < 148 * 16 ? tiles : 148 * 16), 256, 0, (cudaStream_t)stream>>>(
+            slab, (unsigned long long *)keys, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 } // extern "C"

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/tensorgame.h"
 
 namespace tg {
@@ -51,6 +53,68 @@ inline int cuda_fail(cudaError_t e) {
         cudaError_t _e = (call);                       \
         if (_e != cudaSuccess) return tg::cuda_fail(_e); \
     } while (0)
+
+// multiprocessors of the current device (148 if the runtime cannot tell), cached per device
+int sm_count();
+
+// f(std::integral_constant<int, S>{}) for a game-path size, TG_E_ARG for any other S.  In f: constexpr int kS =
+// decltype(s)::value.  For the switches whose cases make the same call with only S changing; the switches that pick a
+// measured configuration per size stay written out.
+template <class F>
+int with_S(int S, F &&f) {
+    switch (S) {
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 9: return f(std::integral_constant<int, 9>{});
+    case 16: return f(std::integral_constant<int, 16>{});
+    case 25: return f(std::integral_constant<int, 25>{});
+    }
+    return TG_E_ARG;
+}
+
+// ---------------------------------------------------------------- argument rules of the game path
+// One function per shape of entry point, shared by the int8, int16 and bit-slab twins.  In order: the scalars (TG_E_ARG),
+// an empty batch (TG_OK, before any pointer is looked at), null pointers (TG_E_ARG), alignment (TG_E_ARG).  LAUNCH means
+// the arguments hold and there is work; the entry point goes on to launch.  It never leaves the library.
+constexpr int LAUNCH = 1;
+
+inline bool misaligned(const void *p, uintptr_t align) { return ((uintptr_t)p & (align - 1)) != 0; }
+
+// tg_step*: slab_in, slab_out and tape 16-byte aligned
+inline int check_step(int S, long long B, int shift, const void *in, const void *tape, const void *out, const void *flags,
+                      const void *nnz) {
+    if (!supported_S(S) || B < 0 || shift < 1 || shift > 4) return TG_E_ARG;
+    if (B == 0) return TG_OK;
+    if (!in || !tape || !out || !flags || !nnz) return TG_E_ARG;
+    if (misaligned(in, 16) || misaligned(out, 16) || misaligned(tape, 16)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_expand_children*: tg_step's rules with k >= 1 children per parent (keys may be NULL)
+inline int check_expand(int S, long long B, int k, int shift, const void *parents, const void *tape, const void *children,
+                        const void *flags, const void *nnz) {
+    if (k < 1) return TG_E_ARG;
+    return check_step(S, B, shift, parents, tape, children, flags, nnz);
+}
+
+// tg_rollout* (freeze: steps required) and tg_replay*: the tape only when K > 0; slabs, tape and step stride 16-byte aligned
+inline int check_rollout(int S, long long B, int K, int shift, const void *in, const void *tape, long long stride, const void *out,
+                         const void *flags, const void *nnz, const void *steps, bool freeze) {
+    if (!supported_S(S) || B < 0 || K < 0 || shift < 1 || shift > 4) return TG_E_ARG;
+    if (B == 0) return TG_OK;
+    if (!in || !out || !flags || !nnz || (freeze && !steps) || (K > 0 && !tape)) return TG_E_ARG;
+    if (misaligned(in, 16) || misaligned(out, 16) || misaligned(tape, 16) || (stride & 15)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// one source and one destination buffer per game (keys, ranks and the conversions), each aligned to its own boundary:
+// slabs and tapes 16, float32 values 4, int64 tokens 8, keys and ranks 1 (not checked)
+inline int check_pair(int S, long long B, const void *src, uintptr_t src_align, const void *dst, uintptr_t dst_align) {
+    if (!supported_S(S) || B < 0) return TG_E_ARG;
+    if (B == 0) return TG_OK;
+    if (!src || !dst) return TG_E_ARG;
+    if (misaligned(src, src_align) || misaligned(dst, dst_align)) return TG_E_ARG;
+    return LAUNCH;
+}
 
 // change of basis: set by a fast kernel on the games it leaves to the exact int32 kernel, which clears it
 constexpr uint8_t BASIS_REDO = 0x80;

@@ -95,56 +95,47 @@ static inline int grid_for(long long total, int block) {
 
 } // namespace tg
 
-#define TG_DISPATCH_S(S, CALL) \
-    switch (S) {               \
-    case 4: { constexpr int kS = 4; CALL; } break;   \
-    case 9: { constexpr int kS = 9; CALL; } break;   \
-    case 16: { constexpr int kS = 16; CALL; } break; \
-    case 25: { constexpr int kS = 25; CALL; } break; \
-    default: return TG_E_ARG;  \
-    }
-
 extern "C" {
 
 int tg_pack_f32(const float *src, int64_t src_stride, int8_t *slab, int64_t B, int S, int32_t *range_flag, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!src || !slab || ((uintptr_t)slab & 15) || ((uintptr_t)src & 3)) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_DISPATCH_S(S, (tg::pack_f32_kernel<kS><<<tg::grid_for(B * (tg::Geo<kS>::GP / 4), 256), 256, 0, st>>>(
-                         src, src_stride, reinterpret_cast<uint32_t *>(slab), B, range_flag)));
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, src, 4, slab, 16); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::pack_f32_kernel<kS><<<tg::grid_for(B * (tg::Geo<kS>::GP / 4), 256), 256, 0, (cudaStream_t)stream>>>(
+            src, src_stride, reinterpret_cast<uint32_t *>(slab), B, range_flag);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_expand_f32(const int8_t *slab, float *dst, int64_t dst_stride, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab || !dst || ((uintptr_t)slab & 15) || ((uintptr_t)dst & 3)) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_DISPATCH_S(S, (tg::expand_f32_kernel<kS><<<tg::grid_for(B * kS * tg::Geo<kS>::WR, 256), 256, 0, st>>>(slab, dst, dst_stride, B)));
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, slab, 16, dst, 4); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::expand_f32_kernel<kS><<<tg::grid_for(B * kS * tg::Geo<kS>::WR, 256), 256, 0, (cudaStream_t)stream>>>(slab, dst, dst_stride, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_pack_actions_i64(const int64_t *actions, uint8_t *tape, int64_t B, int S, int32_t *range_flag, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!actions || !tape) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_DISPATCH_S(S, (tg::pack_actions_kernel<kS><<<tg::grid_for(B * tg::Geo<kS>::TP, 256), 256, 0, st>>>(actions, tape, B, range_flag)));
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, actions, 8, tape, 16); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::pack_actions_kernel<kS><<<tg::grid_for(B * tg::Geo<kS>::TP, 256), 256, 0, (cudaStream_t)stream>>>(actions, tape, B, range_flag);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_unpack_actions_i64(const uint8_t *tape, int64_t *actions, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!actions || !tape) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_DISPATCH_S(S, (tg::unpack_actions_kernel<kS><<<tg::grid_for(B * 3 * kS, 256), 256, 0, st>>>(tape, actions, B)));
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, tape, 16, actions, 8); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::unpack_actions_kernel<kS><<<tg::grid_for(B * 3 * kS, 256), 256, 0, (cudaStream_t)stream>>>(tape, actions, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 } // extern "C"

@@ -310,10 +310,7 @@ static int launch_expand(const int8_t *parents, const uint8_t *tape, int k, int8
 
 extern "C" int tg_expand_children(const int8_t *parents, const uint8_t *tape, int k, int8_t *children, uint8_t *flags,
                                   int32_t *nnz, uint64_t *keys, int64_t B, int S, int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || k < 1 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!parents || !tape || !children || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)parents | (uintptr_t)tape | (uintptr_t)children) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_expand(S, B, k, shift, parents, tape, children, flags, nnz); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     switch (S) {
     case 4: {

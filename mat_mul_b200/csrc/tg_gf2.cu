@@ -449,16 +449,9 @@ __global__ void __launch_bounds__(256) unpack_gf2_kernel(const uint32_t *__restr
     }
 }
 
-int sm_count_gf2() {
-    int dev = 0, n = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0)
-        return 148;
-    return n;
-}
-
 // CTAs for n items of `per` per CTA, at most eight resident CTAs of 256 threads per SM (the kernels loop over the rest)
 unsigned grid_for(long long n, int per) {
-    const long long want = (n + per - 1) / per, cap = 8LL * sm_count_gf2();
+    const long long want = (n + per - 1) / per, cap = 8LL * sm_count();
     return (unsigned)(want < cap ? want : cap);
 }
 
@@ -489,35 +482,22 @@ int launch_rollout_gf2(const uint32_t *in, const uint8_t *tape, long long stride
 
 template <typename E>
 int pack_gf2_any(const E *slab, uint32_t *bits, int64_t B, int S, void *stream) {
-    if (!supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab || !bits) return TG_E_ARG;
-    if (((uintptr_t)slab | (uintptr_t)bits) & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (S) {
-#define TG_PACK(s) \
-    case s: pack_gf2_kernel<s, E><<<grid_for(B * (GeoB<s>::GB / 4), 256), 256, 0, st>>>(slab, bits, B * (GeoB<s>::GB / 4)); break;
-        TG_PACK(4) TG_PACK(9) TG_PACK(16) TG_PACK(25)
-#undef TG_PACK
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = check_pair(S, B, slab, 16, bits, 16); rc != LAUNCH) return rc;
+    return with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        pack_gf2_kernel<kS, E><<<grid_for(B * (GeoB<kS>::GB / 4), 256), 256, 0, (cudaStream_t)stream>>>(slab, bits, B * (GeoB<kS>::GB / 4));
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int rollout_gf2_dispatch(const uint32_t *in, const uint8_t *tape, int64_t stride, int K, uint32_t *out, uint8_t *flags, int32_t *nnz,
                          int32_t *steps, int64_t B, int S, int shift, int freeze, void *stream) {
-    if (!supported_S(S) || B < 0 || K < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!in || !out || !flags || !nnz || (freeze && !steps) || (K > 0 && !tape)) return TG_E_ARG;
-    if (((uintptr_t)in | (uintptr_t)out | (uintptr_t)tape | (uintptr_t)stride) & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (S) {
-    case 4: return launch_rollout_gf2<4>(in, tape, stride, K, out, flags, nnz, steps, B, shift, freeze, st);
-    case 9: return launch_rollout_gf2<9>(in, tape, stride, K, out, flags, nnz, steps, B, shift, freeze, st);
-    case 16: return launch_rollout_gf2<16>(in, tape, stride, K, out, flags, nnz, steps, B, shift, freeze, st);
-    case 25: return launch_rollout_gf2<25>(in, tape, stride, K, out, flags, nnz, steps, B, shift, freeze, st);
-    }
-    return TG_E_ARG;
+    const int rc = check_rollout(S, B, K, shift, in, tape, stride, out, flags, nnz, steps, freeze);
+    if (rc != LAUNCH) return rc;
+    return with_S(S, [&](auto s) {
+        return launch_rollout_gf2<decltype(s)::value>(in, tape, stride, K, out, flags, nnz, steps, B, shift, freeze, (cudaStream_t)stream);
+    });
 }
 
 } // namespace
@@ -540,53 +520,31 @@ int tg_pack_gf2_i16(const int16_t *slab16, uint32_t *bits, int64_t B, int S, voi
 }
 
 int tg_unpack_gf2(const uint32_t *bits, int8_t *slab, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!bits || !slab) return TG_E_ARG;
-    if (((uintptr_t)bits | (uintptr_t)slab) & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    uint32_t *o = reinterpret_cast<uint32_t *>(slab);
-    switch (S) {
-#define TG_UNPACK(s) \
-    case s: tg::unpack_gf2_kernel<s><<<tg::grid_for(B * (tg::Geo<s>::GP / 4), 256), 256, 0, st>>>(bits, o, B * (tg::Geo<s>::GP / 4)); break;
-        TG_UNPACK(4) TG_UNPACK(9) TG_UNPACK(16) TG_UNPACK(25)
-#undef TG_UNPACK
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, bits, 16, slab, 16); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::unpack_gf2_kernel<kS><<<tg::grid_for(B * (tg::Geo<kS>::GP / 4), 256), 256, 0, (cudaStream_t)stream>>>(
+            bits, reinterpret_cast<uint32_t *>(slab), B * (tg::Geo<kS>::GP / 4));
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_step_gf2(const uint32_t *bits_in, const uint8_t *tape, uint32_t *bits_out, uint8_t *flags, int32_t *nnz, int64_t B, int S,
                 int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!bits_in || !tape || !bits_out || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)bits_in | (uintptr_t)bits_out | (uintptr_t)tape) & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (S) {
-    case 4: return tg::launch_step_gf2<4>(bits_in, tape, 1, bits_out, flags, nnz, nullptr, B, shift, st);
-    case 9: return tg::launch_step_gf2<9>(bits_in, tape, 1, bits_out, flags, nnz, nullptr, B, shift, st);
-    case 16: return tg::launch_step_gf2<16>(bits_in, tape, 1, bits_out, flags, nnz, nullptr, B, shift, st);
-    case 25: return tg::launch_step_gf2<25>(bits_in, tape, 1, bits_out, flags, nnz, nullptr, B, shift, st);
-    }
-    return TG_E_ARG;
+    if (const int rc = tg::check_step(S, B, shift, bits_in, tape, bits_out, flags, nnz); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        return tg::launch_step_gf2<decltype(s)::value>(bits_in, tape, 1, bits_out, flags, nnz, nullptr, B, shift, (cudaStream_t)stream);
+    });
 }
 
 int tg_expand_children_gf2(const uint32_t *parents, const uint8_t *tape, int k, uint32_t *children, uint8_t *flags, int32_t *nnz,
                            uint64_t *keys, int64_t B, int S, int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || k < 1 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!parents || !tape || !children || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)parents | (uintptr_t)tape | (uintptr_t)children) & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
+    if (const int rc = tg::check_expand(S, B, k, shift, parents, tape, children, flags, nnz); rc != tg::LAUNCH) return rc;
     const long long N = (long long)B * k;
-    switch (S) {
-    case 4: return tg::launch_step_gf2<4>(parents, tape, k, children, flags, nnz, keys, N, shift, st);
-    case 9: return tg::launch_step_gf2<9>(parents, tape, k, children, flags, nnz, keys, N, shift, st);
-    case 16: return tg::launch_step_gf2<16>(parents, tape, k, children, flags, nnz, keys, N, shift, st);
-    case 25: return tg::launch_step_gf2<25>(parents, tape, k, children, flags, nnz, keys, N, shift, st);
-    }
-    return TG_E_ARG;
+    return tg::with_S(S, [&](auto s) {
+        return tg::launch_step_gf2<decltype(s)::value>(parents, tape, k, children, flags, nnz, keys, N, shift, (cudaStream_t)stream);
+    });
 }
 
 int tg_rollout_gf2(const uint32_t *bits_in, const uint8_t *tape, int64_t tape_step_stride, int K, uint32_t *bits_out, uint8_t *flags,
@@ -600,38 +558,25 @@ int tg_replay_gf2(const uint32_t *bits_in, const uint8_t *tape, int64_t tape_ste
 }
 
 int tg_state_key_gf2(const uint32_t *bits, uint64_t *keys, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!bits || !keys) return TG_E_ARG;
-    if ((uintptr_t)bits & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const uint4 *i4 = reinterpret_cast<const uint4 *>(bits);
-    unsigned long long *kp = reinterpret_cast<unsigned long long *>(keys);
-    switch (S) {
-#define TG_KEY(s) \
-    case s: tg::state_key_gf2_kernel<s><<<tg::grid_for(B, tg::GeoB<s>::GPC), 256, 0, st>>>(i4, kp, B); break;
-        TG_KEY(4) TG_KEY(9) TG_KEY(16) TG_KEY(25)
-#undef TG_KEY
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, bits, 16, keys, 1); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::state_key_gf2_kernel<kS><<<tg::grid_for(B, tg::GeoB<kS>::GPC), 256, 0, (cudaStream_t)stream>>>(
+            reinterpret_cast<const uint4 *>(bits), reinterpret_cast<unsigned long long *>(keys), B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_slice_rank_gf2(const uint32_t *bits, int32_t *ranks, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!bits || !ranks) return TG_E_ARG;
-    if ((uintptr_t)bits & 15) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    const uint4 *i4 = reinterpret_cast<const uint4 *>(bits);
-    switch (S) {
-#define TG_RANK(s) \
-    case s: tg::slice_rank_gf2_kernel<s><<<tg::grid_for(B, tg::GeoB<s>::GPC), 256, 0, st>>>(i4, ranks, B); break;
-        TG_RANK(4) TG_RANK(9) TG_RANK(16) TG_RANK(25)
-#undef TG_RANK
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_pair(S, B, bits, 16, ranks, 1); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::slice_rank_gf2_kernel<kS><<<tg::grid_for(B, tg::GeoB<kS>::GPC), 256, 0, (cudaStream_t)stream>>>(
+            reinterpret_cast<const uint4 *>(bits), ranks, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 } // extern "C"

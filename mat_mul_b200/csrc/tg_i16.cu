@@ -229,13 +229,6 @@ __global__ void __launch_bounds__(NT + 32)
     }
 }
 
-static int sm_count16() {
-    int dev = 0, n = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0)
-        return 148;
-    return n;
-}
-
 template <int S, int NT, int NPASS, int NSTAGE>
 static int launch_step16(const int16_t *slab_in, const uint8_t *tape, int16_t *slab_out, uint8_t *flags, int32_t *nnz, long long B,
                          int shift, cudaStream_t stream) {
@@ -243,7 +236,7 @@ static int launch_step16(const int16_t *slab_in, const uint8_t *tape, int16_t *s
     auto kern = step16_kernel<S, NT, NPASS, NSTAGE>;
     TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
     const long long ntiles = (B + C::TG - 1) / C::TG;
-    const long long cap = (long long)sm_count16() * 32;
+    const long long cap = (long long)sm_count() * 32;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
     kern<<<grid, C::THREADS, C::SMEM_BYTES, stream>>>(slab_in, tape, slab_out, flags, nnz, B, shift);
     TG_CUDA(cudaGetLastError());
@@ -683,10 +676,8 @@ __global__ void slice_rank16_kernel(const int16_t *__restrict__ slab, int32_t *_
 
 static int rollout16_dispatch(const int16_t *slab_in, const uint8_t *tape, int64_t tape_step_stride, int K, int16_t *slab_out,
                               uint8_t *flags, int32_t *nnz, int32_t *steps, int64_t B, int S, int shift, int freeze, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || K < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab_in || !slab_out || !flags || !nnz || (freeze && !steps) || (K > 0 && !tape)) return TG_E_ARG;
-    if (((uintptr_t)slab_in | (uintptr_t)slab_out | (uintptr_t)tape | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    const int rc = tg::check_rollout(S, B, K, shift, slab_in, tape, tape_step_stride, slab_out, flags, nnz, steps, freeze);
+    if (rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     switch (S) {
     case 4: return tg::launch_rollout16<4, 128>(slab_in, tape, tape_step_stride, K, slab_out, flags, nnz, steps, B, shift, freeze, st);
@@ -701,10 +692,7 @@ extern "C" {
 
 int tg_step_i16(const int16_t *slab_in, const uint8_t *tape, int16_t *slab_out, uint8_t *flags, int32_t *nnz, int64_t B, int S,
                 int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab_in || !tape || !slab_out || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)slab_in | (uintptr_t)slab_out | (uintptr_t)tape) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_step(S, B, shift, slab_in, tape, slab_out, flags, nnz); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // the int8 configurations' stage sizes (about 16-20 KB per stage, two stages), with half the games per stage
     switch (S) {
@@ -719,10 +707,7 @@ int tg_step_i16(const int16_t *slab_in, const uint8_t *tape, int16_t *slab_out, 
 
 int tg_expand_children_i16(const int16_t *parents, const uint8_t *tape, int k, int16_t *children, uint8_t *flags, int32_t *nnz,
                            uint64_t *keys, int64_t B, int S, int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || k < 1 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!parents || !tape || !children || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)parents | (uintptr_t)tape | (uintptr_t)children) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_expand(S, B, k, shift, parents, tape, children, flags, nnz); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long *kp = (unsigned long long *)keys;
     switch (S) {
@@ -745,10 +730,7 @@ int tg_replay_i16(const int16_t *slab_in, const uint8_t *tape, int64_t tape_step
 }
 
 int tg_state_key_i16(const int16_t *slab16, uint64_t *keys, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab16 || !keys) return TG_E_ARG;
-    if ((uintptr_t)slab16 & 15) return TG_E_ARG;
+    if (const int rc = tg::check_pair(S, B, slab16, 16, keys, 1); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     unsigned long long *kp = (unsigned long long *)keys;
     auto grid = [B](int tg_) { const long long t = (B + tg_ - 1) / tg_; return (unsigned)(t < 148 * 16 ? t : 148 * 16); };
@@ -764,22 +746,16 @@ int tg_state_key_i16(const int16_t *slab16, uint64_t *keys, int64_t B, int S, vo
 }
 
 int tg_slice_rank_i16(const int16_t *slab16, int32_t *ranks, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab16 || !ranks) return TG_E_ARG;
-    if ((uintptr_t)slab16 & 15) return TG_E_ARG;
+    if (const int rc = tg::check_pair(S, B, slab16, 16, ranks, 1); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     TG_CUDA(cudaMemsetAsync(ranks, 0, (size_t)B * 4, st));
-    auto blocks = [B](int s) { const long long warps = (B * s + (32 / s) - 1) / (32 / s); return (unsigned)((warps * 32 + 127) / 128); };
-    switch (S) {
-    case 4: tg::slice_rank16_kernel<4><<<blocks(4), 128, 0, st>>>(slab16, ranks, B); break;
-    case 9: tg::slice_rank16_kernel<9><<<blocks(9), 128, 0, st>>>(slab16, ranks, B); break;
-    case 16: tg::slice_rank16_kernel<16><<<blocks(16), 128, 0, st>>>(slab16, ranks, B); break;
-    case 25: tg::slice_rank16_kernel<25><<<blocks(25), 128, 0, st>>>(slab16, ranks, B); break;
-    default: return TG_E_ARG;
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        const long long warps = (B * kS + (32 / kS) - 1) / (32 / kS);
+        tg::slice_rank16_kernel<kS><<<(unsigned)((warps * 32 + 127) / 128), 128, 0, st>>>(slab16, ranks, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 } // extern "C"

@@ -323,10 +323,8 @@ static int launch_rollout(const int8_t *slab_in, const uint8_t *tape, long long 
 static int rollout_dispatch(const int8_t *slab_in, const uint8_t *tape, int64_t tape_step_stride, int K, int8_t *slab_out,
                             uint8_t *flags, int32_t *nnz, int32_t *steps, int64_t B, int S, int shift, int freeze,
                             void *stream) {
-    if (!tg::supported_S(S) || B < 0 || K < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab_in || !slab_out || !flags || !nnz || (freeze && !steps) || (K > 0 && !tape)) return TG_E_ARG;
-    if (((uintptr_t)slab_in | (uintptr_t)slab_out | (uintptr_t)tape | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    const int rc = tg::check_rollout(S, B, K, shift, slab_in, tape, tape_step_stride, slab_out, flags, nnz, steps, freeze);
+    if (rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     switch (S) {
     case 4: {

@@ -131,7 +131,7 @@ __global__ void __launch_bounds__(NT + 32)
 }
 
 // ---------------------------------------------------------------- host side
-static int sm_count() {
+int sm_count() {
     static int cached[64] = {0};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
@@ -205,10 +205,7 @@ int tg_tune_step_variant(int v) {
 
 int tg_step(const int8_t *slab_in, const uint8_t *tape, int8_t *slab_out, uint8_t *flags, int32_t *nnz, int64_t B, int S,
             int shift, void *stream) {
-    if (!tg::supported_S(S) || B < 0 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab_in || !tape || !slab_out || !flags || !nnz) return TG_E_ARG;
-    if (((uintptr_t)slab_in | (uintptr_t)slab_out | (uintptr_t)tape) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_step(S, B, shift, slab_in, tape, slab_out, flags, nnz); rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
 #ifdef TG_TUNING
     switch (S * 10 + tg::g_step_variant) { // sweep-only instantiations

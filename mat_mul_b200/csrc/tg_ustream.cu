@@ -223,22 +223,18 @@ int tg_demo_from_ustream(const double *u, int64_t n_u, const int8_t *values, con
         return TG_OK;
     }
     const int mb = (int)((n_tries + 127) / 128);
-    switch (S) {
-    case 4: tg::ustream_map_kernel<4><<<mb, 128, 0, st>>>(u, n_tries, cat, shift, tok, valid); break;
-    case 9: tg::ustream_map_kernel<9><<<mb, 128, 0, st>>>(u, n_tries, cat, shift, tok, valid); break;
-    case 16: tg::ustream_map_kernel<16><<<mb, 128, 0, st>>>(u, n_tries, cat, shift, tok, valid); break;
-    case 25: tg::ustream_map_kernel<25><<<mb, 128, 0, st>>>(u, n_tries, cat, shift, tok, valid); break;
-    }
-    TG_CUDA(cudaGetLastError());
-    tg::scan_block_sums_kernel<<<nb, tg::SCAN_BLOCK, 0, st>>>(valid, n_tries, sums);
-    tg::scan_sums_kernel<<<1, tg::SCAN_BLOCK, 0, st>>>(sums, nb);
-    switch (S) {
-    case 4: tg::ustream_scatter_kernel<4><<<nb, tg::SCAN_BLOCK, 0, st>>>(tok, valid, sums, n_tries, nb, R, N, tape, tape_step_stride, (long long *)result); break;
-    case 9: tg::ustream_scatter_kernel<9><<<nb, tg::SCAN_BLOCK, 0, st>>>(tok, valid, sums, n_tries, nb, R, N, tape, tape_step_stride, (long long *)result); break;
-    case 16: tg::ustream_scatter_kernel<16><<<nb, tg::SCAN_BLOCK, 0, st>>>(tok, valid, sums, n_tries, nb, R, N, tape, tape_step_stride, (long long *)result); break;
-    case 25: tg::ustream_scatter_kernel<25><<<nb, tg::SCAN_BLOCK, 0, st>>>(tok, valid, sums, n_tries, nb, R, N, tape, tape_step_stride, (long long *)result); break;
-    }
-    TG_CUDA(cudaGetLastError());
+    const int rc = tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::ustream_map_kernel<kS><<<mb, 128, 0, st>>>(u, n_tries, cat, shift, tok, valid);
+        TG_CUDA(cudaGetLastError());
+        tg::scan_block_sums_kernel<<<nb, tg::SCAN_BLOCK, 0, st>>>(valid, n_tries, sums);
+        tg::scan_sums_kernel<<<1, tg::SCAN_BLOCK, 0, st>>>(sums, nb);
+        tg::ustream_scatter_kernel<kS><<<nb, tg::SCAN_BLOCK, 0, st>>>(tok, valid, sums, n_tries, nb, R, N, tape, tape_step_stride,
+                                                                     (long long *)result);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
+    if (rc != TG_OK) return rc;
     return tg_demo_accumulate(tape, tape_step_stride, N, R, S, shift, slab, flags, stream);
 }
 

@@ -138,15 +138,6 @@ __global__ void pack_f32_i16_kernel(const float *__restrict__ src, long long src
 
 } // namespace tg
 
-#define TG_SWITCH_S(S, ...)                                 \
-    switch (S) {                                            \
-    case 4: { constexpr int kS = 4; __VA_ARGS__; } break;   \
-    case 9: { constexpr int kS = 9; __VA_ARGS__; } break;   \
-    case 16: { constexpr int kS = 16; __VA_ARGS__; } break; \
-    case 25: { constexpr int kS = 25; __VA_ARGS__; } break; \
-    default: return TG_E_ARG;                               \
-    }
-
 extern "C" {
 
 int tg_demo_accumulate_i16(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift, int16_t *slab16,
@@ -159,48 +150,47 @@ int tg_demo_accumulate_i16(const uint8_t *tape, int64_t tape_step_stride, int64_
     const long long cmax = shift > 255 - shift ? shift : 255 - shift;
     if ((long long)R * cmax * cmax * cmax > 0x7FFFFFFFLL) {
         if (flags) TG_CUDA(cudaMemsetAsync(flags, 0, (size_t)N, st));
-        TG_SWITCH_S(S, {
+        return tg::with_S(S, [&](auto s) {
+            constexpr int kS = decltype(s)::value;
             const long long blocks = (N * tg::Geo<kS>::GP + 255) / 256;
             tg::demo_accumulate_i16_wide_kernel<kS><<<(unsigned)(blocks < 148 * 32 ? blocks : 148 * 32), 256, 0, st>>>(
                 tape, tape_step_stride, N, R, shift, slab16, flags);
+            TG_CUDA(cudaGetLastError());
+            return TG_OK;
         });
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
     }
-    TG_SWITCH_S(S, {
-        constexpr int DPC = 256 / tg::Geo<kS>::WR;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value, DPC = 256 / tg::Geo<kS>::WR;
         const long long grid = (N + DPC - 1) / DPC;
         if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
         tg::demo_accumulate_i16_kernel<kS><<<(unsigned)grid, 256, 0, st>>>(tape, tape_step_stride, N, R, shift, slab16, flags);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 int tg_expand_f32_i16(const int16_t *slab16, float *dst, int64_t dst_stride, int64_t B, int S, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!slab16 || !dst) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_SWITCH_S(S, {
+    if (const int rc = tg::check_pair(S, B, slab16, 16, dst, 4); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
         const long long blocks = (B * tg::Geo<kS>::S3 + 255) / 256;
-        tg::expand_f32_i16_kernel<kS><<<(unsigned)(blocks < 148 * 64 ? blocks : 148 * 64), 256, 0, st>>>(slab16, dst, dst_stride, B);
+        tg::expand_f32_i16_kernel<kS><<<(unsigned)(blocks < 148 * 64 ? blocks : 148 * 64), 256, 0, (cudaStream_t)stream>>>(
+            slab16, dst, dst_stride, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 int tg_pack_f32_i16(const float *src, int64_t src_stride, int16_t *slab16, int64_t B, int S, int32_t *range_flag, void *stream) {
-    if (!tg::supported_S(S) || B < 0) return TG_E_ARG;
-    if (B == 0) return TG_OK;
-    if (!src || !slab16) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
-    TG_SWITCH_S(S, {
+    if (const int rc = tg::check_pair(S, B, src, 4, slab16, 16); rc != tg::LAUNCH) return rc;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
         const long long blocks = (B * tg::Geo<kS>::GP + 255) / 256;
-        tg::pack_f32_i16_kernel<kS><<<(unsigned)(blocks < 148 * 64 ? blocks : 148 * 64), 256, 0, st>>>(src, src_stride, slab16, B, range_flag);
+        tg::pack_f32_i16_kernel<kS><<<(unsigned)(blocks < 148 * 64 ? blocks : 148 * 64), 256, 0, (cudaStream_t)stream>>>(
+            src, src_stride, slab16, B, range_flag);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
     });
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
 }
 
 } // extern "C"

@@ -27,14 +27,6 @@ def test_layout_contract():
     assert L.tg_error_string(-1) == b"bad argument"
 
 
-def test_argument_validation_without_gpu():
-    L = _lib.lib()
-    assert L.tg_step(None, None, None, None, None, 0, 9, 2, None) == 0  # empty batch is a no-op
-    assert L.tg_step(None, None, None, None, None, 4, 9, 2, None) == -1  # null pointers
-    assert L.tg_step(None, None, None, None, None, 4, 7, 2, None) == -1  # unsupported S
-    assert L.tg_step(None, None, None, None, None, 4, 9, 9, None) == -1  # shift out of [1,4]
-
-
 def test_no_cpu_fallback():
     import torch
 

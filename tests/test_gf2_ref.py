@@ -1,5 +1,5 @@
 """CPU checks of the mod-2 game path's reference (tests/gf2_ref.py), pinned against the C oracle (the integer game taken
-mod 2) and against independent rank computations, and of the argument validation of every tg_*_gf2 entry point."""
+mod 2) and against independent rank computations (argument rules: tests/test_cabi_args.py)."""
 import ctypes as C
 import itertools
 
@@ -125,55 +125,3 @@ def test_slice_ranks_of_the_matmul_tensors():
         T = orc.build_matmul_tensor(n)[None]
         # slice i = (a, b) of A: the n x n^2 block pattern has rank n over any field
         assert ref.slice_ranks(T)[0] == n ** 2 * n
-
-
-def test_gf2_argument_validation_without_gpu():
-    L = _lib.lib()
-    n = None
-    for S in SIZES:
-        assert L.tg_step_gf2(n, n, n, n, n, 0, S, 2, n) == 0  # empty batch is a no-op
-        assert L.tg_step_gf2(n, n, n, n, n, 4, S, 2, n) == -1  # null pointers
-        assert L.tg_expand_children_gf2(n, n, 3, n, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_rollout_gf2(n, n, 0, 2, n, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_replay_gf2(n, n, 0, 2, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_state_key_gf2(n, n, 4, S, n) == -1
-        assert L.tg_slice_rank_gf2(n, n, 4, S, n) == -1
-        assert L.tg_pack_gf2(n, n, 4, S, n) == -1
-        assert L.tg_pack_gf2_i16(n, n, 4, S, n) == -1
-        assert L.tg_unpack_gf2(n, n, 4, S, n) == -1
-        for f in (L.tg_pack_gf2, L.tg_pack_gf2_i16, L.tg_unpack_gf2, L.tg_state_key_gf2, L.tg_slice_rank_gf2):
-            assert f(n, n, 0, S, n) == 0
-    fake = C.c_void_p(1 << 20)  # never dereferenced: every call below fails its checks first
-    odd = C.c_void_p((1 << 20) + 8)
-    for S in (5, 7, 36):  # unsupported sizes
-        assert L.tg_step_gf2(fake, fake, fake, fake, fake, 4, S, 2, n) == -1
-        assert L.tg_expand_children_gf2(fake, fake, 2, fake, fake, fake, n, 4, S, 2, n) == -1
-        assert L.tg_rollout_gf2(fake, fake, 32, 2, fake, fake, fake, fake, 4, S, 2, n) == -1
-        assert L.tg_replay_gf2(fake, fake, 32, 2, fake, fake, fake, 4, S, 2, n) == -1
-        assert L.tg_state_key_gf2(fake, fake, 4, S, n) == -1
-        assert L.tg_slice_rank_gf2(fake, fake, 4, S, n) == -1
-        assert L.tg_pack_gf2(fake, fake, 4, S, n) == -1
-        assert L.tg_pack_gf2_i16(fake, fake, 4, S, n) == -1
-        assert L.tg_unpack_gf2(fake, fake, 4, S, n) == -1
-    assert L.tg_step_gf2(fake, fake, fake, fake, fake, 4, 9, 0, n) == -1  # shift out of [1, 4]
-    assert L.tg_step_gf2(fake, fake, fake, fake, fake, 4, 9, 5, n) == -1
-    assert L.tg_step_gf2(fake, fake, fake, fake, fake, -1, 9, 2, n) == -1
-    assert L.tg_step_gf2(odd, fake, fake, fake, fake, 4, 9, 2, n) == -1   # misaligned pointers
-    assert L.tg_step_gf2(fake, odd, fake, fake, fake, 4, 9, 2, n) == -1
-    assert L.tg_step_gf2(fake, fake, odd, fake, fake, 4, 9, 2, n) == -1
-    assert L.tg_expand_children_gf2(fake, fake, 0, fake, fake, fake, n, 4, 9, 2, n) == -1  # k < 1
-    assert L.tg_expand_children_gf2(fake, odd, 3, fake, fake, fake, n, 4, 9, 2, n) == -1
-    assert L.tg_expand_children_gf2(fake, fake, 3, odd, fake, fake, n, 4, 9, 2, n) == -1
-    assert L.tg_expand_children_gf2(fake, fake, 3, fake, fake, fake, n, 4, 16, 9, n) == -1
-    assert L.tg_rollout_gf2(fake, fake, 8, 2, fake, fake, fake, fake, 4, 9, 2, n) == -1  # misaligned step stride
-    assert L.tg_rollout_gf2(odd, fake, 32, 2, fake, fake, fake, fake, 4, 9, 2, n) == -1
-    assert L.tg_rollout_gf2(fake, fake, 32, 2, fake, fake, fake, n, 4, 9, 2, n) == -1    # rollout needs steps
-    assert L.tg_rollout_gf2(fake, fake, 32, -1, fake, fake, fake, fake, 4, 9, 2, n) == -1
-    assert L.tg_replay_gf2(fake, fake, 32, 2, fake, fake, fake, 4, 25, 0, n) == -1
-    assert L.tg_replay_gf2(fake, fake, 32, 2, odd, fake, fake, 4, 25, 1, n) == -1
-    assert L.tg_state_key_gf2(odd, fake, 4, 9, n) == -1
-    assert L.tg_slice_rank_gf2(fake, fake, -1, 9, n) == -1
-    assert L.tg_slice_rank_gf2(odd, fake, 4, 9, n) == -1
-    assert L.tg_pack_gf2(odd, fake, 4, 9, n) == -1 and L.tg_pack_gf2(fake, odd, 4, 9, n) == -1
-    assert L.tg_pack_gf2_i16(odd, fake, 4, 9, n) == -1
-    assert L.tg_unpack_gf2(odd, fake, 4, 9, n) == -1 and L.tg_unpack_gf2(fake, odd, 4, 9, n) == -1

@@ -1,12 +1,8 @@
-"""CPU checks of the int16 game path's references (tests/i16_ref.py) and of the six tg_*_i16 entry points' argument
-validation.  The references are pinned against the C oracle on int8-zone inputs, where the int8 and int16 contracts
-coincide."""
-import ctypes as C
-
+"""CPU checks of the int16 game path's references (tests/i16_ref.py).  The references are pinned against the C oracle on
+int8-zone inputs, where the int8 and int16 contracts coincide (argument rules: tests/test_cabi_args.py)."""
 import numpy as np
 import pytest
 
-from mat_mul_b200 import _lib
 from oracle import tg_oracle as orc
 from tests import i16_ref as ref
 from tests.test_edges_ref import det_int, rank_int, slice_ranks
@@ -111,33 +107,3 @@ def test_slab16_round_trip():
         T = rng.integers(-32768, 32768, size=(3, S, S, S))
         slab = ref.dense_to_slab16(T)
         assert slab.shape == (3, ref.geo(S)[1]) and np.array_equal(ref.slab16_to_dense(slab, S), T)
-
-
-def test_i16_argument_validation_without_gpu():
-    L = _lib.lib()
-    n = None
-    for S in (4, 9, 16, 25):
-        assert L.tg_step_i16(n, n, n, n, n, 0, S, 2, n) == 0  # empty batch is a no-op
-        assert L.tg_step_i16(n, n, n, n, n, 4, S, 2, n) == -1  # null pointers
-        assert L.tg_expand_children_i16(n, n, 3, n, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_rollout_i16(n, n, 0, 2, n, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_replay_i16(n, n, 0, 2, n, n, n, 4, S, 2, n) == -1
-        assert L.tg_state_key_i16(n, n, 4, S, n) == -1
-        assert L.tg_slice_rank_i16(n, n, 4, S, n) == -1
-    fake = C.c_void_p(1 << 20)  # never dereferenced: every call below fails its checks first
-    odd = C.c_void_p((1 << 20) + 8)
-    assert L.tg_step_i16(fake, fake, fake, fake, fake, 4, 7, 2, n) == -1  # unsupported S
-    assert L.tg_step_i16(fake, fake, fake, fake, fake, 4, 9, 0, n) == -1  # shift out of [1, 4]
-    assert L.tg_step_i16(fake, fake, fake, fake, fake, 4, 9, 5, n) == -1
-    assert L.tg_step_i16(odd, fake, fake, fake, fake, 4, 9, 2, n) == -1   # misaligned slab
-    assert L.tg_expand_children_i16(fake, fake, 0, fake, fake, fake, n, 4, 9, 2, n) == -1  # k < 1
-    assert L.tg_expand_children_i16(fake, odd, 3, fake, fake, fake, n, 4, 9, 2, n) == -1
-    assert L.tg_expand_children_i16(fake, fake, 3, fake, fake, fake, n, 4, 16, 9, n) == -1
-    assert L.tg_rollout_i16(fake, fake, 8, 2, fake, fake, fake, fake, 4, 9, 2, n) == -1  # misaligned step stride
-    assert L.tg_rollout_i16(fake, fake, 32, 2, fake, fake, fake, n, 4, 9, 2, n) == -1    # rollout needs steps
-    assert L.tg_rollout_i16(fake, fake, 32, -1, fake, fake, fake, fake, 4, 9, 2, n) == -1
-    assert L.tg_replay_i16(fake, fake, 32, 2, fake, fake, fake, 4, 25, 0, n) == -1
-    assert L.tg_state_key_i16(fake, fake, 4, 5, n) == -1
-    assert L.tg_state_key_i16(odd, fake, 4, 9, n) == -1
-    assert L.tg_slice_rank_i16(fake, fake, -1, 9, n) == -1
-    assert L.tg_slice_rank_i16(fake, fake, 4, 8, n) == -1
