@@ -36,8 +36,8 @@
  *     steps, keys and ranks are naturally aligned arrays (not checked).
  *
  * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
- * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths).  The change of basis (K5) stays
- * {4, 9, 16} and tg_demo_accumulate_tc 16; at 25 tg_demo_gen_philox keeps
+ * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths, and the change of basis mod 2).  The
+ * change of basis over Z (K5) stays {4, 9, 16} and tg_demo_accumulate_tc 16; at 25 tg_demo_gen_philox keeps
  * contract v1 for every alphabet (tg_demo_alias_tables returns TG_E_ARG).
  *
  * Device formats (see DESIGN.md "Data layout")
@@ -69,7 +69,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 202
+#define TG_VERSION 203
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -315,6 +315,32 @@ int tg_replay_gf2(const uint32_t *bits_in, const uint8_t *tape, int64_t tape_ste
                   int32_t *nnz, int64_t B, int S, int shift, void *stream);
 int tg_state_key_gf2(const uint32_t *bits, uint64_t *keys, int64_t B, int S, void *stream);
 int tg_slice_rank_gf2(const uint32_t *bits, int32_t *ranks, int64_t B, int S, void *stream);
+
+/* ---- change of basis mod 2: K5 over GF(2) on bit slabs (S in {4, 9, 16, 25}) -------------------------------------- */
+/* The AlphaTensor augmentation of the game over Z_2: T'[i][j][k] = sum_abc A[i][a] B[j][b] C[k][c] T[a][b][c] mod 2 with
+ * (A, B, C) invertible over GF(2), and the factors u' = A u, v' = B v, w' = C w of the same basis, so that a transformed
+ * tape still sums to the transformed tensor.
+ *   mats  uint32 [N or 1][3][S]  a triple (A, B, C) mod 2: word r of matrix f is row r, bit c is M[r][c] mod 2; bits S to
+ *                          31 are ignored.  4-byte aligned; per_game != 0: one triple per game, otherwise one shared triple.
+ *                          In torch an int32 tensor (N, 3, S).
+ * Over GF(2) no entry and no token can leave its format, so none of the three takes a flags array.  Argument rules as on
+ * the game path: a bad scalar (S, N < 0, R < 1, shift_in or shift_out outside [1, 4], p_nonzero outside [0, 1] or NaN)
+ * returns TG_E_ARG; N == 0 returns TG_OK; a null pointer returns TG_E_ARG; bit slabs, tapes and step strides must be
+ * 16-byte aligned and mats 4-byte aligned (TG_E_ARG). */
+/* T' = T x1 A x2 B x3 C over GF(2); in place allowed; padding bits and words of the output zero */
+int tg_change_of_basis_gf2(const uint32_t *bits_in, const uint32_t *mats, int per_game, uint32_t *bits_out, int64_t N, int S,
+                           void *stream);
+/* u' = A u, v' = B v, w' = C w over GF(2) for every record of a step-major tape uint8 [R][N][TP]: the residue of token t
+ * is (t - shift_in) & 1, the output token is residue' + shift_out, padding bytes zero; in place allowed */
+int tg_change_of_basis_factors_gf2(const uint8_t *tape_in, int64_t in_step_stride, int shift_in, const uint32_t *mats,
+                                   int per_game, uint8_t *tape_out, int64_t out_step_stride, int shift_out, int64_t N, int R,
+                                   int S, void *stream);
+/* (A, B, C) per game, each L*U mod 2 and so invertible over GF(2) -> uint32 [N][3][S].  The draws of
+ * tg_sample_unimodular (Philox ctr = (block, f, 0x6D617473, d_lo), the demo-stream key of (seed, d = first + n)): L[r][c]
+ * = 1 below the diagonal and U[r][c] = 1 above it where the low 7 bits of the draw byte are below floor(128 p_nonzero),
+ * both diagonals 1.  At S <= 16 the result is tg_sample_unimodular of the same arguments mod 2; at 25 the same recipe
+ * reads 40 Philox blocks per matrix. */
+int tg_sample_invertible_gf2(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, uint32_t *mats, void *stream);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

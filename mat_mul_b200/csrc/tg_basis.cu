@@ -607,18 +607,6 @@ __global__ void __launch_bounds__(252)
     }
 }
 
-__device__ __forceinline__ void philox_block(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
-                                             uint32_t out[4]) {
-#pragma unroll
-    for (int r = 0; r < 10; r++) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        c0 = hi1 ^ c1 ^ k0, c1 = lo1, c2 = hi0 ^ c3 ^ k1, c3 = lo0;
-        k0 += 0x9E3779B9u, k1 += 0xBB67AE85u;
-    }
-    out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
-}
-
 // one thread per (game, matrix): M = L * U, L unit-lower, U upper with diagonal +-1, off-diagonal entries
 // -1/0/+1 with probabilities (p_nz/2, 1-p_nz, p_nz/2).  Draw for entry (r,c): byte (r*S+c)%16 of Philox block
 // (r*S+c)/16 with ctr = (block, matrix f, 0x6D617473, d_lo), key as in the unimodular contract of the oracle.

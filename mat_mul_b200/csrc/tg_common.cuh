@@ -116,6 +116,34 @@ inline int check_pair(int S, long long B, const void *src, uintptr_t src_align, 
     return LAUNCH;
 }
 
+// tg_change_of_basis_gf2: bit slabs 16-byte aligned, the uint32 matrix rows 4-byte aligned
+inline int check_basis_gf2(int S, long long N, const void *in, const void *mats, const void *out) {
+    if (!supported_S(S) || N < 0) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!in || !mats || !out) return TG_E_ARG;
+    if (misaligned(in, 16) || misaligned(out, 16) || misaligned(mats, 4)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_change_of_basis_factors_gf2: both shifts in [1, 4], R >= 1; tapes and step strides 16-byte aligned, matrices 4
+inline int check_basis_factors_gf2(int S, long long N, int R, int shift_in, int shift_out, const void *tape_in, long long in_stride,
+                                   const void *mats, const void *tape_out, long long out_stride) {
+    if (!supported_S(S) || N < 0 || R < 1 || shift_in < 1 || shift_in > 4 || shift_out < 1 || shift_out > 4) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!tape_in || !mats || !tape_out) return TG_E_ARG;
+    if (misaligned(tape_in, 16) || misaligned(tape_out, 16) || (in_stride & 15) || (out_stride & 15) || misaligned(mats, 4)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_sample_invertible_gf2: p_nonzero in [0, 1] (NaN refused), matrices 4-byte aligned
+inline int check_sample_gf2(int S, long long N, double p_nonzero, const void *mats) {
+    if (!supported_S(S) || N < 0 || !(p_nonzero >= 0.0 && p_nonzero <= 1.0)) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!mats) return TG_E_ARG;
+    if (misaligned(mats, 4)) return TG_E_ARG;
+    return LAUNCH;
+}
+
 // change of basis: set by a fast kernel on the games it leaves to the exact int32 kernel, which clears it
 constexpr uint8_t BASIS_REDO = 0x80;
 // tg_basis_mma.cu: 16x16x16 games, one warp per game on mma.sync int8 + f16; tg_basis_mma9.cu: 9x9x9 games on mma.sync f16.
@@ -132,6 +160,19 @@ int launch_rollout_rows(const int8_t *slab_in, const uint8_t *tape, long long st
 bool demo_acc16_mma_applies(int R);
 int launch_demo_acc16_mma(const uint8_t *tape, long long tape_step_stride, long long N, int R, int shift, int8_t *slab,
                           uint8_t *flags, int or_flags, cudaStream_t st);
+
+// Philox4x32-10 (oracle/tg_oracle.c orc_philox4x32_10): the block of counter (c0, c1, c2, c3) under key (k0, k1)
+__device__ __forceinline__ void philox_block(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
+                                             uint32_t out[4]) {
+#pragma unroll
+    for (int r = 0; r < 10; r++) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0, c1 = lo1, c2 = hi0 ^ c3 ^ k1, c3 = lo0;
+        k0 += 0x9E3779B9u, k1 += 0xBB67AE85u;
+    }
+    out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
+}
 
 // ---------------------------------------------------------------- PTX: mbarrier + bulk async copy (TMA 1-D)
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }

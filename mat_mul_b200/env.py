@@ -630,6 +630,56 @@ def change_of_basis(slab: torch.Tensor, mats: torch.Tensor, S: int, tape: torch.
     return (out, tape_out, flags, stats) if return_path_stats else (out, tape_out, flags)
 
 
+# ---------------------------------------------------------------- K5 mod 2
+def sample_invertible_gf2(n: int, S: int, seed: int = 0, first: int = 0, p_nonzero: float = 0.3, device="cuda") -> torch.Tensor:
+    """Random (A, B, C) per game, each invertible over GF(2), as bit matrices int32 (n, 3, S): word r of a matrix is its
+    row r, bit c its entry (r, c) (tg_sample_invertible_gf2).  At S <= 16 these are sample_unimodular(n, S, seed, first,
+    p_nonzero) mod 2."""
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise TensorGameError("sample_invertible_gf2 needs a CUDA device (there is no CPU path)")
+    mats = torch.empty((n, 3, S), dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _call("tg_sample_invertible_gf2", (mats,), seed, first, n, S, float(p_nonzero), _p(mats))
+    return mats
+
+
+def change_of_basis_gf2(bits: torch.Tensor, mats: torch.Tensor, S: int, tape: torch.Tensor | None = None, shift: int = 1,
+                        shift_out: int | None = None, out: torch.Tensor | None = None):
+    """T' = T x1 A x2 B x3 C over GF(2) on a bit slab (tg_change_of_basis_gf2), and u' = A u, v' = B v, w' = C w mod 2
+    for a step-major tape (R, N, TP) (tg_change_of_basis_factors_gf2: tokens read with `shift`, written as residue +
+    shift_out, default shift).  mats: bit matrices int32 (N, 3, S) per game, or (1, 3, S) / (3, S) shared.  out may be
+    bits (in place).  Returns bits', or (bits', tape') when a tape is given.  Nothing can leave the format mod 2, so there
+    are no flags.  Not in the reference: AlphaTensor paper, Methods "Change of basis", in modular arithmetic."""
+    _need_cuda(bits, "bits", torch.int32)
+    _need_cuda(mats, "mats", torch.int32)
+    gw = layout_gf2(S).game_words
+    N = bits.shape[0]
+    if bits.shape != (N, gw):
+        raise TensorGameError(f"expected bits (N,{gw})")
+    m = mats.reshape(-1, 3, S)
+    if m.shape[0] not in (1, N):
+        raise TensorGameError("mats must hold one (A,B,C) triple or one per game")
+    per_game = int(m.shape[0] == N and N > 1)
+    out = torch.empty_like(bits) if out is None else out
+    _need_cuda(out, "out", torch.int32)
+    if out.shape != bits.shape:
+        raise TensorGameError("out must be a bit slab of the input's shape")
+    _call("tg_change_of_basis_gf2", (bits, m, out), _p(bits), _p(m), per_game, _p(out), N, S)
+    if tape is None:
+        return out
+    _need_cuda(tape, "tape", torch.uint8)
+    tp = layout(S).token_pitch
+    if tape.dim() != 3 or tape.shape[1:] != (N, tp):
+        raise TensorGameError(f"tape must be (R, N, {tp})")
+    tape_out = torch.empty_like(tape)
+    if tape.shape[0] == 0:
+        return out, tape_out
+    _call("tg_change_of_basis_factors_gf2", (tape, m, tape_out), _p(tape), N * tp, shift, _p(m), per_game, _p(tape_out), N * tp,
+          shift if shift_out is None else shift_out, N, tape.shape[0], S)
+    return out, tape_out
+
+
 def bind_host_to_gpu(device: int = 0) -> list[int]:
     """Pin the calling process to the CPU cores that are local to GPU `device` (NVML cpu affinity), so that the
     pinned host buffers it allocates next are first-touched on that GPU's NUMA node.  Matters for the host-buffer
