@@ -69,7 +69,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 203
+#define TG_VERSION 204
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -341,6 +341,29 @@ int tg_change_of_basis_factors_gf2(const uint8_t *tape_in, int64_t in_step_strid
  * both diagonals 1.  At S <= 16 the result is tg_sample_unimodular of the same arguments mod 2; at 25 the same recipe
  * reads 40 Philox blocks per matrix. */
 int tg_sample_invertible_gf2(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, uint32_t *mats, void *stream);
+
+/* ---- mod-2 training samples: K4 and the float32 conversion on bit slabs (S in {4, 9, 16, 25}) ---------------------- */
+/* SyntheticDemoDataset.__getitem__ (datasets.py:77-122) modulo 2, from a demo-major store with bit-slab targets: the
+ * arguments of tg_demo_sample_dm without targets_i16 and target_bound, the targets a bit slab [N][GB/4].  The records are
+ * tg_demo_sample_dm's uint8 [N][R][TP]; token t has residue (t - replay_shift) & 1, replay_shift in [0, 8].  With
+ * idx[b] = d*R + a and term(r) = (u mod 2) (x) (v mod 2) (x) (w mod 2) of record r of demo d:
+ *   - slot 0 of states[b] = target_d xor term(a+1) xor ... xor term(R-1) (the target as given, so a target transformed
+ *     by tg_change_of_basis_gf2 works too);
+ *   - slot t, 1 <= t < dim_t, = term(hi - t) with hi = min(a + dim_t, R), zero where hi - t <= a;
+ *   - entries 0.0f or 1.0f, dense (dim_t, S, S, S) per sample; states may start at any float;
+ *   - scalars = R - a, actions = the record's 3S tokens as int64, rewards = -(a+1), as tg_demo_sample_dm writes them;
+ *   - an index outside [0, N*R) gets all-zero states, its other outputs untouched.
+ * Checks in tg_demo_sample_dm's order: a bad scalar (S, N < 0, R < 1, dim_t < 1, nb < 0) returns TG_E_ARG; nb == 0
+ * returns TG_OK; a null pointer returns TG_E_ARG; tape_dm and the targets must be 16-byte aligned (TG_E_ARG); then
+ * replay_shift outside [0, 8] returns TG_E_ARG.  Records are read from the store as they are replayed, so R has no upper
+ * bound. */
+int tg_demo_sample_gf2(const uint8_t *tape_dm, const uint32_t *targets_bits, int64_t N, int R, int S, int dim_t,
+                       int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
+                       float *rewards, void *stream);
+/* bit slab -> float32 dense (S,S,S) of 0.0f / 1.0f at dst + b*dst_stride: the state the model consumes;
+ * tg_expand_f32(tg_unpack_gf2(bits)) in one pass.  The game path's argument rules (bits 16-byte aligned, dst 4-byte);
+ * dst may start at any float, and floats outside each game's S^3 are not written. */
+int tg_expand_f32_gf2(const uint32_t *bits, float *dst, int64_t dst_stride, int64_t B, int S, void *stream);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

@@ -144,6 +144,19 @@ inline int check_sample_gf2(int S, long long N, double p_nonzero, const void *ma
     return LAUNCH;
 }
 
+// tg_demo_sample_gf2: the rules of tg_demo_sample_dm in its order -- the scalars, an empty batch, null pointers, tape_dm
+// and the targets 16-byte aligned, then replay_shift in [0, 8]; states may start at any float
+inline int check_demo_sample_gf2(int S, long long N, int R, int dim_t, int replay_shift, long long nb, const void *tape_dm,
+                                 const void *targets, const void *idx, const void *states, const void *scalars, const void *actions,
+                                 const void *rewards) {
+    if (!supported_S(S) || N < 0 || R < 1 || dim_t < 1 || nb < 0) return TG_E_ARG;
+    if (nb == 0) return TG_OK;
+    if (!tape_dm || !targets || !idx || !states || !scalars || !actions || !rewards) return TG_E_ARG;
+    if (misaligned(tape_dm, 16) || misaligned(targets, 16)) return TG_E_ARG;
+    if (replay_shift < 0 || replay_shift > 8) return TG_E_ARG;
+    return LAUNCH;
+}
+
 // change of basis: set by a fast kernel on the games it leaves to the exact int32 kernel, which clears it
 constexpr uint8_t BASIS_REDO = 0x80;
 // tg_basis_mma.cu: 16x16x16 games, one warp per game on mma.sync int8 + f16; tg_basis_mma9.cu: 9x9x9 games on mma.sync f16.

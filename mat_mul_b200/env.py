@@ -129,13 +129,17 @@ def pack_states(heads: torch.Tensor, S: int | None = None, out: torch.Tensor | N
 
 
 def expand_states(slab: torch.Tensor, S: int, out: torch.Tensor | None = None) -> torch.Tensor:
-    """slab -> float32 (B, S, S, S) (the dtype model.py consumes)."""
-    _need_cuda(slab, "slab", torch.int8)
+    """slab -> float32 (B, S, S, S) (the dtype model.py consumes).  An int32 bit slab (B, GB/4) gives its 0/1 values
+    in one pass (tg_expand_f32_gf2)."""
+    bits = isinstance(slab, torch.Tensor) and slab.dtype == torch.int32
+    _need_cuda(slab, "slab", torch.int32 if bits else torch.int8)
+    if bits and (slab.dim() != 2 or slab.shape[1] != layout_gf2(S).game_words):
+        raise TensorGameError(f"expected bits (B,{layout_gf2(S).game_words})")
     B = slab.shape[0]
     if out is None:
         out = torch.empty((B, S, S, S), dtype=torch.float32, device=slab.device)
     stride = out.stride(0) if B > 1 else S ** 3
-    _call("tg_expand_f32", (slab, out,), _p(slab), _p(out), stride, B, S)
+    _call("tg_expand_f32_gf2" if bits else "tg_expand_f32", (slab, out,), _p(slab), _p(out), stride, B, S)
     return out
 
 
@@ -500,18 +504,28 @@ def demo_samples(tape: torch.Tensor, slab: torch.Tensor, idx: torch.Tensor, S: i
 class DemoStore:
     """The in-HBM demonstration store the training-sample batcher reads (replaces the two .pt files per demo of
     datasets.py:62-69): demo-major action records uint8 (N, R, TP) -- the records a .. R-1 one sample needs are one
-    contiguous run -- and the targets as an int8 slab, or an int16 slab when a target left the int8 zone."""
+    contiguous run -- and the targets as an int8 slab, or an int16 slab when a target left the int8 zone.
+
+    Modulo 2 the targets are an int32 bit slab (N, GB/4): samples() then returns the states mod 2 as 0/1 floats
+    (tg_demo_sample_gf2) and target_bound is ignored.  Bit targets of generated demos are exact whatever the integer
+    targets' range: pack_gf2 of make_synthetic_demos' int8 targets (RANGE-flagged ones included: they keep their
+    parity), or replay(zeros, tape, S, shift) of a zeroed bit slab, which xors the demo's terms into it."""
 
     def __init__(self, records: torch.Tensor, targets: torch.Tensor, S: int, shift: int, target_bound: int | None = None):
         _need_cuda(records, "records", torch.uint8)
         lay = layout(S)
         if records.dim() != 3 or records.shape[2] != lay.token_pitch:
             raise TensorGameError(f"records must be (N, R, {lay.token_pitch})")
-        if targets.dtype not in (torch.int8, torch.int16) or targets.shape != (records.shape[0], lay.game_pitch) or not targets.is_cuda:
-            raise TensorGameError(f"targets must be an int8 or int16 slab (N, {lay.game_pitch})")
+        self.bits = targets.dtype == torch.int32
+        pitch = layout_gf2(S).game_words if self.bits else lay.game_pitch
+        if targets.dtype not in (torch.int8, torch.int16, torch.int32) or targets.shape != (records.shape[0], pitch) or not targets.is_cuda:
+            raise TensorGameError(f"targets must be an int8 or int16 slab (N, {lay.game_pitch}) or an int32 bit slab "
+                                  f"(N, {layout_gf2(S).game_words})")
         self.records, self.targets, self.S, self.shift = records, targets.contiguous(), S, shift
         self.N, self.R = records.shape[0], records.shape[1]
-        if target_bound is None:
+        if self.bits:
+            target_bound = 0
+        elif target_bound is None:
             target_bound = 127 if targets.dtype == torch.int8 else (int(targets.abs().max()) if self.N else 0)
         self.target_bound = int(target_bound)
 
@@ -531,16 +545,21 @@ class DemoStore:
 
     def samples(self, idx: torch.Tensor, dim_t: int, replay_shift: int = 1):
         """Batch of SyntheticDemoDataset.__getitem__ results (datasets.py:77-122) for sample indices demo * R + action
-        (tg_demo_sample_dm).  Returns (states f32 (nb,dim_t,S,S,S), scalars f32 (nb,1), actions i64 (nb,3S), rewards f32 (nb,1))."""
+        (tg_demo_sample_dm; with bit targets tg_demo_sample_gf2, states mod 2 as 0/1).  Returns (states f32
+        (nb,dim_t,S,S,S), scalars f32 (nb,1), actions i64 (nb,3S), rewards f32 (nb,1))."""
         _need_cuda(idx, "idx", torch.int64)
         S, nb, dev = self.S, idx.numel(), self.records.device
         states = torch.empty((nb, dim_t, S, S, S), dtype=torch.float32, device=dev)
         scalars = torch.empty((nb, 1), dtype=torch.float32, device=dev)
         actions = torch.empty((nb, 3 * S), dtype=torch.int64, device=dev)
         rewards = torch.empty((nb, 1), dtype=torch.float32, device=dev)
-        _call("tg_demo_sample_dm", (self.records, self.targets, idx, states, scalars, actions, rewards), _p(self.records),
-              _p(self.targets), int(self.targets.dtype == torch.int16), self.target_bound, self.N, self.R, S, dim_t, replay_shift,
-              _p(idx), nb, _p(states), _p(scalars), _p(actions), _p(rewards))
+        operands = (self.records, self.targets, idx, states, scalars, actions, rewards)
+        outputs = (_p(idx), nb, _p(states), _p(scalars), _p(actions), _p(rewards))
+        if self.bits:
+            _call("tg_demo_sample_gf2", operands, _p(self.records), _p(self.targets), self.N, self.R, S, dim_t, replay_shift, *outputs)
+        else:
+            _call("tg_demo_sample_dm", operands, _p(self.records), _p(self.targets), int(self.targets.dtype == torch.int16),
+                  self.target_bound, self.N, self.R, S, dim_t, replay_shift, *outputs)
         return states, scalars, actions, rewards
 
 
