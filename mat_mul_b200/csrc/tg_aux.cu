@@ -1,4 +1,4 @@
-// tg_aux.cu -- K4 demo_sample (training-sample batcher), K6 slice_rank, K7 state_key.
+// tg_aux.cu -- K4 demo_sample (training-sample batcher), K6 slice_rank (int8 and int16 slabs), K7 state_key.
 #include <mutex>
 #include <type_traits>
 
@@ -1023,13 +1023,16 @@ __global__ void tape_to_demo_major_kernel(const uint4 *__restrict__ src, long lo
 // matrix per group of S lanes, lane = matrix row.  rank_p <= rank_Q.  With r the largest rank_p over primes p_1 .. p_k,
 // rank_Q > r needs a non-zero (r+1) x (r+1) minor divisible by every p_j, i.e. one of size >= p_1 ... p_k > 2^(30 k)
 // (primes 2^31 - c).  By Hadamard a minor is at most the product of the norms of its rows; a lane bounds its row's
-// |row|^2 by 2^e (e = ceil(log2 |row|^2) <= 19), so once the r+1 largest e of the slice sum to at most 60 k -- or r is the
-// slice's count of non-zero rows -- r = rank_Q.  Until then the slice is eliminated again mod the next prime: one prime
-// for the few-unit entries of most game states, up to eight for int8 extremes at 25x25x25.
-__constant__ uint32_t c_rank_c[8] = {1, 19, 61, 69, 85, 99, 105, 151}; // p = 2^31 - c, all prime
+// |row|^2 by 2^e (e = ceil(log2 |row|^2): <= 19 for int8, <= 35 for int16), so once the r+1 largest e of the slice sum
+// to at most 60 k -- or r is the slice's count of non-zero rows -- r = rank_Q.  Until then the slice is eliminated again
+// mod the next prime: one prime for the few-unit entries of most game states, up to eight for int8 extremes and
+// fifteen (a product above 2^900 against r+1 largest e summing to at most 875) for int16 extremes at 25x25x25.
+__constant__ uint32_t c_rank_c[15] = {1, 19, 61, 69, 85, 99, 105, 151, 159, 171, 225, 249, 295, 325, 379}; // p = 2^31 - c, all prime
+template <typename T>
+constexpr int RANK_PRIMES = sizeof(T) == 1 ? 8 : 15;
 
-template <int S>
-__device__ __forceinline__ int rank_mod_p(const int8_t *__restrict__ src, bool live, int lane, uint32_t gmask, uint32_t P, uint32_t C) {
+template <int S, typename T>
+__device__ __forceinline__ int rank_mod_p(const T *__restrict__ src, bool live, int lane, uint32_t gmask, uint32_t P, uint32_t C) {
     uint32_t row[S];
 #pragma unroll
     for (int c = 0; c < S; c++) {
@@ -1053,10 +1056,10 @@ __device__ __forceinline__ int rank_mod_p(const int8_t *__restrict__ src, bool l
         for (int k = c + 1; k < S; k++) {
             const uint32_t pk = __shfl_sync(0xFFFFFFFFu, row[k], pl);
             if (elim) {
-                // 2^31 = C (mod P): fold the bits above 31 twice, then one conditional subtraction (C <= 151)
+                // 2^31 = C (mod P): fold the bits above 31 twice, then one conditional subtraction (C < 2^9)
                 const unsigned long long z = (unsigned long long)row[k] * pv + (unsigned long long)nmine * pk; // < 2^63
-                unsigned long long r = (z & 0x7FFFFFFFull) + (z >> 31) * C;                                    // < 2^40
-                uint32_t q = (uint32_t)(r & 0x7FFFFFFFull) + (uint32_t)(r >> 31) * C;                          // < P + 2^18
+                unsigned long long r = (z & 0x7FFFFFFFull) + (z >> 31) * C;                                    // < 2^41
+                uint32_t q = (uint32_t)(r & 0x7FFFFFFFull) + (uint32_t)(r >> 31) * C;                          // < P + 2^19
                 row[k] = q >= P ? q - P : q;
             }
         }
@@ -1066,8 +1069,8 @@ __device__ __forceinline__ int rank_mod_p(const int8_t *__restrict__ src, bool l
     return rank;
 }
 
-template <int S>
-__global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__restrict__ ranks, long long B) {
+template <int S, typename T>
+__global__ void slice_rank_kernel(const T *__restrict__ slab, int32_t *__restrict__ ranks, long long B) {
     using G = Geo<S>;
     constexpr int LG = S;       // lanes per matrix: 4 / 9 / 16 (the shuffles address absolute lanes, so any group size works)
     constexpr int MPW = 32 / LG; // matrices per warp: 8 / 3 (lanes 27..31 idle; two per warp with groups of 16 was 1.5x slower) / 2
@@ -1078,16 +1081,19 @@ __global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__re
     const long long game = mat / S;
     const int slice = (int)(mat - game * S);
     const bool live = sub < MPW && game < B && r < S;
-    const int8_t *src = slab + (live ? game * G::GP + slice * G::RP + r * S : 0);
+    const T *src = slab + (live ? game * G::GP + slice * G::RP + r * S : 0);
     const uint32_t gmask = sub < MPW ? (((1u << LG) - 1u) << (sub * LG)) : 0u;
     int rank = rank_mod_p<S>(src, live, lane, gmask, 0x7FFFFFFFu, 1u);
-    uint32_t n2 = 0; // |row|^2 <= 25 * 128^2 < 2^19
+    using N2 = std::conditional_t<sizeof(T) == 1, uint32_t, unsigned long long>;
+    N2 n2 = 0; // |row|^2 <= 25 * 128^2 < 2^19 (int8), 25 * 2^30 < 2^35 (int16)
 #pragma unroll
     for (int c = 0; c < S; c++) {
         const int v = live ? src[c] : 0;
-        n2 += (uint32_t)(v * v);
+        n2 += (N2)(v * v);
     }
-    const int e = n2 <= 1 ? 0 : 32 - __clz(n2 - 1); // |row|^2 <= 2^e
+    int e = 0; // |row|^2 <= 2^e
+    if constexpr (sizeof(N2) == 4) e = n2 <= 1 ? 0 : 32 - __clz(n2 - 1);
+    else e = n2 <= 1 ? 0 : 64 - __clzll((long long)(n2 - 1));
     const int emax = (int)__reduce_max_sync(0xFFFFFFFFu, (unsigned)e);
     const int nzrows = __popc(__ballot_sync(0xFFFFFFFFu, n2 != 0) & gmask);
     // sum of the m largest e of the group (sum over t of min(m, #{e >= t})): an m x m minor is at most 2^(that / 2)
@@ -1104,7 +1110,7 @@ __global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__re
         fin = fin || E <= 60;
     }
 #pragma unroll 1
-    for (int j = 1; j < 8 && !__all_sync(0xFFFFFFFFu, fin); j++) { // every lane runs the shuffles
+    for (int j = 1; j < RANK_PRIMES<T> && !__all_sync(0xFFFFFFFFu, fin); j++) { // every lane runs the shuffles
         const int rj = rank_mod_p<S>(src, live, lane, gmask, 0x80000000u - c_rank_c[j], c_rank_c[j]);
         if (!fin) rank = max(rank, rj);
         const int E = top_e(rank + 1);
@@ -1115,20 +1121,7 @@ __global__ void slice_rank_kernel(const int8_t *__restrict__ slab, int32_t *__re
 }
 
 // ------------------------------------------------------------------ K7
-// 64-bit state key replacing the string key of utils.py:164-169 (dict key of
-// the MCTS tree, act.py:37...210): a linear hash, sum over entries of value * A_i * B_j * C_k (the trilinear form of
-// the state at three fixed odd 64-bit vectors, A_i = splitmix64(0x1000 + i) | 1, B_j = splitmix64(0x2000 + j) | 1,
-// C_k = splitmix64(0x3000 + k) | 1).  The product structure is what lets tg_expand_children (tg_expand.cu) get a
-// child's key from its action's 3 S tokens alone.
-__device__ __forceinline__ unsigned long long splitmix64(unsigned long long z) {
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-
-__device__ __forceinline__ unsigned long long key_const(unsigned base, int i) { return splitmix64((unsigned long long)(base + i)) | 1ull; }
-
+// tg_state_key: the 64-bit state key of tg_common.cuh (key_const).
 // key(T) = sum T[i][j][k] * A_i * B_j * C_k (mod 2^64).  One thread per word column of a game: its four entries of row i
 // as unsigned offset-binary bytes (entry + 128) times the compile-time A_i go into four 64-bit accumulators (one wide
 // and one 32-bit multiply-add per entry; the offset's share -128 sum_i A_i is their start value), which then meet the
@@ -1412,6 +1405,19 @@ int tg_slice_rank(const int8_t *slab, int32_t *ranks, int64_t B, int S, void *st
         constexpr int kS = decltype(s)::value;
         const long long warps = (B * kS + (32 / kS) - 1) / (32 / kS);
         tg::slice_rank_kernel<kS><<<(unsigned)((warps * 32 + 127) / 128), 128, 0, st>>>(slab, ranks, B);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
+}
+
+int tg_slice_rank_i16(const int16_t *slab16, int32_t *ranks, int64_t B, int S, void *stream) {
+    if (const int rc = tg::check_pair(S, B, slab16, 16, ranks, 1); rc != tg::LAUNCH) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    TG_CUDA(cudaMemsetAsync(ranks, 0, (size_t)B * 4, st));
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        const long long warps = (B * kS + (32 / kS) - 1) / (32 / kS);
+        tg::slice_rank_kernel<kS><<<(unsigned)((warps * 32 + 127) / 128), 128, 0, st>>>(slab16, ranks, B);
         TG_CUDA(cudaGetLastError());
         return TG_OK;
     });

@@ -12,7 +12,7 @@ namespace tg {
 // ---------------------------------------------------------------- geometry
 // Device slab: int8 [B][GP]; entry (i,j,k) at i*RP + j*S + k.  One 32-bit word
 // holds four consecutive (j,k) entries of one i-row, so the rank-1 update of a
-// word is  u_i * pack(v_j w_k)  -- one IMAD per word (see tg_step.cu).
+// word is  u_i * pack(v_j w_k)  -- one IMAD per word (see tg_step.cuh).
 template <int S>
 struct Geo {
     static constexpr int S2 = S * S;
@@ -186,6 +186,20 @@ __device__ __forceinline__ void philox_block(uint32_t c0, uint32_t c1, uint32_t 
     }
     out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
 }
+
+// 64-bit state key replacing the string key of utils.py:164-169 (dict key of the MCTS tree, act.py:37...210): a linear
+// hash, key(T) = sum T[i][j][k] * A_i * B_j * C_k (mod 2^64), the trilinear form of the state at three fixed odd 64-bit
+// vectors, A_i = key_const(0x1000, i), B_j = key_const(0x2000, j), C_k = key_const(0x3000, k), distinct per mode
+// so that transposed states differ.  The int8, int16 and bit-slab kernels use the same constants, so a state has the
+// same key in every format that holds it.  The product structure is what lets the leaf expansion get a child's key
+// from its action's 3 S tokens alone.
+__device__ __forceinline__ unsigned long long splitmix64(unsigned long long z) {
+    z += 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+__device__ __forceinline__ unsigned long long key_const(unsigned base, int i) { return splitmix64((unsigned long long)(base + i)) | 1ull; }
 
 // ---------------------------------------------------------------- PTX: mbarrier + bulk async copy (TMA 1-D)
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }

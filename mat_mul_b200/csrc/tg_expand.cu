@@ -8,178 +8,10 @@
 //     children[b][c] = parents[b] - rank1(tape[b][c]),  c < k,
 // with per-child flags (terminal / null action / range), non-zero count and 64-bit state key.
 //
-// The parent is read ONCE: thread (parent, word column) keeps its S row words in registers and produces the k
-// children one after the other into a three-stage shared-memory tile; each child game leaves with a TMA bulk store
-// while the next ones are computed (three stages so that ONE CTA barrier per child is enough: a stage is rewritten two
-// barriers after the threads that issued its stores have seen them drain).  HBM traffic per child: GP * (1 + 1/k) + TP + 13 bytes.
-// The state key is the trilinear form of the state at three fixed 64-bit vectors (sum T[i][j][k] A_i B_j C_k mod 2^64,
-// tg_state_key), so a child's key is the parent's key (hashed once per parent) minus
-// (sum u_i A_i)(sum v_j B_j)(sum w_k C_k): 3 S multiply-adds on the action's tokens, done for all TG * k children of the
-// block before the child loop -- no pass over the child, no per-entry work.
+// The word-column kernel expand_kernel (tg_step.cuh) serves 9x9x9, 16x16x16 and 25x25x25; 4x4x4 has a row kernel here.
 #include "tg_step.cuh"
 
 namespace tg {
-
-template <int S, int NT>
-struct ExpCfg {
-    using G = Geo<S>;
-    static constexpr int TG = NT / G::WR; // parents per CTA (one word column per thread)
-    static constexpr int ACTIVE = TG * G::WR;
-    static constexpr int STAGE_BYTES = TG * G::GP;
-    static __host__ __device__ constexpr int tok_bytes(int k) { return (TG * k * G::TP + 15) & ~15; }
-    static constexpr int NSTAGE = 3;
-    // tokens, NSTAGE child stages, per-(stage, game) partial word and key
-    static __host__ __device__ constexpr int smem_bytes(int k) {
-        return tok_bytes(k) + NSTAGE * STAGE_BYTES + ((NSTAGE * TG * 4 + 7) & ~7) + TG * 8 + 16 + NT * 8;
-    }
-};
-
-__device__ __forceinline__ unsigned long long splitmix64_e(unsigned long long z) {
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-// A_i / B_j / C_k of the state key (tg_state_key): base 0x1000 / 0x2000 / 0x3000
-__device__ __forceinline__ unsigned long long key_const(unsigned base, int i) { return splitmix64_e((unsigned long long)(base + i)) | 1ull; }
-__device__ __forceinline__ unsigned long long splitmix_or1(unsigned x) { return splitmix64_e((unsigned long long)x) | 1ull; } // the same constant from a run-time index
-
-template <int S, int NT, bool KEYS>
-__global__ void __launch_bounds__(NT)
-    expand_kernel(const int8_t *__restrict__ parents, const uint8_t *__restrict__ tape, int k, int8_t *__restrict__ children,
-                  uint8_t *__restrict__ flags, int32_t *__restrict__ nnz, unsigned long long *__restrict__ keys, long long B,
-                  int shift) {
-    using C = ExpCfg<S, NT>;
-    using G = Geo<S>;
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint8_t *s_tok = smem;                                                            // [TG][k][TP]
-    constexpr int NSTAGE = C::NSTAGE;
-    uint8_t *s_out = smem + C::tok_bytes(k);                                          // [NSTAGE][TG][GP]
-    uint32_t *s_part = reinterpret_cast<uint32_t *>(s_out + NSTAGE * C::STAGE_BYTES); // [NSTAGE][TG]
-    unsigned long long *s_pkey = reinterpret_cast<unsigned long long *>(reinterpret_cast<uint8_t *>(s_part) + ((NSTAGE * C::TG * 4 + 7) & ~7)); // [TG] parent keys
-    uint64_t *s_bar = reinterpret_cast<uint64_t *>(s_pkey + C::TG);
-    unsigned long long *s_ph = reinterpret_cast<unsigned long long *>(s_bar + 2); // [NT] parent key, per word column
-
-    const int tid = threadIdx.x;
-    const long long g0 = (long long)blockIdx.x * C::TG;
-    const int ng = (int)min((long long)C::TG, B - g0);
-    const int g = tid / G::WR;
-    const bool active = tid < C::ACTIVE && g < ng;
-    Lane<S> L;
-    L.init(tid < C::ACTIVE ? tid % G::WR : 0);
-
-    if (tid == 0) {
-        mbar_init(s_bar, 1);
-        mbar_fence_init();
-    }
-    // game padding of the child stages is zero and stays zero (threads only write their word columns of the S rows)
-    for (int w = tid; w < NSTAGE * C::STAGE_BYTES / 4; w += NT) reinterpret_cast<uint32_t *>(s_out)[w] = 0;
-    for (int i = tid; i < NSTAGE * C::TG; i += NT) s_part[i] = 0;
-    // key constants of this thread's word column: B_j C_k of its four entries (0 in the row padding)
-    unsigned long long kb[4] = {0, 0, 0, 0};
-    if constexpr (KEYS) {
-#pragma unroll
-        for (int q = 0; q < 4; q++) {
-            const int jk = 4 * L.c + q;
-            kb[q] = jk < G::S2 ? key_const(0x2000, jk / S) * key_const(0x3000, jk % S) : 0ull;
-        }
-    }
-    __syncthreads();
-    if (tid == 0) {
-        mbar_expect_tx(s_bar, (uint32_t)(ng * k * G::TP));
-        bulk_g2s(s_tok, tape + g0 * k * G::TP, (uint32_t)(ng * k * G::TP), s_bar);
-    }
-    // the parent's rows of this thread's word column, offset-binary
-    uint32_t row[S];
-    if (active) {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(parents + (g0 + g) * G::GP) + L.c;
-#pragma unroll
-        for (int i = 0; i < S; i++) row[i] = src[i * G::WR] ^ H4;
-    } else {
-#pragma unroll
-        for (int i = 0; i < S; i++) row[i] = H4;
-    }
-    if constexpr (KEYS) {
-        // the parent's key, once: this thread's word column gives sum_q (B C)[4c + q] * sum_i A_i T[i][4c + q]; the rows
-        // are offset-binary bytes (entry + 128, unsigned: one wide multiply-add and one 32-bit one per entry), the
-        // offset's share -128 sum_i A_i is the accumulators' start value
-        unsigned long long a0 = 0;
-#pragma unroll
-        for (int i = 0; i < S; i++) a0 -= 128ull * key_const(0x1000, i);
-        unsigned long long acc[4] = {a0, a0, a0, a0};
-#pragma unroll
-        for (int i = 0; i < S; i++) {
-#pragma unroll
-            for (int q = 0; q < 4; q++) acc[q] += (unsigned long long)((row[i] >> (8 * q)) & 0xFFu) * key_const(0x1000, i);
-        }
-        s_ph[tid] = acc[0] * kb[0] + acc[1] * kb[1] + acc[2] * kb[2] + acc[3] * kb[3];
-    }
-    mbar_wait(s_bar, 0);
-    if constexpr (KEYS) {
-        __syncthreads();
-        if (tid < ng) {
-            unsigned long long h = 0;
-            for (int c = 0; c < G::WR; c++) h += s_ph[tid * G::WR + c];
-            s_pkey[tid] = h;
-        }
-        __syncthreads();
-        // child key = parent key - key of its rank-1 action, the latter from the action's tokens alone; one coalesced
-        // store of the block's TG * k keys
-        for (int x = tid; x < ng * k; x += NT) {
-            const uint8_t *tok = s_tok + (size_t)x * G::TP;
-            unsigned long long f[3];
-#pragma unroll
-            for (int m = 0; m < 3; m++) {
-                unsigned long long a = 0;
-#pragma unroll
-                for (int i = 0; i < S; i++) a += (unsigned long long)(long long)((int)tok[m * S + i] - shift) * key_const(0x1000 * (m + 1), i);
-                f[m] = a;
-            }
-            keys[g0 * k + x] = s_pkey[x / k] - f[0] * f[1] * f[2];
-        }
-    }
-
-    for (int c = 0, st = 0; c < k; c++, st = st + 1 == NSTAGE ? 0 : st + 1) {
-        uint8_t *stage = s_out + st * C::STAGE_BYTES;
-        // the bulk stores of child c-3 have finished reading this stage: the threads that issued them waited for child c-2's
-        // predecessor to drain (bulk_wait_read<1> below, iteration c-2) before they arrived at the barrier of iteration c-1
-        if (active) {
-            const uint8_t *tok = s_tok + ((size_t)g * k + c) * G::TP;
-            const int32_t vw = pack_vw<S>(tok, L, shift);
-            uint32_t uw[UW<S>];
-            load_u<S>(tok, uw);
-            const uint32_t nvw = (uint32_t)(-vw);
-            uint32_t cnt = 0, rng = 0;
-            int uany = 0;
-            uint32_t *col = reinterpret_cast<uint32_t *>(stage + (size_t)g * G::GP) + L.c;
-#pragma unroll
-            for (int i = 0; i < S; i++) {
-                const int negu = coef_u(uw, i, shift);
-                const uint32_t t = (row[i] + (uint32_t)negu * nvw) ^ H4; // child word, two's complement bytes
-                col[i * G::WR] = t;
-                cnt += ((((t & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | t) & L.hv) >> 7;
-                rng |= t ^ (t << 1);
-                uany |= negu;
-            }
-            atomicAdd(&s_part[st * C::TG + g], make_partial(byte_sum(cnt), vw != 0 && uany != 0,
-                                                            (rng & L.hv) != 0 || tokens_out_of_range<S>(tok, L, shift)));
-        }
-        fence_proxy_async();
-        __syncthreads();
-        if (tid < ng) {
-            const long long child = (g0 + tid) * k + c;
-            bulk_s2g(children + child * G::GP, stage + (size_t)tid * G::GP, (uint32_t)G::GP);
-            bulk_commit();
-            const uint32_t sum = s_part[st * C::TG + tid];
-            flags[child] = (uint8_t)partial_flags(sum);
-            nnz[child] = (int32_t)(sum & 0xFFFFu);
-            s_part[st * C::TG + tid] = 0;
-            bulk_wait_read<1>(); // the store of child c-1 has drained; its stage is rewritten at c+2, one barrier from here
-        }
-        // no second barrier: the partial words of this stage are reset here and next touched at child c+3, two barriers away
-    }
-    if (tid < ng) bulk_wait<0>();
-}
 
 // ------------------------------------------------------------------ 4x4x4: four threads per parent, rows in registers
 // A 4x4x4 parent is 16 words: thread (parent, i) keeps ROW i (4 words, offset-binary) in registers while the k children are
@@ -238,7 +70,7 @@ __global__ void __launch_bounds__(128)
     unsigned long long kc[S] = {0, 0, 0, 0}; // lane i < 3: the constants of factor i of an action's key
     if constexpr (KEYS) {
 #pragma unroll
-        for (int x = 0; x < S; x++) kc[x] = splitmix_or1(0x1000u * (unsigned)(i + 1) + (unsigned)x);
+        for (int x = 0; x < S; x++) kc[x] = key_const(0x1000u * (unsigned)(i + 1), x);
     }
     uint4 q = __ldg(rec);
     for (int c = 0; c < k; c++) {
@@ -285,27 +117,6 @@ __global__ void __launch_bounds__(128)
     }
 }
 
-template <int S, int NT>
-static int launch_expand(const int8_t *parents, const uint8_t *tape, int k, int8_t *children, uint8_t *flags, int32_t *nnz,
-                         unsigned long long *keys, long long B, int shift, cudaStream_t st) {
-    using C = ExpCfg<S, NT>;
-    const int smem = C::smem_bytes(k);
-    if (smem > 200 * 1024) return TG_E_ARG;
-    const long long grid = (B + C::TG - 1) / C::TG;
-    if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
-    if (keys) {
-        auto kern = expand_kernel<S, NT, true>;
-        TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        kern<<<(int)grid, NT, smem, st>>>(parents, tape, k, children, flags, nnz, keys, B, shift);
-    } else {
-        auto kern = expand_kernel<S, NT, false>;
-        TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        kern<<<(int)grid, NT, smem, st>>>(parents, tape, k, children, flags, nnz, keys, B, shift);
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
-}
-
 } // namespace tg
 
 extern "C" int tg_expand_children(const int8_t *parents, const uint8_t *tape, int k, int8_t *children, uint8_t *flags,
@@ -316,7 +127,7 @@ extern "C" int tg_expand_children(const int8_t *parents, const uint8_t *tape, in
     case 4: {
 #ifdef TG_TUNING
         if (tg::tuning_env("TG_EXPAND_COLUMNS", 0)) // A/B: the word-column kernel
-            return tg::launch_expand<4, 256>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
+            return tg::launch_expand<4, 256, tg::W8>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
 #endif
         const long long grid = (B * 4 + 127) / 128;
         if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
@@ -325,9 +136,9 @@ extern "C" int tg_expand_children(const int8_t *parents, const uint8_t *tape, in
         TG_CUDA(cudaGetLastError());
         return TG_OK;
     }
-    case 9: return tg::launch_expand<9, 128>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
-    case 16: return tg::launch_expand<16, 128>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
-    case 25: return tg::launch_expand<25, 160>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st); // one parent per CTA
+    case 9: return tg::launch_expand<9, 128, tg::W8>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
+    case 16: return tg::launch_expand<16, 128, tg::W8>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st);
+    case 25: return tg::launch_expand<25, 160, tg::W8>(parents, tape, k, children, flags, nnz, (unsigned long long *)keys, B, shift, st); // one parent per CTA
     }
     return TG_E_ARG;
 }

@@ -50,27 +50,19 @@ __device__ __forceinline__ T group_sum(T x) {
 // ------------------------------------------------------------------ state key tables
 // key(T) = sum T[i][j][k] A_i B_j C_k (mod 2^64) over the 0/1 values (tg_state_key).  A word r of row i adds
 // A_i * sum_{bits b} (B C)[32 r + b]; that sum is read from nibble tables tab[r][n][16] of the (B C) products.
-__device__ __forceinline__ unsigned long long splitmix(unsigned long long z) {
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-__device__ __forceinline__ unsigned long long kconst(unsigned base, int i) { return splitmix((unsigned long long)(base + i)) | 1ull; }
-
 template <int S>
 struct KeyTab {
     unsigned long long a[S];
     unsigned long long tab[GeoB<S>::RW * 128];
 
     __device__ __forceinline__ void build() {
-        for (int i = threadIdx.x; i < S; i += blockDim.x) a[i] = kconst(0x1000, i);
+        for (int i = threadIdx.x; i < S; i += blockDim.x) a[i] = key_const(0x1000, i);
         for (int e = threadIdx.x; e < GeoB<S>::RW * 128; e += blockDim.x) {
             const int r = e / 128, n = (e / 16) % 8, v = e % 16;
             unsigned long long s = 0;
             for (int b = 0; b < 4; b++) {
                 const int jk = 32 * r + 4 * n + b;
-                if (((v >> b) & 1) && jk < GeoB<S>::S2) s += kconst(0x2000, jk / S) * kconst(0x3000, jk % S);
+                if (((v >> b) & 1) && jk < GeoB<S>::S2) s += key_const(0x2000, jk / S) * key_const(0x3000, jk % S);
             }
             tab[e] = s;
         }

@@ -121,7 +121,7 @@ __global__ void __launch_bounds__(NT + 32)
             mbar_wait(&s_full[st], parity);
             if (alive) {
                 const uint8_t *tok = tok0 + st * C::TOK_BYTES;
-                const int32_t vw = pack_vw<S>(tok, L, shift);
+                const int32_t vw = W8::pack_vw<S>(tok, L, shift);
                 uint32_t uw[UW<S>];
                 load_u<S>(tok, uw);
                 uint32_t any = 0;

@@ -20,6 +20,22 @@ OK, E_ARG = 0, -1
 
 BASE = 1 << 20  # never dereferenced
 
+# tg_expand_children*: threads per CTA of the word-column kernel (int8 at 4 uses a row kernel without shared memory)
+EXPAND_NT = {"": {9: 128, 16: 128, 25: 160}, "_i16": {4: 128, 9: 256, 16: 256, 25: 320}}
+EXPAND_SMEM_CAP = 200 * 1024  # bytes of shared memory the records and child stages of a CTA may take
+
+
+def expand_limits(sfx: str, S: int):
+    """(k whose TG * k * TP bytes of records is a multiple of 2^32, the first k whose records exceed shared memory)"""
+    rp = (S * S + 3) & ~3
+    gp, tp = (S * rp + 15) & ~15, (3 * S + 15) & ~15
+    eb = 2 if sfx else 1
+    nt = EXPAND_NT[sfx][S]
+    tg = nt // (rp * eb // 4)
+    smem0 = 3 * tg * gp * eb + ((3 * tg * 4 + 7) & ~7) + tg * 8 + 16 + nt * 8
+    wrap = next(1 << e for e in range(1, 31) if (tg * tp << e) % (1 << 32) == 0)
+    return wrap, (EXPAND_SMEM_CAP - smem0) // (tg * tp) + 1
+
 
 def ptr(offset: int = 0) -> C.c_void_p:
     return C.c_void_p(BASE + offset)
@@ -85,6 +101,11 @@ def _rows(S: int):
             add(fn, EXPAND, f"k {k}", E_ARG, k=k)
         add(fn, EXPAND, "empty batch, k 0", E_ARG, B=0, k=0)
         add(fn, EXPAND, "all null but keys", E_ARG, **{k: n for k in ("in", "tape", "out", "flags", "nnz")}, keys=ptr())
+        if S in EXPAND_NT.get(sfx, {}):  # the records of a CTA must fit shared memory, also where their size wraps int
+            wrap, over = expand_limits(sfx, S)
+            for k in (wrap, over):
+                for keys in (n, ptr()):
+                    add(fn, EXPAND, f"k {k}{' with keys' if keys else ''}", E_ARG, k=k, keys=keys)
 
         for fn, names in (("tg_rollout" + sfx, ROLLOUT), ("tg_replay" + sfx, REPLAY)):
             common(fn, names, tuple(k for k in ("in", "out", "flags", "nnz", "steps") if k in names), slabs16)
