@@ -13,11 +13,13 @@
  *   - unless the name ends in _host, every pointer is a CUDA DEVICE pointer
  *     owned by the caller; calls are asynchronous on `stream` (a cudaStream_t
  *     passed as void*), never allocate and never synchronise -- with one
- *     exception: tg_demo_gen_philox keeps the device form of up to eight
- *     alias-table sets per device in static device memory (uploaded on
- *     `stream` the first time a distribution is used; launches on other
- *     streams wait for that upload by event); a NINTH distinct distribution
- *     evicts one after a cudaDeviceSynchronize.  tg_demo_sample_dm (9x9x9)
+ *     exception: tg_demo_gen_philox and tg_demo_gen_gf2 keep the device form
+ *     of up to eight alias-table sets per device in static device memory,
+ *     one cache for both (uploaded on `stream` the first time a distribution
+ *     is used; launches on other streams wait for that upload by event; the
+ *     mod-2 tables of an alphabet whose only even value is 0 are the integer
+ *     ones and share their slot); a NINTH distinct set evicts one after a
+ *     cudaDeviceSynchronize.  tg_demo_sample_dm (9x9x9)
  *     zeroes a per-launch work counter in static device memory on `stream`.
  *   - *_host entry points take HOST pointers (pinned for full speed), move the
  *     data themselves through a caller-created tg_host_ctx and return after
@@ -69,7 +71,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 204
+#define TG_VERSION 205
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -364,6 +366,35 @@ int tg_demo_sample_gf2(const uint8_t *tape_dm, const uint32_t *targets_bits, int
  * tg_expand_f32(tg_unpack_gf2(bits)) in one pass.  The game path's argument rules (bits 16-byte aligned, dst 4-byte);
  * dst may start at any float, and floats outside each game's S^3 are not written. */
 int tg_expand_f32_gf2(const uint32_t *bits, float *dst, int64_t dst_stride, int64_t B, int S, void *stream);
+
+/* ---- mod-2 synthetic demonstrations: K3 with bit-slab targets (S in {4, 9, 16, 25}) -------------------------------- */
+/* tg_demo_gen_philox modulo 2: the same arguments, with a bit slab [N][GB/4] (16-byte aligned) for the int8 slab.  Each
+ * factor is an i.i.d. factor of the alphabet conditioned on having at least one ODD entry -- the reference's rejection
+ * rule (utils.py:222-232) with "zero" read as "zero mod 2" -- so every term of a demo is a non-null action of the mod-2
+ * game.  (tg_demo_gen_philox conditions on non-zero over Z: with an even value besides 0, such as 2 in {-2..2}, some of
+ * its terms vanish mod 2.)  Demo d = first_demo + n is keyed by its global index, as there.
+ *  v2 mod 2 (n_values <= 5, S <= 16, P(value even) <= 0.999): contract v2 with its groups, counters, 16-bit draws,
+ *   128-bucket tables and Vose order; in the tilted table of group g EVERY outcome whose entries are all even is weighed
+ *   by 1 - P(every later entry even), and "all groups so far even" selects the tilted tables.  max_tries does not apply.
+ *  v1 mod 2 (other alphabets, and every alphabet at 25): contract v1's counters and draws; a try is rejected iff u, v or
+ *   w has no odd entry; after max_tries tries the term is u = v = w = x e_0 with x the LAST ODD value of the alphabet,
+ *   and the demo gets TG_FLAG_EXHAUSTED.
+ * Writes the tape (tokens = value + shift, step-major [R][N][TP], padding zero, tape_step_stride as there), the bit
+ * target = the xor of the R terms mod 2 (padding bits and words zero) and flags (may be NULL): TG_FLAG_EXHAUSTED or 0;
+ * TG_FLAG_RANGE is never raised.  Checks in tg_demo_gen_philox's order: a bad scalar (S, N < 0, R outside [1, 65535],
+ * shift outside [1, 4], n_values outside [1, 8], max_tries outside [1, 65535]) returns TG_E_ARG; N == 0 returns TG_OK;
+ * a null values, probs, tape or bits returns TG_E_ARG; a misaligned tape, step stride or bit slab returns TG_E_ARG;
+ * then a negative or NaN probability, a zero sum, a value outside [-shift, shift] or an alphabet with no odd value
+ * returns TG_E_ARG.
+ * Where 0 is the only even value (listed once) and, under v1, the last value is odd, the tables and the accept rule are
+ * the integer ones: the tape is tg_demo_gen_philox's byte for byte, the bits are tg_pack_gf2 of its targets and the
+ * EXHAUSTED flags are the same -- a mod-2 run and an integer run with one seed see the same demos. */
+int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int shift, const int8_t *values,
+                    const double *probs, int n_values, int max_tries, uint8_t *tape, int64_t tape_step_stride,
+                    uint32_t *bits, uint8_t *flags, void *stream);
+/* HOST function: the tables of v2 mod 2 in tg_demo_alias_tables' layout (uint16 [8][128]); TG_E_ARG where v2 mod 2 does
+ * not apply (also at S = 25). */
+int tg_demo_alias_tables_gf2(const int8_t *values, const double *probs, int n_values, int S, uint16_t *tables_host);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

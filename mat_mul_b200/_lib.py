@@ -143,6 +143,9 @@ _SIGNATURES = {
     "tg_demo_sample_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp,
                                      _vp]),
     "tg_expand_f32_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
+    "tg_demo_gen_gf2": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
+                                  _vp, C.c_int64, _vp, _vp, _vp]),
+    "tg_demo_alias_tables_gf2": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
     "tg_change_of_basis_factors": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp, C.c_int64,
                                              C.c_int, C.c_int, _vp]),
     "tg_sample_unimodular": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),

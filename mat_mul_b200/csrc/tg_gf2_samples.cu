@@ -79,28 +79,6 @@ __device__ __forceinline__ void split(long long x, int d, long long &q, int &r) 
     }
 }
 
-// xor the term of a record (parities p) into rows r0 .. r0 + RPT - 1
-template <int S, int RPT>
-__device__ __forceinline__ void xor_term(uint32_t (&row)[RPT][GeoB<S>::RW], const Par &p, int r0) {
-    constexpr int RW = GeoB<S>::RW;
-    uint32_t V[RW];
-#pragma unroll
-    for (int w = 0; w < RW; w++) V[w] = 0;
-#pragma unroll
-    for (int j = 0; j < S; j++) {
-        const uint32_t x = p.w & (0u - ((p.v >> j) & 1u));
-        const int o = j * S, q = o / 32, s = o % 32;
-        V[q] |= x << s;
-        if (s + S > 32) V[q + 1] |= x >> (32 - s);
-    }
-#pragma unroll
-    for (int k = 0; k < RPT; k++) {
-        const uint32_t on = 0u - ((p.u >> (r0 + k)) & 1u);
-#pragma unroll
-        for (int w = 0; w < RW; w++) row[k][w] ^= V[w] & on;
-    }
-}
-
 template <int S>
 __global__ void __launch_bounds__(256) demo_sample_gf2_kernel(const uint8_t *__restrict__ tape_dm, const uint32_t *__restrict__ targets,
                                                               long long N, int R, int dim_t, int shift, const long long *__restrict__ idx,

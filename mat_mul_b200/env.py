@@ -363,6 +363,32 @@ def make_synthetic_demos(n_demos: int, max_actions: int, S: int, values=(-1, 0, 
     return tape, slab, flags
 
 
+def make_synthetic_demos_gf2(n_demos: int, max_actions: int, S: int, values=(-1, 0, 1), probs=(0.15, 0.7, 0.15), shift: int = 1,
+                             seed: int = 0, first_demo: int = 0, device="cuda", max_tries: int = 64, tape: torch.Tensor | None = None,
+                             bits: torch.Tensor | None = None):
+    """Throughput-mode demo generation modulo 2 (tg_demo_gen_gf2): every factor has an odd entry, so no term vanishes mod 2,
+    and the targets are bit slabs (the xor of the terms), written without an int8 slab.
+
+    Returns (tape uint8 (R, N, TP) step-major, bits int32 (N, GB/4), flags uint8 (N,): TG_FLAG_EXHAUSTED or 0).  Where 0
+    is the only even value of the alphabet, the tape is make_synthetic_demos' for the same arguments and the bits are
+    pack_gf2 of its targets."""
+    lay, lb = layout(S), layout_gf2(S)
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise TensorGameError("make_synthetic_demos_gf2 needs a CUDA device (there is no CPU path)")
+    v, p = _cat_arrays(values, probs)
+    if tape is None:
+        tape = torch.empty((max_actions, n_demos, lay.token_pitch), dtype=torch.uint8, device=dev)
+    if bits is None:
+        bits = torch.empty((n_demos, lb.game_words), dtype=torch.int32, device=dev)
+    flags = torch.empty(n_demos, dtype=torch.uint8, device=dev)
+    stride = tape.stride(0) if max_actions > 1 else n_demos * lay.token_pitch
+    with torch.cuda.device(dev):
+        _call("tg_demo_gen_gf2", (tape, bits, flags), seed, first_demo, n_demos, max_actions, S, shift, v.ctypes.data, p.ctypes.data,
+              len(v), max_tries, _p(tape), stride, _p(bits), _p(flags))
+    return tape, bits, flags
+
+
 def accumulate_demos(tape: torch.Tensor, S: int, shift: int, slab: torch.Tensor | None = None):
     """slab[n] = sum_r rank1(tape[r, n]) (tg_demo_accumulate).  Returns (slab, flags)."""
     _need_cuda(tape, "tape", torch.uint8)
@@ -507,9 +533,11 @@ class DemoStore:
     contiguous run -- and the targets as an int8 slab, or an int16 slab when a target left the int8 zone.
 
     Modulo 2 the targets are an int32 bit slab (N, GB/4): samples() then returns the states mod 2 as 0/1 floats
-    (tg_demo_sample_gf2) and target_bound is ignored.  Bit targets of generated demos are exact whatever the integer
-    targets' range: pack_gf2 of make_synthetic_demos' int8 targets (RANGE-flagged ones included: they keep their
-    parity), or replay(zeros, tape, S, shift) of a zeroed bit slab, which xors the demo's terms into it."""
+    (tg_demo_sample_gf2) and target_bound is ignored.  Generated demos for a mod-2 run come from
+    make_synthetic_demos_gf2, which writes the bit targets directly and conditions every factor on an odd entry (no term
+    vanishes mod 2).  For any other tape, replay(zeros, tape, S, shift) of a zeroed bit slab xors the demo's terms into
+    it, and pack_gf2 of make_synthetic_demos' int8 targets gives the same bits (RANGE-flagged ones included: they keep
+    their parity)."""
 
     def __init__(self, records: torch.Tensor, targets: torch.Tensor, S: int, shift: int, target_bound: int | None = None):
         _need_cuda(records, "records", torch.uint8)
