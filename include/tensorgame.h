@@ -38,9 +38,9 @@
  *     steps, keys and ranks are naturally aligned arrays (not checked).
  *
  * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
- * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths, and the change of basis mod 2).  The
- * change of basis over Z (K5) stays {4, 9, 16} and tg_demo_accumulate_tc 16; at 25 tg_demo_gen_philox keeps
- * contract v1 for every alphabet (tg_demo_alias_tables returns TG_E_ARG).
+ * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths, and the change of basis mod 2 with its
+ * inverses).  The change of basis over Z (K5, tg_invert_bases included) stays {4, 9, 16} and tg_demo_accumulate_tc
+ * 16; at 25 tg_demo_gen_philox keeps contract v1 for every alphabet (tg_demo_alias_tables returns TG_E_ARG).
  *
  * Device formats (see DESIGN.md "Data layout")
  *   slab   int8  [B][GP]   residual tensors, entry (i,j,k) at i*RP + j*S + k,
@@ -71,7 +71,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 205
+#define TG_VERSION 206
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -85,6 +85,7 @@ extern "C" {
 #define TG_FLAG_TOKEN_RANGE 16u /* change of basis: a transformed factor entry left [-shift_out, shift_out] */
 #define TG_FLAG_PATH_PLANES 32u /* change of basis, informational: 16x16x16 game computed on int8 byte planes (not f16) */
 #define TG_FLAG_PATH_EXACT 64u  /* change of basis, informational: game computed by the exact int32 kernel (no fast path held it) */
+#define TG_FLAG_SINGULAR 128u   /* basis inversion: a matrix of the triple has no inverse in the output format */
 
 int tg_version(void);
 int tg_last_cuda_error(void);
@@ -343,6 +344,13 @@ int tg_change_of_basis_factors_gf2(const uint8_t *tape_in, int64_t in_step_strid
  * both diagonals 1.  At S <= 16 the result is tg_sample_unimodular of the same arguments mod 2; at 25 the same recipe
  * reads 40 Philox blocks per matrix. */
 int tg_sample_invertible_gf2(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, uint32_t *mats, void *stream);
+/* The inverse triples over GF(2): inv[n][f] = mats[n][f]^-1 mod 2 for f = A, B, C, in the layout of mats (uint32
+ * [N][3][S], bits S to 31 ignored on input and zero on output).  A matrix that is singular over GF(2) is written as S
+ * zero rows and flags[n] = TG_FLAG_SINGULAR; flags[n] = 0 otherwise.  With these, tg_change_of_basis_gf2 and
+ * tg_change_of_basis_factors_gf2 map a transformed tensor and its factors back: a game solved from T' gives a
+ * factorization of T mod 2.  In place (inv == mats) allowed.  Argument rules as above: a bad S or N < 0 returns TG_E_ARG;
+ * N == 0 returns TG_OK; a null mats, inv or flags returns TG_E_ARG; mats and inv must be 4-byte aligned (TG_E_ARG). */
+int tg_invert_bases_gf2(const uint32_t *mats, uint32_t *inv, uint8_t *flags, int64_t N, int S, void *stream);
 
 /* ---- mod-2 training samples: K4 and the float32 conversion on bit slabs (S in {4, 9, 16, 25}) ---------------------- */
 /* SyntheticDemoDataset.__getitem__ (datasets.py:77-122) modulo 2, from a demo-major store with bit-slab targets: the
@@ -422,6 +430,19 @@ int tg_change_of_basis_factors(const uint8_t *tape_in, int64_t in_step_stride, i
  * off-diagonal entries -1/0/+1, P(non-zero) = p_nonzero quantised to 1/128),
  * Philox-keyed by (seed, first + n) like the demo stream -> int8 [N][3][S][S]. */
 int tg_sample_unimodular(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, int8_t *mats, void *stream);
+/* The inverse triples over Z, for mapping factors back from a changed basis (u = A^-1 u', v = B^-1 v', w = C^-1 w' with
+ * tg_change_of_basis_factors): mats and inv int8 [N][3][S][S], (A, B, C) row-major as tg_sample_unimodular writes them.
+ * inv[n][f] is the integer inverse of mats[n][f] when M has an integer inverse whose entries all lie in [-128, 127];
+ * otherwise (det M not +-1, or an inverse entry outside int8) that matrix is written as all zeros and flags[n] =
+ * TG_FLAG_SINGULAR.  flags[n] = 0 for a triple whose three inverses were written.
+ *   Exactness: Gauss-Jordan elimination modulo the prime p = 32749 gives X, lifted to (-p/2, p/2); the matrix passes iff
+ *   every entry of X is in [-128, 127] and M X = I holds exactly (int32).  If an int8 integer inverse Y exists, det M =
+ *   +-1, so M is invertible mod p, X = Y mod p and, as p > 256, the lift is Y; if the check passes, X is one.  So the
+ *   predicate is exact for every input, whatever det M is mod p.
+ * Any byte alignment (slices of an (n, 3, 9, 9) tensor start at odd addresses); in place (inv == mats) allowed.  A bad S
+ * (25 included, as for the rest of K5) or N < 0 returns TG_E_ARG; N == 0 returns TG_OK; a null mats, inv or flags
+ * returns TG_E_ARG. */
+int tg_invert_bases(const int8_t *mats, int8_t *inv, uint8_t *flags, int64_t N, int S, void *stream);
 
 /* ---- host-buffer path (end-to-end through PCIe) -------------------------- */
 typedef struct tg_host_ctx tg_host_ctx;

@@ -32,6 +32,7 @@ FLAG_EXHAUSTED = 8
 FLAG_TOKEN_RANGE = 16
 FLAG_PATH_PLANES = 32
 FLAG_PATH_EXACT = 64
+FLAG_SINGULAR = 128
 
 
 class TensorGameError(RuntimeError):
@@ -140,6 +141,7 @@ _SIGNATURES = {
     "tg_change_of_basis_factors_gf2": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, C.c_int64, C.c_int,
                                                  C.c_int, _vp]),
     "tg_sample_invertible_gf2": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),
+    "tg_invert_bases_gf2": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp]),
     "tg_demo_sample_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp,
                                      _vp]),
     "tg_expand_f32_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
@@ -149,6 +151,7 @@ _SIGNATURES = {
     "tg_change_of_basis_factors": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp, C.c_int64,
                                              C.c_int, C.c_int, _vp]),
     "tg_sample_unimodular": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),
+    "tg_invert_bases": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp]),
     "tg_mt19937_fill_f64": (C.c_int, [C.c_uint32, C.c_int64, C.c_int64, _vp]),
     "tg_mt19937_fill_f64_state": (C.c_int, [_vp, C.c_int, C.c_int64, C.c_int64, _vp]),
     "tg_demo_from_ustream_workspace": (C.c_int64, [C.c_int64, C.c_int]),

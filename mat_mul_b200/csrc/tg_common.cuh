@@ -144,6 +144,23 @@ inline int check_sample_gf2(int S, long long N, double p_nonzero, const void *ma
     return LAUNCH;
 }
 
+// tg_invert_bases: int8 matrices at any byte address (slices of (n, 3, 9, 9) tensors start at odd ones), flags required
+inline int check_invert_bases(int S, long long N, const void *mats, const void *inv, const void *flags) {
+    if (!basis_supported_S(S) || N < 0) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!mats || !inv || !flags) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_invert_bases_gf2: check_basis_gf2's rules for the matrices (4-byte aligned uint32 rows), flags required
+inline int check_invert_bases_gf2(int S, long long N, const void *mats, const void *inv, const void *flags) {
+    if (!supported_S(S) || N < 0) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!mats || !inv || !flags) return TG_E_ARG;
+    if (misaligned(mats, 4) || misaligned(inv, 4)) return TG_E_ARG;
+    return LAUNCH;
+}
+
 // tg_demo_sample_gf2: the rules of tg_demo_sample_dm in its order -- the scalars, an empty batch, null pointers, tape_dm
 // and the targets 16-byte aligned, then replay_shift in [0, 8]; states may start at any float
 inline int check_demo_sample_gf2(int S, long long N, int R, int dim_t, int replay_shift, long long nb, const void *tape_dm,

@@ -14,8 +14,8 @@ from dataclasses import dataclass
 import torch
 
 from . import _lib
-from ._lib import (FLAG_EXHAUSTED, FLAG_NULL, FLAG_PATH_EXACT, FLAG_PATH_PLANES, FLAG_RANGE, FLAG_TERMINAL,  # noqa: F401
-                   FLAG_TOKEN_RANGE, TensorGameError, check)
+from ._lib import (FLAG_EXHAUSTED, FLAG_NULL, FLAG_PATH_EXACT, FLAG_PATH_PLANES, FLAG_RANGE, FLAG_SINGULAR,  # noqa: F401
+                   FLAG_TERMINAL, FLAG_TOKEN_RANGE, TensorGameError, check)
 
 
 @dataclass(frozen=True)
@@ -677,6 +677,50 @@ def change_of_basis(slab: torch.Tensor, mats: torch.Tensor, S: int, tape: torch.
     return (out, tape_out, flags, stats) if return_path_stats else (out, tape_out, flags)
 
 
+def change_of_basis_factors(tape: torch.Tensor, mats: torch.Tensor, S: int, shift: int, shift_out: int | None = None):
+    """u' = A u, v' = B v, w' = C w for every record of a step-major tape (R, N, TP), without a slab
+    (tg_change_of_basis_factors): coefficients are token - shift, tokens out are coefficient + shift_out (default shift,
+    in [1, 127]).  mats int8 (N, 3, S, S) per game or (1, 3, S, S) / (3, S, S) shared.  Returns (tape', flags uint8
+    (N,)): FLAG_TOKEN_RANGE where a transformed entry left [-shift_out, shift_out].  With the triples of invert_bases this
+    maps factors found in a changed basis back to the original one."""
+    _need_cuda(tape, "tape", torch.uint8)
+    _need_cuda(mats, "mats", torch.int8)
+    tp = layout(S).token_pitch
+    if tape.dim() != 3 or tape.shape[2] != tp:
+        raise TensorGameError(f"tape must be (R, N, {tp})")
+    R, N = tape.shape[0], tape.shape[1]
+    m = mats.reshape(-1, 3, S, S)
+    if m.shape[0] not in (1, N):
+        raise TensorGameError("mats must hold one (A,B,C) triple or one per game")
+    tape_out = torch.empty_like(tape)
+    flags = torch.zeros(N, dtype=torch.uint8, device=tape.device)
+    if R == 0:
+        return tape_out, flags
+    _call("tg_change_of_basis_factors", (tape, m, tape_out, flags), _p(tape), N * tp, shift, _p(m), int(m.shape[0] == N and N > 1),
+          _p(tape_out), N * tp, shift if shift_out is None else shift_out, _p(flags), N, R, S)
+    return tape_out, flags
+
+
+def invert_bases(mats: torch.Tensor, out: torch.Tensor | None = None):
+    """The inverse of every matrix of (A, B, C) triples over Z (tg_invert_bases): mats int8 (N, 3, S, S), or (3, S, S) as
+    N = 1, S in {4, 9, 16}.  Returns (inv int8 (N, 3, S, S), flags uint8 (N,)): inv[n, f] is the integer inverse of
+    mats[n, f] where one exists with every entry in [-128, 127]; otherwise that matrix is all zeros and flags[n] =
+    FLAG_SINGULAR.  out may be mats (in place)."""
+    _need_cuda(mats, "mats", torch.int8)
+    S = mats.shape[-1]
+    if mats.dim() not in (3, 4) or mats.shape[-3:] != (3, S, S):
+        raise TensorGameError("mats must be (N, 3, S, S) or (3, S, S)")
+    m = mats.reshape(-1, 3, S, S)
+    out = torch.empty_like(m) if out is None else out
+    _need_cuda(out, "out", torch.int8)
+    if out.numel() != m.numel():
+        raise TensorGameError("out must hold as many matrices as mats")
+    out = out.view(m.shape)
+    flags = torch.empty(m.shape[0], dtype=torch.uint8, device=mats.device)
+    _call("tg_invert_bases", (m, out, flags), _p(m), _p(out), _p(flags), m.shape[0], S)
+    return out, flags
+
+
 # ---------------------------------------------------------------- K5 mod 2
 def sample_invertible_gf2(n: int, S: int, seed: int = 0, first: int = 0, p_nonzero: float = 0.3, device="cuda") -> torch.Tensor:
     """Random (A, B, C) per game, each invertible over GF(2), as bit matrices int32 (n, 3, S): word r of a matrix is its
@@ -725,6 +769,46 @@ def change_of_basis_gf2(bits: torch.Tensor, mats: torch.Tensor, S: int, tape: to
     _call("tg_change_of_basis_factors_gf2", (tape, m, tape_out), _p(tape), N * tp, shift, _p(m), per_game, _p(tape_out), N * tp,
           shift if shift_out is None else shift_out, N, tape.shape[0], S)
     return out, tape_out
+
+
+def change_of_basis_factors_gf2(tape: torch.Tensor, mats: torch.Tensor, S: int, shift: int = 1, shift_out: int | None = None):
+    """u' = A u, v' = B v, w' = C w mod 2 for every record of a step-major tape (R, N, TP), without a bit slab
+    (tg_change_of_basis_factors_gf2): tokens read with `shift`, written as residue + shift_out (default shift), both in
+    [1, 4].  mats: bit matrices int32 (N, 3, S) per game, or (1, 3, S) / (3, S) shared.  Returns tape'."""
+    _need_cuda(tape, "tape", torch.uint8)
+    _need_cuda(mats, "mats", torch.int32)
+    tp = layout(S).token_pitch
+    if tape.dim() != 3 or tape.shape[2] != tp:
+        raise TensorGameError(f"tape must be (R, N, {tp})")
+    R, N = tape.shape[0], tape.shape[1]
+    m = mats.reshape(-1, 3, S)
+    if m.shape[0] not in (1, N):
+        raise TensorGameError("mats must hold one (A,B,C) triple or one per game")
+    tape_out = torch.empty_like(tape)
+    if R == 0:
+        return tape_out
+    _call("tg_change_of_basis_factors_gf2", (tape, m, tape_out), _p(tape), N * tp, shift, _p(m), int(m.shape[0] == N and N > 1),
+          _p(tape_out), N * tp, shift if shift_out is None else shift_out, N, R, S)
+    return tape_out
+
+
+def invert_bases_gf2(mats: torch.Tensor, out: torch.Tensor | None = None):
+    """The inverse over GF(2) of every matrix of bit-matrix triples (tg_invert_bases_gf2): mats int32 (N, 3, S), or (3, S)
+    as N = 1, S in {4, 9, 16, 25}; bits S to 31 of a row are ignored.  Returns (inv int32 (N, 3, S), flags uint8 (N,)):
+    a matrix singular over GF(2) comes back as zero rows with flags[n] = FLAG_SINGULAR.  out may be mats (in place)."""
+    _need_cuda(mats, "mats", torch.int32)
+    S = mats.shape[-1]
+    if mats.dim() not in (2, 3) or mats.shape[-2] != 3:
+        raise TensorGameError("mats must be (N, 3, S) or (3, S)")
+    m = mats.reshape(-1, 3, S)
+    out = torch.empty_like(m) if out is None else out
+    _need_cuda(out, "out", torch.int32)
+    if out.numel() != m.numel():
+        raise TensorGameError("out must hold as many matrices as mats")
+    out = out.view(m.shape)
+    flags = torch.empty(m.shape[0], dtype=torch.uint8, device=mats.device)
+    _call("tg_invert_bases_gf2", (m, out, flags), _p(m), _p(out), _p(flags), m.shape[0], S)
+    return out, flags
 
 
 def bind_host_to_gpu(device: int = 0) -> list[int]:
