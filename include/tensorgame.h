@@ -23,7 +23,10 @@
  *     zeroes a per-launch work counter in static device memory on `stream`.
  *   - *_host entry points take HOST pointers (pinned for full speed), move the
  *     data themselves through a caller-created tg_host_ctx and return after
- *     the results are in host memory.
+ *     the results are in host memory.  They allocate only inside the context:
+ *     the first int16 call grows its slab staging from GP to 2 GP bytes per
+ *     game of a chunk (after a cudaDeviceSynchronize), as a K-step call grows
+ *     its tape staging; a context that never sees int16 keeps its size.
  *   - return value: 0 on success, a negative TG_E_* code otherwise; nothing
  *     throws.  There is no CPU fallback: without a CUDA device every compute
  *     entry point returns TG_E_CUDA.
@@ -71,7 +74,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 206
+#define TG_VERSION 207
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -445,13 +448,26 @@ int tg_sample_unimodular(uint64_t seed, uint64_t first, int64_t N, int S, double
 int tg_invert_bases(const int8_t *mats, int8_t *inv, uint8_t *flags, int64_t N, int S, void *stream);
 
 /* ---- host-buffer path (end-to-end through PCIe) -------------------------- */
+/* For callers whose games live in host memory: chunks of up to max_chunk games (in every slab format) flow through three
+ * dedicated streams -- H2D copies, device calls, D2H copies -- chained by events per staging buffer, so that both copy
+ * engines stream back to back.  Every call returns when its results are in host memory.
+ *   - Results: every output equals, byte for byte, what the device twin writes on the whole batch; the chunking does not
+ *     show (demos are keyed by their global index first_demo + n).
+ *   - Host buffers may be pinned (full speed) or pageable and need only their element type's alignment; in place
+ *     (slab_out == slab_in) is allowed: each chunk's download writes only the games its own upload read.
+ *   - Tapes are dense and step-major: [B][TP] for a step, [K][B][TP] for a rollout, [R][N][TP] for demos.
+ *   - Argument rules, in order: a null context, B (N) < 0, K < 0 or R < 1 returns TG_E_ARG; B == 0 returns TG_OK; a null
+ *     pointer the call needs returns TG_E_ARG; then the device twin's own checks (shift outside [1, 4], an alphabet the
+ *     generator refuses, ...) return TG_E_ARG.  All of them run before the first copy is enqueued, and a call that fails
+ *     returns with no copy from or to the caller's memory in flight.
+ *   - Bytes per game-step across PCIe (slab in + tape + slab out + flags + nnz): int8 2 GP + TP + 5, int16 4 GP + TP + 5,
+ *     bits 2 GB + TP + 5 -- 149 / 277 / 53 B at 4x4x4, 1573 / 3109 / 261 B at 9x9x9, 8245 / 16437 / 1077 B at 16x16x16,
+ *     31509 / 62933 / 4085 B at 25x25x25: a mod-2 game crosses in 1/2.8 to 1/7.7 of the int8 bytes. */
 typedef struct tg_host_ctx tg_host_ctx;
 /* creates three streams, events and four device staging buffers for chunks of up to max_chunk games */
 int tg_host_ctx_create(tg_host_ctx **ctx, int device, int S, int64_t max_chunk);
 int tg_host_ctx_destroy(tg_host_ctx *ctx);
-/* same contract as tg_step with HOST slabs/tapes/flags/nnz; chunks flow
- * through dedicated H2D / kernel / D2H streams chained by events per staging
- * buffer (both copy engines stream back to back); returns when done. */
+/* tg_step with HOST slabs/tapes/flags/nnz. */
 int tg_step_host(tg_host_ctx *ctx, const int8_t *slab_in, const uint8_t *tape, int8_t *slab_out, uint8_t *flags,
                  int32_t *nnz, int64_t B, int shift);
 /* tg_rollout with HOST buffers: the slab crosses PCIe once per K steps instead of once per step -- the case where the
@@ -464,6 +480,20 @@ int tg_rollout_host(tg_host_ctx *ctx, const int8_t *slab_in, const uint8_t *tape
  * datasets.py:124-142 for a caller that wants the demonstrations in host memory. */
 int tg_demo_gen_host(tg_host_ctx *ctx, uint64_t seed, uint64_t first_demo, int64_t N, int R, int shift, const int8_t *values,
                      const double *probs, int n_values, int max_tries, uint8_t *tape, int8_t *slab, uint8_t *flags);
+/* The int16 twins: tg_step_i16 / tg_rollout_i16 with HOST int16 slabs [B][GP] of int16 (2-byte aligned). */
+int tg_step_host_i16(tg_host_ctx *ctx, const int16_t *slab_in, const uint8_t *tape, int16_t *slab_out, uint8_t *flags,
+                     int32_t *nnz, int64_t B, int shift);
+int tg_rollout_host_i16(tg_host_ctx *ctx, const int16_t *slab_in, const uint8_t *tape, int K, int16_t *slab_out,
+                        uint8_t *flags, int32_t *nnz, int32_t *steps, int64_t B, int shift);
+/* The mod-2 twins: tg_step_gf2 / tg_rollout_gf2 with HOST bit slabs uint32 [B][GB/4] (4-byte aligned), and
+ * tg_demo_gen_gf2 into a HOST tape [R][N][TP], bit slab [N][GB/4] and flags [N]. */
+int tg_step_host_gf2(tg_host_ctx *ctx, const uint32_t *bits_in, const uint8_t *tape, uint32_t *bits_out, uint8_t *flags,
+                     int32_t *nnz, int64_t B, int shift);
+int tg_rollout_host_gf2(tg_host_ctx *ctx, const uint32_t *bits_in, const uint8_t *tape, int K, uint32_t *bits_out,
+                        uint8_t *flags, int32_t *nnz, int32_t *steps, int64_t B, int shift);
+int tg_demo_gen_host_gf2(tg_host_ctx *ctx, uint64_t seed, uint64_t first_demo, int64_t N, int R, int shift,
+                         const int8_t *values, const double *probs, int n_values, int max_tries, uint8_t *tape,
+                         uint32_t *bits, uint8_t *flags);
 
 #ifdef TG_TUNING
 /* Sweep build only (-DTG_TUNING, libtensorgame_b200_tuning.so): CTAs launched per SM (0 = default) and kernel

@@ -163,6 +163,12 @@ _SIGNATURES = {
     "tg_rollout_host": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
     "tg_demo_gen_host": (C.c_int, [_vp, C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
                                    _vp, _vp, _vp]),
+    "tg_step_host_i16": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
+    "tg_rollout_host_i16": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
+    "tg_step_host_gf2": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
+    "tg_rollout_host_gf2": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
+    "tg_demo_gen_host_gf2": (C.c_int, [_vp, C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
+                                       _vp, _vp, _vp]),
 }
 if TUNING:  # sweep build only (declared under TG_TUNING in include/tensorgame.h)
     _SIGNATURES["tg_tune_step_ctas_per_sm"] = (C.c_int, [C.c_int])

@@ -836,12 +836,33 @@ def bind_host_to_gpu(device: int = 0) -> list[int]:
 class HostStepper:
     """End-to-end step for callers whose data lives in host memory (pinned
     numpy/torch CPU buffers): chunked H2D -> tg_step -> D2H over three streams
-    inside the C library (tg_step_host)."""
+    inside the C library (tg_step_host).
+
+    step and rollout take int8 slabs (B, GP), int16 slabs (B, GP) or int32 bit slabs (B, GB/4) and dispatch on the
+    dtype as step_batch does (tg_step_host, tg_step_host_i16, tg_step_host_gf2); make_demos takes an int8 slab or an
+    int32 bit slab for the targets.  One context serves every format; the first int16 call doubles its slab staging."""
 
     def __init__(self, S: int, device: int = 0, chunk: int = 1 << 16):
         self.S, self.lay = S, layout(S)
         self._ctx = C.c_void_p()
         check(_lib.lib().tg_host_ctx_create(C.byref(self._ctx), device, S, chunk), "tg_host_ctx_create")
+
+    def _host_format(self, slab: torch.Tensor, out: torch.Tensor, records: torch.Tensor, steps: bool, B: int,
+                     *per_game: torch.Tensor) -> str:
+        """The entry-point suffix of an int16 or bit-slab call ("_i16" / "_gf2") after checking its shapes: slab and out
+        (B, GP) int16 or (B, GB/4) int32, records uint8 (B, TP) or, with steps, a step-major tape (K, B, TP), per-game
+        arrays of B elements."""
+        sfx = _SLAB_SUFFIX[slab.dtype]
+        width = _game_pitch(sfx, self.S)
+        for name, t in (("slab", slab), ("out", out)):
+            if t.dtype != slab.dtype or t.dim() != 2 or tuple(t.shape) != (B, width):
+                raise TensorGameError(f"HostStepper: {name} must be {slab.dtype} ({B}, {width})")
+        shape = (records.shape[0],) * steps + (B, self.lay.token_pitch)
+        if records.dtype != torch.uint8 or records.dim() != 2 + steps or tuple(records.shape) != shape:
+            raise TensorGameError(f"HostStepper: the tape must be uint8 ({'K, ' * steps}{B}, {self.lay.token_pitch})")
+        if any(t.numel() != B for t in per_game):
+            raise TensorGameError(f"HostStepper: flags, nnz and steps must hold {B} games")
+        return sfx
 
     def step(self, slab: torch.Tensor, tape: torch.Tensor, out: torch.Tensor, flags: torch.Tensor, nnz: torch.Tensor,
              shift: int) -> None:
@@ -849,6 +870,10 @@ class HostStepper:
             if t.is_cuda or not t.is_contiguous():
                 raise TensorGameError("HostStepper takes contiguous CPU tensors")
         B = slab.shape[0]
+        if slab.dtype in _SLAB_SUFFIX:
+            name = "tg_step_host" + self._host_format(slab, out, tape, False, B, flags, nnz)
+            check(getattr(_lib.lib(), name)(self._ctx, _p(slab), _p(tape), _p(out), _p(flags), _p(nnz), B, shift), name)
+            return
         check(_lib.lib().tg_step_host(self._ctx, _p(slab), _p(tape), _p(out), _p(flags), _p(nnz), B, shift), "tg_step_host")
 
     def rollout(self, slab: torch.Tensor, tape: torch.Tensor, out: torch.Tensor, flags: torch.Tensor, nnz: torch.Tensor,
@@ -858,17 +883,29 @@ class HostStepper:
             if t.is_cuda or not t.is_contiguous():
                 raise TensorGameError("HostStepper takes contiguous CPU tensors")
         K, B = tape.shape[0], slab.shape[0]
+        if slab.dtype in _SLAB_SUFFIX:
+            name = "tg_rollout_host" + self._host_format(slab, out, tape, True, B, flags, nnz, steps)
+            check(getattr(_lib.lib(), name)(self._ctx, _p(slab), _p(tape), K, _p(out), _p(flags), _p(nnz), _p(steps), B, shift), name)
+            return
         check(_lib.lib().tg_rollout_host(self._ctx, _p(slab), _p(tape), K, _p(out), _p(flags), _p(nnz), _p(steps), B, shift),
               "tg_rollout_host")
 
     def make_demos(self, tape: torch.Tensor, slab: torch.Tensor, flags: torch.Tensor, shift: int, values, probs, seed: int = 0,
                    first_demo: int = 0, max_tries: int = 64) -> None:
-        """Synthetic demonstrations straight into CPU buffers (tg_demo_gen_host): tape (R, N, TP), slab (N, GP), flags (N,)."""
+        """Synthetic demonstrations straight into CPU buffers (tg_demo_gen_host): tape (R, N, TP), slab (N, GP), flags (N,).
+        An int32 bit slab (N, GB/4) takes the demos modulo 2 (tg_demo_gen_host_gf2, the demos of make_synthetic_demos_gf2)."""
         for t in (tape, slab, flags):
             if t.is_cuda or not t.is_contiguous():
                 raise TensorGameError("HostStepper takes contiguous CPU tensors")
         v, p = _cat_arrays(values, probs)
         R, N = tape.shape[0], tape.shape[1]
+        if slab.dtype == torch.int16:
+            raise TensorGameError("HostStepper.make_demos writes int8 slabs or int32 bit slabs, not int16 targets")
+        if slab.dtype == torch.int32:
+            name = "tg_demo_gen_host" + self._host_format(slab, slab, tape, True, N, flags)
+            check(getattr(_lib.lib(), name)(self._ctx, seed, first_demo, N, R, shift, v.ctypes.data, p.ctypes.data, len(v), max_tries,
+                                            _p(tape), _p(slab), _p(flags)), name)
+            return
         check(_lib.lib().tg_demo_gen_host(self._ctx, seed, first_demo, N, R, shift, v.ctypes.data, p.ctypes.data, len(v), max_tries,
                                           _p(tape), _p(slab), _p(flags)), "tg_demo_gen_host")
 
