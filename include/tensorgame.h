@@ -30,15 +30,21 @@
  *   - return value: 0 on success, a negative TG_E_* code otherwise; nothing
  *     throws.  There is no CPU fallback: without a CUDA device every compute
  *     entry point returns TG_E_CUDA.
- *   - argument rules of the game path (tg_step, tg_expand_children,
- *     tg_rollout, tg_replay, tg_state_key, tg_slice_rank and the conversions,
- *     for every slab format), checked in this order: a bad scalar (S, B < 0,
- *     shift outside [1, 4], k < 1, K < 0) returns TG_E_ARG; an empty batch
- *     (B == 0) returns TG_OK before any pointer is looked at; a null pointer
+ *   - argument rules of every device entry point, checked in this order: a
+ *     bad scalar returns TG_E_ARG; an empty batch (B, N or nb == 0) returns
+ *     TG_OK before any pointer is looked at and writes nothing; a null pointer
  *     the call needs returns TG_E_ARG; a misaligned buffer returns TG_E_ARG.
- *     Slabs of every format, tapes and tape_step_stride are 16-byte aligned,
- *     float32 arrays 4-byte and int64 token arrays 8-byte aligned; flags, nnz,
- *     steps, keys and ranks are naturally aligned arrays (not checked).
+ *     Bad scalars: S outside the call's sizes (below), a negative batch, R < 1
+ *     (R > 65535 for the demo generators), shift outside [1, 4] (the
+ *     exceptions are stated with their calls), k < 1, K < 0, dim_t < 1,
+ *     target_bound < 0, n_values outside [1, 8], max_tries outside
+ *     [1, 65535], p_nonzero outside [0, 1] or NaN.
+ *     Slabs of every format, tapes, demo-major records, the targets of the
+ *     sample batchers and every tape step stride are 16-byte aligned (the
+ *     exceptions are stated with their calls), float32 arrays and GF(2)
+ *     matrices 4-byte, int64 token arrays 8-byte aligned; int8 matrices,
+ *     flags, nnz, steps, keys, ranks, idx and the sample outputs are naturally
+ *     aligned arrays (not checked).
  *
  * Sizes: S = dim_3d in {4, 9, 16, 25} on the game path (layout, conversions,
  * K1-K4, K6-K8, parity mode, host buffers, the int16 and mod-2 game paths, and the change of basis mod 2 with its
@@ -206,7 +212,8 @@ int tg_demo_accumulate_tc(const uint8_t *tape, int64_t tape_step_stride, int64_t
  * that stream exactly as the reference's rejection loop does (utils.py:
  * 222-232; Categorical == multinomial, float32 CDF) and emits the first N
  * demos: result[0] = demos completed (<= N), result[1] = doubles consumed by
- * them.  workspace: tg_demo_from_ustream_workspace(n_u, S) bytes, 16-aligned. */
+ * them.  workspace: tg_demo_from_ustream_workspace(n_u, S) bytes, 16-aligned
+ * (TG_E_ARG when smaller).  N == 0 leaves result unwritten. */
 int tg_mt19937_fill_f64(uint32_t seed, int64_t skip, int64_t n, double *out_host);
 int tg_mt19937_fill_f64_state(const uint32_t *state624, int pos, int64_t skip, int64_t n, double *out_host);
 int64_t tg_demo_from_ustream_workspace(int64_t n_u, int S);
@@ -220,7 +227,8 @@ int tg_demo_from_ustream(const double *u, int64_t n_u, const int8_t *values, con
  * + target slab): states float32 [nb][dim_t][S][S][S], scalars [nb] = R - a,
  * actions int64 [nb][3S], rewards [nb] = -(a+1).  replay_shift is the shift
  * action_to_tensor applies while replaying (the reference hard-codes 1,
- * utils.py:88-96); pass the demos' own shift for the true residual. */
+ * utils.py:88-96); pass the demos' own shift for the true residual.  Any
+ * replay_shift goes, and the tape (not the slab) may start at any byte. */
 int tg_demo_sample(const uint8_t *tape, int64_t tape_step_stride, const int8_t *slab, int64_t N, int R, int S, int dim_t,
                    int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
                    float *rewards, void *stream);
@@ -231,7 +239,8 @@ int tg_demo_sample(const uint8_t *tape, int64_t tape_step_stride, const int8_t *
  * are kept in, tg_demo_accumulate_i16).  target_bound >= max |target entry| (127 for an int8 slab) selects the packed
  * 16-bit arithmetic when target_bound + R * cmax^3 fits an int16.  Inputs and outputs move by TMA bulk copies; states may
  * start at any float (16-byte aligned batches leave with one bulk store per CTA).  Samples whose index is out of range
- * get all-zero states (scalars / actions / rewards untouched). */
+ * get all-zero states (scalars / actions / rewards untouched).  replay_shift outside [0, 8] returns TG_E_ARG, tested
+ * after the alignment (an empty batch takes any). */
 int tg_demo_sample_dm(const uint8_t *tape_dm, const void *targets, int targets_i16, int target_bound, int64_t N, int R, int S,
                       int dim_t, int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
                       float *rewards, void *stream);
@@ -329,10 +338,7 @@ int tg_slice_rank_gf2(const uint32_t *bits, int32_t *ranks, int64_t B, int S, vo
  *   mats  uint32 [N or 1][3][S]  a triple (A, B, C) mod 2: word r of matrix f is row r, bit c is M[r][c] mod 2; bits S to
  *                          31 are ignored.  4-byte aligned; per_game != 0: one triple per game, otherwise one shared triple.
  *                          In torch an int32 tensor (N, 3, S).
- * Over GF(2) no entry and no token can leave its format, so none of the three takes a flags array.  Argument rules as on
- * the game path: a bad scalar (S, N < 0, R < 1, shift_in or shift_out outside [1, 4], p_nonzero outside [0, 1] or NaN)
- * returns TG_E_ARG; N == 0 returns TG_OK; a null pointer returns TG_E_ARG; bit slabs, tapes and step strides must be
- * 16-byte aligned and mats 4-byte aligned (TG_E_ARG). */
+ * Over GF(2) no entry and no token can leave its format, so none of the three takes a flags array. */
 /* T' = T x1 A x2 B x3 C over GF(2); in place allowed; padding bits and words of the output zero */
 int tg_change_of_basis_gf2(const uint32_t *bits_in, const uint32_t *mats, int per_game, uint32_t *bits_out, int64_t N, int S,
                            void *stream);
@@ -351,8 +357,7 @@ int tg_sample_invertible_gf2(uint64_t seed, uint64_t first, int64_t N, int S, do
  * [N][3][S], bits S to 31 ignored on input and zero on output).  A matrix that is singular over GF(2) is written as S
  * zero rows and flags[n] = TG_FLAG_SINGULAR; flags[n] = 0 otherwise.  With these, tg_change_of_basis_gf2 and
  * tg_change_of_basis_factors_gf2 map a transformed tensor and its factors back: a game solved from T' gives a
- * factorization of T mod 2.  In place (inv == mats) allowed.  Argument rules as above: a bad S or N < 0 returns TG_E_ARG;
- * N == 0 returns TG_OK; a null mats, inv or flags returns TG_E_ARG; mats and inv must be 4-byte aligned (TG_E_ARG). */
+ * factorization of T mod 2.  In place (inv == mats) allowed; flags is required. */
 int tg_invert_bases_gf2(const uint32_t *mats, uint32_t *inv, uint8_t *flags, int64_t N, int S, void *stream);
 
 /* ---- mod-2 training samples: K4 and the float32 conversion on bit slabs (S in {4, 9, 16, 25}) ---------------------- */
@@ -366,16 +371,13 @@ int tg_invert_bases_gf2(const uint32_t *mats, uint32_t *inv, uint8_t *flags, int
  *   - entries 0.0f or 1.0f, dense (dim_t, S, S, S) per sample; states may start at any float;
  *   - scalars = R - a, actions = the record's 3S tokens as int64, rewards = -(a+1), as tg_demo_sample_dm writes them;
  *   - an index outside [0, N*R) gets all-zero states, its other outputs untouched.
- * Checks in tg_demo_sample_dm's order: a bad scalar (S, N < 0, R < 1, dim_t < 1, nb < 0) returns TG_E_ARG; nb == 0
- * returns TG_OK; a null pointer returns TG_E_ARG; tape_dm and the targets must be 16-byte aligned (TG_E_ARG); then
- * replay_shift outside [0, 8] returns TG_E_ARG.  Records are read from the store as they are replayed, so R has no upper
- * bound. */
+ * replay_shift is checked as there.  Records are read from the store as they are replayed, so R has no upper bound. */
 int tg_demo_sample_gf2(const uint8_t *tape_dm, const uint32_t *targets_bits, int64_t N, int R, int S, int dim_t,
                        int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
                        float *rewards, void *stream);
 /* bit slab -> float32 dense (S,S,S) of 0.0f / 1.0f at dst + b*dst_stride: the state the model consumes;
- * tg_expand_f32(tg_unpack_gf2(bits)) in one pass.  The game path's argument rules (bits 16-byte aligned, dst 4-byte);
- * dst may start at any float, and floats outside each game's S^3 are not written. */
+ * tg_expand_f32(tg_unpack_gf2(bits)) in one pass.  dst may start at any float, and floats outside each game's S^3 are
+ * not written. */
 int tg_expand_f32_gf2(const uint32_t *bits, float *dst, int64_t dst_stride, int64_t B, int S, void *stream);
 
 /* ---- mod-2 synthetic demonstrations: K3 with bit-slab targets (S in {4, 9, 16, 25}) -------------------------------- */
@@ -392,11 +394,8 @@ int tg_expand_f32_gf2(const uint32_t *bits, float *dst, int64_t dst_stride, int6
  *   and the demo gets TG_FLAG_EXHAUSTED.
  * Writes the tape (tokens = value + shift, step-major [R][N][TP], padding zero, tape_step_stride as there), the bit
  * target = the xor of the R terms mod 2 (padding bits and words zero) and flags (may be NULL): TG_FLAG_EXHAUSTED or 0;
- * TG_FLAG_RANGE is never raised.  Checks in tg_demo_gen_philox's order: a bad scalar (S, N < 0, R outside [1, 65535],
- * shift outside [1, 4], n_values outside [1, 8], max_tries outside [1, 65535]) returns TG_E_ARG; N == 0 returns TG_OK;
- * a null values, probs, tape or bits returns TG_E_ARG; a misaligned tape, step stride or bit slab returns TG_E_ARG;
- * then a negative or NaN probability, a zero sum, a value outside [-shift, shift] or an alphabet with no odd value
- * returns TG_E_ARG.
+ * TG_FLAG_RANGE is never raised.  After the argument rules, a negative or NaN probability, a zero sum, a value outside
+ * [-shift, shift] or an alphabet with no odd value returns TG_E_ARG.
  * Where 0 is the only even value (listed once) and, under v1, the last value is odd, the tables and the accept rule are
  * the integer ones: the tape is tg_demo_gen_philox's byte for byte, the bits are tg_pack_gf2 of its targets and the
  * EXHAUSTED flags are the same -- a mod-2 run and an integer run with one seed see the same demos. */
@@ -425,7 +424,9 @@ int tg_change_of_basis_i16(const int8_t *slab_in, const int8_t *mats, int per_ga
                            int S, void *stream);
 /* factors follow: u' = A u, v' = B v, w' = C w for every step of a step-major
  * tape; token' = coef' + shift_out.  ORs TG_FLAG_TOKEN_RANGE into flags[n] if a
- * transformed entry leaves [-shift_out, shift_out] (flags must be initialised). */
+ * transformed entry leaves [-shift_out, shift_out] (flags required and
+ * initialised).  shift_in >= 0 and shift_out in [1, 127]; tape_out and its
+ * step stride may have any alignment. */
 int tg_change_of_basis_factors(const uint8_t *tape_in, int64_t in_step_stride, int shift_in, const int8_t *mats, int per_game,
                                uint8_t *tape_out, int64_t out_step_stride, int shift_out, uint8_t *flags, int64_t N, int R,
                                int S, void *stream);
@@ -442,9 +443,8 @@ int tg_sample_unimodular(uint64_t seed, uint64_t first, int64_t N, int S, double
  *   every entry of X is in [-128, 127] and M X = I holds exactly (int32).  If an int8 integer inverse Y exists, det M =
  *   +-1, so M is invertible mod p, X = Y mod p and, as p > 256, the lift is Y; if the check passes, X is one.  So the
  *   predicate is exact for every input, whatever det M is mod p.
- * Any byte alignment (slices of an (n, 3, 9, 9) tensor start at odd addresses); in place (inv == mats) allowed.  A bad S
- * (25 included, as for the rest of K5) or N < 0 returns TG_E_ARG; N == 0 returns TG_OK; a null mats, inv or flags
- * returns TG_E_ARG. */
+ * Any byte alignment (slices of an (n, 3, 9, 9) tensor start at odd addresses); in place (inv == mats) allowed; flags is
+ * required. */
 int tg_invert_bases(const int8_t *mats, int8_t *inv, uint8_t *flags, int64_t N, int S, void *stream);
 
 /* ---- host-buffer path (end-to-end through PCIe) -------------------------- */

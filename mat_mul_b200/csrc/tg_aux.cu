@@ -247,9 +247,10 @@ __global__ void __launch_bounds__(128, PACK16 ? (S == 16 ? 6 : (S == 25 ? 3 : 8)
 // entries in the same instruction.
 template <int S>
 struct SampleCfg {
+    static_assert(S == 9 || S == 16, "4x4x4 and 25x25x25 samples have kernels of their own");
     using G = Geo<S>;
-    static constexpr int SPC = S == 4 ? 32 : (S == 9 ? 4 : 2);       // samples per CTA: SPC * dim_t * S^3 * 4 bytes is a multiple of 16
-    static constexpr int NT = ((SPC * G::WR + 31) / 32) * 32;         // 128 / 96 / 128
+    static constexpr int SPC = S == 9 ? 4 : 2;                        // samples per CTA: SPC * dim_t * S^3 * 4 bytes is a multiple of 16
+    static constexpr int NT = ((SPC * G::WR + 31) / 32) * 32;         // 96 / 128
     static __host__ __device__ constexpr long long smem_bytes(int R, int dim_t, bool tgt16) {
         return (((long long)SPC * dim_t * G::S3 * 4 + 15) & ~15LL) + (long long)SPC * R * G::TP + (long long)SPC * G::GP * (tgt16 ? 2 : 1) +
                ((SPC * 4 + 15) & ~15) + 16;
@@ -386,12 +387,8 @@ __global__ void __launch_bounds__(SampleCfg<S>::NT)
                 const int p0 = (inA[0] ? nvA : nvB) * (int)rec[offw[0]], p1 = (inA[1] ? nvA : nvB) * (int)rec[offw[1]],
                           p2 = (inA[2] ? nvA : nvB) * (int)rec[offw[2]], p3 = (inA[3] ? nvA : nvB) * (int)rec[offw[3]];
                 uint32_t uq[4];
-                if constexpr (S <= 4) {
-                    uq[0] = *reinterpret_cast<const uint32_t *>(rec);
-                } else {
-                    const uint4 q4 = *reinterpret_cast<const uint4 *>(rec);
-                    uq[0] = q4.x, uq[1] = q4.y, uq[2] = q4.z, uq[3] = q4.w;
-                }
+                const uint4 q4 = *reinterpret_cast<const uint4 *>(rec);
+                uq[0] = q4.x, uq[1] = q4.y, uq[2] = q4.z, uq[3] = q4.w;
                 const int np0 = p0 + p1 * 65536, np1 = p2 + p3 * 65536;
 #pragma unroll
                 for (int i = 0; i < S; i++) {
@@ -1280,9 +1277,8 @@ extern "C" {
 int tg_demo_sample(const uint8_t *tape, int64_t tape_step_stride, const int8_t *slab, int64_t N, int R, int S, int dim_t,
                    int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
                    float *rewards, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || dim_t < 1 || nb < 0) return TG_E_ARG;
-    if (nb == 0) return TG_OK;
-    if (!tape || !slab || !idx || !states || !scalars || !actions || !rewards) return TG_E_ARG;
+    const int rc = tg::check_demo_sample(S, N, R, dim_t, 0, nb, false, replay_shift, tape, slab, idx, states, scalars, actions, rewards);
+    if (rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // tokens are <= 2 * 4 (tape contract), so |coefficient| <= cmax; the 16-bit packed head is exact while
     // 127 + R * cmax^3 fits an int16 lane
@@ -1301,93 +1297,57 @@ int tg_demo_sample(const uint8_t *tape, int64_t tape_step_stride, const int8_t *
 int tg_demo_sample_dm(const uint8_t *tape_dm, const void *targets, int targets_i16, int target_bound, int64_t N, int R, int S,
                       int dim_t, int replay_shift, const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions,
                       float *rewards, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || dim_t < 1 || nb < 0 || target_bound < 0) return TG_E_ARG;
-    if (nb == 0) return TG_OK;
-    if (!tape_dm || !targets || !idx || !states || !scalars || !actions || !rewards) return TG_E_ARG;
-    if (((uintptr_t)tape_dm | (uintptr_t)targets) & 15) return TG_E_ARG;
-    if (replay_shift < 0 || replay_shift > 8) return TG_E_ARG;
+    const int rc = tg::check_demo_sample(S, N, R, dim_t, target_bound, nb, true, replay_shift, tape_dm, targets, idx, states, scalars,
+                                         actions, rewards);
+    if (rc != tg::LAUNCH) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     // tokens are <= 8 (tape contract), so |coefficient| <= cmax; the 16-bit packed head is exact while
     // target_bound + R * cmax^3 fits an int16 lane
     const long long cmax = replay_shift > 8 - replay_shift ? replay_shift : 8 - replay_shift;
     const bool pack16 = (long long)target_bound + (long long)R * cmax * cmax * cmax <= 32767;
-    if (S == 9 && pack16 && (long long)tg::rows9::WARPS * tg::rows9::warp_bytes(R) <= 200 * 1024) {
-        // 9x9x9: one thread per (sample, row), three samples per warp
-        const int smem = tg::rows9::WARPS * tg::rows9::warp_bytes(R);
-        const long long per_cta = (long long)tg::rows9::WARPS * tg::rows9::SPW;
-        const long long want = (nb + per_cta - 1) / per_cta;
-        const unsigned grid = (unsigned)(want < 148 * 4 ? want : 148 * 4); // persistent warps: four CTAs per SM
-        unsigned long long *ticket = nullptr;
-        cudaEvent_t done = nullptr;
-        const int trc = tg::ticket_acquire(st, &ticket, &done);
-        if (trc != TG_OK) return trc;
-        if (targets_i16) {
-            auto kern = tg::rows9::demo_sample_rows9_kernel<true, true>;
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        if constexpr (kS == 4) { // one thread per (sample, row), exact int32 (any target bound)
+            auto kern = targets_i16 ? tg::rows4::demo_sample_rows4_kernel<true> : tg::rows4::demo_sample_rows4_kernel<false>;
+            kern<<<(unsigned)((nb * 4 + 127) / 128), 128, 0, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift,
+                                                                   (const long long *)idx, nb, states, scalars, (long long *)actions, rewards);
+        } else if constexpr (kS == 25) { // one CTA per sample, states straight from the registers
+            const long long smem = (long long)R * tg::Geo<25>::TP;
+            if (smem > 227 * 1024 || nb > 0x7FFFFFFFLL) return TG_E_ARG;
+            auto kern = targets_i16 ? (pack16 ? tg::demo_sample_dm25_kernel<true, true> : tg::demo_sample_dm25_kernel<true, false>)
+                                    : (pack16 ? tg::demo_sample_dm25_kernel<false, true> : tg::demo_sample_dm25_kernel<false, false>);
+            TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            kern<<<(unsigned)nb, 160, (size_t)smem, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift, (const long long *)idx,
+                                                         states, scalars, (long long *)actions, rewards);
+        } else if (kS == 9 && pack16 && (long long)tg::rows9::WARPS * tg::rows9::warp_bytes(R) <= 200 * 1024) {
+            // 9x9x9: one thread per (sample, row), three samples per warp
+            const int smem = tg::rows9::WARPS * tg::rows9::warp_bytes(R);
+            const long long per_cta = (long long)tg::rows9::WARPS * tg::rows9::SPW;
+            const long long want = (nb + per_cta - 1) / per_cta;
+            const unsigned grid = (unsigned)(want < 148 * 4 ? want : 148 * 4); // persistent warps: four CTAs per SM
+            unsigned long long *ticket = nullptr;
+            cudaEvent_t done = nullptr;
+            if (const int trc = tg::ticket_acquire(st, &ticket, &done); trc != TG_OK) return trc;
+            auto kern = targets_i16 ? tg::rows9::demo_sample_rows9_kernel<true, true> : tg::rows9::demo_sample_rows9_kernel<false, true>;
             TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
             kern<<<grid, 32 * tg::rows9::WARPS, smem, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift, (const long long *)idx,
                                                             nb, states, scalars, (long long *)actions, rewards, ticket);
+            TG_CUDA(cudaGetLastError());
+            TG_CUDA(cudaEventRecord(done, st));
+            return TG_OK;
         } else {
-            auto kern = tg::rows9::demo_sample_rows9_kernel<false, true>;
-            TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-            kern<<<grid, 32 * tg::rows9::WARPS, smem, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift, (const long long *)idx,
-                                                            nb, states, scalars, (long long *)actions, rewards, ticket);
+            const int lrc = tg::launch_demo_sample_dm<kS>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t,
+                                                          replay_shift, (const long long *)idx, nb, states, scalars, (long long *)actions,
+                                                          rewards, st);
+            if (lrc != TG_OK) return lrc;
         }
         TG_CUDA(cudaGetLastError());
-        TG_CUDA(cudaEventRecord(done, st));
         return TG_OK;
-    }
-    if (S == 4) { // one thread per (sample, row), exact int32 (any target bound)
-        const long long threads = nb * 4;
-        const unsigned grid = (unsigned)((threads + 127) / 128);
-        if (targets_i16)
-            tg::rows4::demo_sample_rows4_kernel<true><<<grid, 128, 0, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift,
-                                                                         (const long long *)idx, nb, states, scalars, (long long *)actions, rewards);
-        else
-            tg::rows4::demo_sample_rows4_kernel<false><<<grid, 128, 0, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift,
-                                                                          (const long long *)idx, nb, states, scalars, (long long *)actions, rewards);
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
-    }
-    if (S == 25) { // one CTA per sample, states straight from the registers
-        const long long smem = (long long)R * tg::Geo<25>::TP;
-        if (smem > 227 * 1024 || nb > 0x7FFFFFFFLL) return TG_E_ARG;
-#define TG_DM25(T16, P16)                                                                                                     \
-    {                                                                                                                         \
-        auto kern = tg::demo_sample_dm25_kernel<T16, P16>;                                                                    \
-        TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                          \
-        kern<<<(unsigned)nb, 160, (size_t)smem, st>>>(tape_dm, (const uint8_t *)targets, N, R, dim_t, replay_shift, (const long long *)idx, \
-                                                     states, scalars, (long long *)actions, rewards);                         \
-    }
-        if (targets_i16) {
-            if (pack16) TG_DM25(true, true) else TG_DM25(true, false)
-        } else {
-            if (pack16) TG_DM25(false, true) else TG_DM25(false, false)
-        }
-#undef TG_DM25
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
-    }
-    switch (S) {
-    case 4: { const int rc = tg::launch_demo_sample_dm<4>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
-                                                          (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
-              if (rc != TG_OK) return rc; } break;
-    case 9: { const int rc = tg::launch_demo_sample_dm<9>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
-                                                          (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
-              if (rc != TG_OK) return rc; } break;
-    case 16: { const int rc = tg::launch_demo_sample_dm<16>(tape_dm, (const uint8_t *)targets, targets_i16 != 0, pack16, N, R, dim_t, replay_shift,
-                                                            (const long long *)idx, nb, states, scalars, (long long *)actions, rewards, st);
-               if (rc != TG_OK) return rc; } break;
-    default: return TG_E_ARG;
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    });
 }
 
 int tg_tape_to_demo_major(const uint8_t *tape, int64_t tape_step_stride, uint8_t *tape_dm, int64_t N, int R, int S, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!tape || !tape_dm) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)tape_dm | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_tape_to_demo_major(S, N, R, tape, tape_step_stride, tape_dm); rc != tg::LAUNCH) return rc;
     const int tp16 = ((3 * S + 15) & ~15) / 16;
     const long long total = N * R * tp16;
     const long long blocks = (total + 255) / 256;

@@ -831,11 +831,10 @@ __global__ void __launch_bounds__(128)
 // int8 slab in; int8 slab out (out16 == 0) or int16 slab out
 static int change_of_basis_impl(const int8_t *slab_in, const int8_t *mats, int per_game, void *slab_out, int out16, uint8_t *flags,
                                 int64_t N, int S, void *stream) {
-    if (!tg::basis_supported_S(S) || N < 0) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!slab_in || !mats || !slab_out || (const void *)slab_in == (const void *)slab_out) return TG_E_ARG;
-    if (((uintptr_t)slab_in | (uintptr_t)slab_out) & 15) return TG_E_ARG;
-    if (N > 0x7FFFFFFFLL) return TG_E_ARG;
+    if (const int rc = tg::check_basis(tg::basis_supported_S(S), N, slab_in, mats, 1, slab_out); rc != tg::LAUNCH) return rc;
+    // not in place: the exact kernel reads slab_in again for the games a fast kernel has already written to slab_out
+    if ((const void *)slab_in == (const void *)slab_out) return TG_E_ARG;
+    if (N > 0x7FFFFFFFLL) return TG_E_ARG; // the exact kernel without flags runs one CTA per game
     cudaStream_t st = (cudaStream_t)stream;
     const long long ms = per_game ? 3LL * S * S : 0;
     // a fast kernel first (tensor cores for 9x9x9 and 16x16x16, packed integer lanes for 4x4x4); it marks the games whose
@@ -891,7 +890,7 @@ static int change_of_basis_impl(const int8_t *slab_in, const int8_t *mats, int p
 #ifdef TG_TUNING
             if (out16) TG_BASIS_FAST(16, true) else TG_BASIS_FAST(16, false)
 #else
-            cudaMemsetAsync(flags, tg::BASIS_REDO, (size_t)N, st); // unaligned matrices: every game through the exact kernel
+            TG_CUDA(cudaMemsetAsync(flags, tg::BASIS_REDO, (size_t)N, st)); // unaligned matrices: every game through the exact kernel
 #endif
         }
         if (out16) { TG_BASIS_EXACT(16, true) } else { TG_BASIS_EXACT(16, false) }
@@ -918,43 +917,34 @@ int tg_change_of_basis_i16(const int8_t *slab_in, const int8_t *mats, int per_ga
 int tg_change_of_basis_factors(const uint8_t *tape_in, int64_t in_step_stride, int shift_in, const int8_t *mats, int per_game,
                                uint8_t *tape_out, int64_t out_step_stride, int shift_out, uint8_t *flags, int64_t N, int R,
                                int S, void *stream) {
-    if (!tg::basis_supported_S(S) || N < 0 || R < 1 || shift_in < 0 || shift_out < 1 || shift_out > 127) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!tape_in || !mats || !tape_out || !flags) return TG_E_ARG;
+    // coefficient = token - shift_in for any byte; token' = coefficient' + shift_out, a byte while |coefficient'| <= shift_out
+    if (shift_in < 0 || shift_out < 1 || shift_out > 127) return TG_E_ARG;
+    const int rc = tg::check_basis_factors(tg::basis_supported_S(S), N, R, tape_in, in_step_stride, mats, 1, tape_out);
+    if (rc != tg::LAUNCH) return rc;
+    if (!flags) return TG_E_ARG; // TG_FLAG_TOKEN_RANGE is OR-ed into it
     cudaStream_t st = (cudaStream_t)stream;
     const long long ms = per_game ? 3LL * S * S : 0;
-    const long long blocks = (N + (256 / S) - 1) / (256 / S);
-    const int grid = (int)(blocks < 148 * 16 ? blocks : 148 * 16);
-    if (((uintptr_t)tape_in | (uintptr_t)in_step_stride) & 15) return TG_E_ARG;
-    switch (S) {
-    case 4: tg::basis_factors_kernel<4><<<grid, 256, 0, st>>>(tape_in, in_step_stride, shift_in, mats, ms, tape_out, out_step_stride, shift_out, flags, N, R); break;
-    case 9: tg::basis_factors_kernel<9><<<grid, 256, 0, st>>>(tape_in, in_step_stride, shift_in, mats, ms, tape_out, out_step_stride, shift_out, flags, N, R); break;
-    case 16: {
-        const long long b16 = (N + 20) / 21;
-        if ((((uintptr_t)tape_out | (uintptr_t)out_step_stride) & 3) == 0)
+    return tg::with_basis_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        const long long blocks = (N + (256 / kS) - 1) / (256 / kS), b16 = (N + 20) / 21;
+        if (kS == 16 && (((uintptr_t)tape_out | (uintptr_t)out_step_stride) & 3) == 0)
             tg::basis_factors16_kernel<<<(int)(b16 < 148 * 16 ? b16 : 148 * 16), 252, 0, st>>>(tape_in, in_step_stride, shift_in, mats, ms, tape_out, out_step_stride, shift_out, flags, N, R);
         else
-            tg::basis_factors_kernel<16><<<grid, 256, 0, st>>>(tape_in, in_step_stride, shift_in, mats, ms, tape_out, out_step_stride, shift_out, flags, N, R);
-    } break;
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+            tg::basis_factors_kernel<kS><<<(int)(blocks < 148 * 16 ? blocks : 148 * 16), 256, 0, st>>>(tape_in, in_step_stride, shift_in, mats, ms, tape_out, out_step_stride, shift_out, flags, N, R);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_sample_unimodular(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, int8_t *mats, void *stream) {
-    if (!tg::basis_supported_S(S) || N < 0 || !(p_nonzero >= 0.0) || p_nonzero > 1.0) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!mats) return TG_E_ARG;
-    cudaStream_t st = (cudaStream_t)stream;
+    if (const int rc = tg::check_sample_bases(tg::basis_supported_S(S), N, p_nonzero, mats, 1); rc != tg::LAUNCH) return rc;
     const uint32_t thr = (uint32_t)(p_nonzero * 128.0);
-    const int grid = (int)((N * 3 + 63) / 64);
-    switch (S) {
-    case 4: tg::unimodular_kernel<4><<<grid, 64, 0, st>>>(seed, first, N, thr, mats); break;
-    case 9: tg::unimodular_kernel<9><<<grid, 64, 0, st>>>(seed, first, N, thr, mats); break;
-    case 16: tg::unimodular_kernel<16><<<grid, 64, 0, st>>>(seed, first, N, thr, mats); break;
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    return tg::with_basis_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        tg::unimodular_kernel<kS><<<(int)((N * 3 + 63) / 64), 64, 0, (cudaStream_t)stream>>>(seed, first, N, thr, mats);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 } // extern "C"

@@ -177,19 +177,18 @@ __global__ void __launch_bounds__(256) invert_bases_gf2_kernel(const uint32_t *m
 extern "C" {
 
 int tg_invert_bases(const int8_t *mats, int8_t *inv, uint8_t *flags, int64_t N, int S, void *stream) {
-    if (const int rc = tg::check_invert_bases(S, N, mats, inv, flags); rc != tg::LAUNCH) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (S) {
-    case 4: tg::invert_bases_kernel<4><<<tg::grid_for(N, 4 * 8), 128, 0, st>>>(mats, inv, flags, N); break;
-    case 9: tg::invert_bases_kernel<9><<<tg::grid_for(N, 4 * 3), 128, 0, st>>>(mats, inv, flags, N); break;
-    case 16: tg::invert_bases_kernel<16><<<tg::grid_for(N, 4 * 2), 128, 0, st>>>(mats, inv, flags, N); break;
-    }
-    TG_CUDA(cudaGetLastError());
-    return TG_OK;
+    if (const int rc = tg::check_invert_bases(tg::basis_supported_S(S), N, mats, inv, 1, flags); rc != tg::LAUNCH) return rc;
+    return tg::with_basis_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        // four warps of 32 / S triples per CTA
+        tg::invert_bases_kernel<kS><<<tg::grid_for(N, 4 * (32 / kS)), 128, 0, (cudaStream_t)stream>>>(mats, inv, flags, N);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    });
 }
 
 int tg_invert_bases_gf2(const uint32_t *mats, uint32_t *inv, uint8_t *flags, int64_t N, int S, void *stream) {
-    if (const int rc = tg::check_invert_bases_gf2(S, N, mats, inv, flags); rc != tg::LAUNCH) return rc;
+    if (const int rc = tg::check_invert_bases(tg::supported_S(S), N, mats, inv, 4, flags); rc != tg::LAUNCH) return rc;
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;
         tg::invert_bases_gf2_kernel<kS><<<tg::grid_for(N, 256), 256, 0, (cudaStream_t)stream>>>(mats, inv, flags, N);

@@ -71,8 +71,20 @@ int with_S(int S, F &&f) {
     return TG_E_ARG;
 }
 
-// ---------------------------------------------------------------- argument rules of the game path
-// One function per shape of entry point, shared by the int8, int16 and bit-slab twins.  In order: the scalars (TG_E_ARG),
+// with_S for the sizes of the change of basis over Z
+template <class F>
+int with_basis_S(int S, F &&f) {
+    switch (S) {
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 9: return f(std::integral_constant<int, 9>{});
+    case 16: return f(std::integral_constant<int, 16>{});
+    }
+    return TG_E_ARG;
+}
+
+// ---------------------------------------------------------------- argument rules of the device entry points
+// One function per shape of entry point, shared by its twins (int8, int16 and bit slabs; Z and GF(2)); each entry point
+// keeps only its own extra conditions.  In order: the scalars (TG_E_ARG),
 // an empty batch (TG_OK, before any pointer is looked at), null pointers (TG_E_ARG), alignment (TG_E_ARG).  LAUNCH means
 // the arguments hold and there is work; the entry point goes on to launch.  It never leaves the library.
 constexpr int LAUNCH = 1;
@@ -116,61 +128,90 @@ inline int check_pair(int S, long long B, const void *src, uintptr_t src_align, 
     return LAUNCH;
 }
 
-// tg_change_of_basis_gf2: bit slabs 16-byte aligned, the uint32 matrix rows 4-byte aligned
-inline int check_basis_gf2(int S, long long N, const void *in, const void *mats, const void *out) {
-    if (!supported_S(S) || N < 0) return TG_E_ARG;
+// tg_demo_gen_philox and tg_demo_gen_gf2: R, max_tries in [1, 65535], shift in [1, 4], n_values in [1, 8]; the tape, its
+// step stride and the slab or bit slab 16-byte aligned.  values and probs are host arrays; the generator tests the alphabet.
+inline int check_demo_gen(int S, long long N, int R, int shift, int n_values, int max_tries, const void *values, const void *probs,
+                          const void *tape, long long stride, const void *target) {
+    if (!supported_S(S) || N < 0 || R < 1 || R > 65535 || shift < 1 || shift > 4 || n_values < 1 || n_values > 8 || max_tries < 1 ||
+        max_tries > 65535)
+        return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!values || !probs || !tape || !target) return TG_E_ARG;
+    if (misaligned(tape, 16) || misaligned(target, 16) || (stride & 15)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_demo_accumulate*: S where size_ok, R >= 1, shift in [shift_lo, shift_hi]; the tape, its step stride and the slab
+// 16-byte aligned (flags may be NULL)
+inline int check_accumulate(bool size_ok, long long N, int R, int shift, int shift_lo, int shift_hi, const void *tape, long long stride,
+                            const void *slab) {
+    if (!size_ok || N < 0 || R < 1 || shift < shift_lo || shift > shift_hi) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!tape || !slab) return TG_E_ARG;
+    if (misaligned(tape, 16) || misaligned(slab, 16) || (stride & 15)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_demo_sample, tg_demo_sample_dm and tg_demo_sample_gf2 (target_bound 0 but for tg_demo_sample_dm): the targets
+// 16-byte aligned.  demo_major: the records also 16-byte aligned (they move by bulk copies), then replay_shift in [0, 8]
+// (the packed replay needs it).  The step-major batcher reads misaligned records by bytes and replays any shift on
+// int32 lanes.
+inline int check_demo_sample(int S, long long N, int R, int dim_t, int target_bound, long long nb, bool demo_major, int replay_shift,
+                             const void *tape, const void *targets, const void *idx, const void *states, const void *scalars,
+                             const void *actions, const void *rewards) {
+    if (!supported_S(S) || N < 0 || R < 1 || dim_t < 1 || target_bound < 0 || nb < 0) return TG_E_ARG;
+    if (nb == 0) return TG_OK;
+    if (!tape || !targets || !idx || !states || !scalars || !actions || !rewards) return TG_E_ARG;
+    if (misaligned(targets, 16) || (demo_major && misaligned(tape, 16))) return TG_E_ARG;
+    if (demo_major && (replay_shift < 0 || replay_shift > 8)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// tg_tape_to_demo_major: R >= 1; both tapes and the step stride 16-byte aligned
+inline int check_tape_to_demo_major(int S, long long N, int R, const void *tape, long long stride, const void *tape_dm) {
+    if (!supported_S(S) || N < 0 || R < 1) return TG_E_ARG;
+    if (N == 0) return TG_OK;
+    if (!tape || !tape_dm) return TG_E_ARG;
+    if (misaligned(tape, 16) || misaligned(tape_dm, 16) || (stride & 15)) return TG_E_ARG;
+    return LAUNCH;
+}
+
+// The change of basis over Z (size_ok = basis_supported_S(S), int8 matrices: mat_align 1) and over GF(2) (supported_S(S),
+// uint32 matrix rows: mat_align 4).
+// tg_change_of_basis*: slabs and bit slabs 16-byte aligned
+inline int check_basis(bool size_ok, long long N, const void *in, const void *mats, uintptr_t mat_align, const void *out) {
+    if (!size_ok || N < 0) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!in || !mats || !out) return TG_E_ARG;
-    if (misaligned(in, 16) || misaligned(out, 16) || misaligned(mats, 4)) return TG_E_ARG;
+    if (misaligned(in, 16) || misaligned(out, 16) || misaligned(mats, mat_align)) return TG_E_ARG;
     return LAUNCH;
 }
 
-// tg_change_of_basis_factors_gf2: both shifts in [1, 4], R >= 1; tapes and step strides 16-byte aligned, matrices 4
-inline int check_basis_factors_gf2(int S, long long N, int R, int shift_in, int shift_out, const void *tape_in, long long in_stride,
-                                   const void *mats, const void *tape_out, long long out_stride) {
-    if (!supported_S(S) || N < 0 || R < 1 || shift_in < 1 || shift_in > 4 || shift_out < 1 || shift_out > 4) return TG_E_ARG;
+// tg_change_of_basis_factors*: R >= 1 (each entry point tests its shifts first); tape_in and its step stride 16-byte aligned
+inline int check_basis_factors(bool size_ok, long long N, int R, const void *tape_in, long long in_stride, const void *mats,
+                               uintptr_t mat_align, const void *tape_out) {
+    if (!size_ok || N < 0 || R < 1) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!tape_in || !mats || !tape_out) return TG_E_ARG;
-    if (misaligned(tape_in, 16) || misaligned(tape_out, 16) || (in_stride & 15) || (out_stride & 15) || misaligned(mats, 4)) return TG_E_ARG;
+    if (misaligned(tape_in, 16) || (in_stride & 15) || misaligned(mats, mat_align)) return TG_E_ARG;
     return LAUNCH;
 }
 
-// tg_sample_invertible_gf2: p_nonzero in [0, 1] (NaN refused), matrices 4-byte aligned
-inline int check_sample_gf2(int S, long long N, double p_nonzero, const void *mats) {
-    if (!supported_S(S) || N < 0 || !(p_nonzero >= 0.0 && p_nonzero <= 1.0)) return TG_E_ARG;
+// tg_sample_unimodular, tg_sample_invertible_gf2: p_nonzero in [0, 1] (NaN refused)
+inline int check_sample_bases(bool size_ok, long long N, double p_nonzero, const void *mats, uintptr_t mat_align) {
+    if (!size_ok || N < 0 || !(p_nonzero >= 0.0 && p_nonzero <= 1.0)) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!mats) return TG_E_ARG;
-    if (misaligned(mats, 4)) return TG_E_ARG;
+    if (misaligned(mats, mat_align)) return TG_E_ARG;
     return LAUNCH;
 }
 
-// tg_invert_bases: int8 matrices at any byte address (slices of (n, 3, 9, 9) tensors start at odd ones), flags required
-inline int check_invert_bases(int S, long long N, const void *mats, const void *inv, const void *flags) {
-    if (!basis_supported_S(S) || N < 0) return TG_E_ARG;
+// tg_invert_bases*: flags required; int8 matrices at any byte address (slices of (n, 3, 9, 9) tensors start at odd ones)
+inline int check_invert_bases(bool size_ok, long long N, const void *mats, const void *inv, uintptr_t mat_align, const void *flags) {
+    if (!size_ok || N < 0) return TG_E_ARG;
     if (N == 0) return TG_OK;
     if (!mats || !inv || !flags) return TG_E_ARG;
-    return LAUNCH;
-}
-
-// tg_invert_bases_gf2: check_basis_gf2's rules for the matrices (4-byte aligned uint32 rows), flags required
-inline int check_invert_bases_gf2(int S, long long N, const void *mats, const void *inv, const void *flags) {
-    if (!supported_S(S) || N < 0) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!mats || !inv || !flags) return TG_E_ARG;
-    if (misaligned(mats, 4) || misaligned(inv, 4)) return TG_E_ARG;
-    return LAUNCH;
-}
-
-// tg_demo_sample_gf2: the rules of tg_demo_sample_dm in its order -- the scalars, an empty batch, null pointers, tape_dm
-// and the targets 16-byte aligned, then replay_shift in [0, 8]; states may start at any float
-inline int check_demo_sample_gf2(int S, long long N, int R, int dim_t, int replay_shift, long long nb, const void *tape_dm,
-                                 const void *targets, const void *idx, const void *states, const void *scalars, const void *actions,
-                                 const void *rewards) {
-    if (!supported_S(S) || N < 0 || R < 1 || dim_t < 1 || nb < 0) return TG_E_ARG;
-    if (nb == 0) return TG_OK;
-    if (!tape_dm || !targets || !idx || !states || !scalars || !actions || !rewards) return TG_E_ARG;
-    if (misaligned(tape_dm, 16) || misaligned(targets, 16)) return TG_E_ARG;
-    if (replay_shift < 0 || replay_shift > 8) return TG_E_ARG;
+    if (misaligned(mats, mat_align) || misaligned(inv, mat_align)) return TG_E_ARG;
     return LAUNCH;
 }
 

@@ -956,12 +956,8 @@ extern "C" {
 int tg_demo_gen_philox(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int shift, const int8_t *values,
                        const double *probs, int n_values, int max_tries, uint8_t *tape, int64_t tape_step_stride,
                        int8_t *slab, uint8_t *flags, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || shift < 1 || shift > 4 || n_values < 1 || n_values > 8 || max_tries < 1 ||
-        max_tries > 65535)
-        return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!values || !probs || !tape || !slab) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)slab | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_demo_gen(S, N, R, shift, n_values, max_tries, values, probs, tape, tape_step_stride, slab); rc != tg::LAUNCH)
+        return rc;
     if (!tg::alphabet_ok(values, probs, n_values, shift)) return TG_E_ARG;
     tg::Categorical cat = tg::categorical(values, probs, n_values, shift, seed);
     // measured (profiles/README.md): skipping the zero-coefficient terms in the accumulation pays at 9x9x9 (+10 %) when most
@@ -1004,22 +1000,13 @@ int tg_demo_gen_philox(uint64_t seed, uint64_t first_demo, int64_t N, int R, int
 }
 
 int tg_demo_alias_tables(const int8_t *values, const double *probs, int n_values, int S, uint16_t *tables_host) {
-    if (!values || !probs || !tables_host || !tg::alias_applies(values, probs, n_values, S)) return TG_E_ARG;
-    tg::AliasParams ap;
-    tg::build_alias(values, probs, n_values, S, 0, 0, ap);
-    // oracle order: [0] plain size 3, [1] plain size 1, [2 + g] tilted table of group g
-    memcpy(tables_host, ap.tab[6], sizeof(ap.tab[6]));
-    memcpy(tables_host + tg::ALIAS_BUCKETS, ap.tab[7], sizeof(ap.tab[7]));
-    memcpy(tables_host + 2 * tg::ALIAS_BUCKETS, ap.tab[0], 6 * sizeof(ap.tab[0]));
-    return TG_OK;
+    return tg::alias_tables_host<false>(values, probs, n_values, S, tables_host);
 }
 
 int tg_demo_accumulate(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift, int8_t *slab,
                        uint8_t *flags, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!tape || !slab) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)slab | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_accumulate(tg::supported_S(S), N, R, shift, 1, 4, tape, tape_step_stride, slab); rc != tg::LAUNCH)
+        return rc;
     // 16x16x16: tensor cores (tg_demo_mma.cu); TG_DEMO_MMA=0 keeps the packed-IMAD kernel (A/B timing only)
 #ifdef TG_TUNING
     static const int use_mma = tg::tuning_env("TG_DEMO_MMA", 1);

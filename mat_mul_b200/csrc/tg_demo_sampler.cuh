@@ -379,6 +379,19 @@ inline void alias_to_dev(const AliasParams &A, const int8_t *values, int n, int 
     memcpy(D.rk, A.rk, sizeof(D.rk));
 }
 
+// tg_demo_alias_tables(_gf2): the host tables uint16 [8][128] in the oracle's order -- [0] plain size 3, [1] plain size 1,
+// [2 + g] tilted table of group g
+template <bool GF2>
+inline int alias_tables_host(const int8_t *values, const double *probs, int n, int S, uint16_t *tables_host) {
+    if (!values || !probs || !tables_host || !alias_applies<GF2>(values, probs, n, S)) return TG_E_ARG;
+    AliasParams ap;
+    build_alias<GF2>(values, probs, n, S, 0, 0, ap);
+    memcpy(tables_host, ap.tab[6], sizeof(ap.tab[6]));
+    memcpy(tables_host + ALIAS_BUCKETS, ap.tab[7], sizeof(ap.tab[7]));
+    memcpy(tables_host + 2 * ALIAS_BUCKETS, ap.tab[0], 6 * sizeof(ap.tab[0]));
+    return TG_OK;
+}
+
 // ---- per-device cache of device-format tables (tg_demo.cu).  A table set is uploaded by a one-CTA kernel on the caller's
 // stream the first time it is asked for; a later launch -- on any stream -- waits for that upload's event.  Eight sets
 // per device; a ninth distinct set evicts the least recently used one after a cudaDeviceSynchronize (kernels of other

@@ -348,9 +348,7 @@ extern "C" int tg_debug_tc(unsigned long long *out, int reset) {
 
 extern "C" int tg_demo_accumulate_tc(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift,
                                      int8_t *slab, uint8_t *flags, void *stream) {
-    if (S != 16 || N < 0 || R < 1 || R > 64 || shift < 1 || shift > 4) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!tape || !slab) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)slab | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (R > 64) return TG_E_ARG; // the MMA's K dimension is the demo's R terms, padded to 32 or 64
+    if (const int rc = tg::check_accumulate(S == 16, N, R, shift, 1, 4, tape, tape_step_stride, slab); rc != tg::LAUNCH) return rc;
     return tg::launch_demo_tc(tape, tape_step_stride, N, R, shift, slab, flags, (cudaStream_t)stream);
 }

@@ -232,7 +232,7 @@ extern "C" {
 
 int tg_change_of_basis_gf2(const uint32_t *bits_in, const uint32_t *mats, int per_game, uint32_t *bits_out, int64_t N, int S,
                            void *stream) {
-    if (const int rc = tg::check_basis_gf2(S, N, bits_in, mats, bits_out); rc != tg::LAUNCH) return rc;
+    if (const int rc = tg::check_basis(tg::supported_S(S), N, bits_in, mats, 4, bits_out); rc != tg::LAUNCH) return rc;
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;
         using P = tg::BasisB<kS>;
@@ -245,8 +245,10 @@ int tg_change_of_basis_gf2(const uint32_t *bits_in, const uint32_t *mats, int pe
 
 int tg_change_of_basis_factors_gf2(const uint8_t *tape_in, int64_t in_step_stride, int shift_in, const uint32_t *mats, int per_game,
                                    uint8_t *tape_out, int64_t out_step_stride, int shift_out, int64_t N, int R, int S, void *stream) {
-    const int rc = tg::check_basis_factors_gf2(S, N, R, shift_in, shift_out, tape_in, in_step_stride, mats, tape_out, out_step_stride);
+    if (shift_in < 1 || shift_in > 4 || shift_out < 1 || shift_out > 4) return TG_E_ARG; // the game path's shifts
+    const int rc = tg::check_basis_factors(tg::supported_S(S), N, R, tape_in, in_step_stride, mats, 4, tape_out);
     if (rc != tg::LAUNCH) return rc;
+    if (tg::misaligned(tape_out, 16) || (out_step_stride & 15)) return TG_E_ARG; // records leave as 16-byte words
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;
         tg::basis_factors_gf2_kernel<kS><<<tg::grid_for(N, 256), 256, 0, (cudaStream_t)stream>>>(
@@ -257,7 +259,7 @@ int tg_change_of_basis_factors_gf2(const uint8_t *tape_in, int64_t in_step_strid
 }
 
 int tg_sample_invertible_gf2(uint64_t seed, uint64_t first, int64_t N, int S, double p_nonzero, uint32_t *mats, void *stream) {
-    if (const int rc = tg::check_sample_gf2(S, N, p_nonzero, mats); rc != tg::LAUNCH) return rc;
+    if (const int rc = tg::check_sample_bases(tg::supported_S(S), N, p_nonzero, mats, 4); rc != tg::LAUNCH) return rc;
     const uint32_t thr = (uint32_t)(p_nonzero * 128.0);
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;

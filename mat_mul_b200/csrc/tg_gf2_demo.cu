@@ -175,12 +175,8 @@ extern "C" {
 int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int shift, const int8_t *values,
                     const double *probs, int n_values, int max_tries, uint8_t *tape, int64_t tape_step_stride,
                     uint32_t *bits, uint8_t *flags, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || R > 65535 || shift < 1 || shift > 4 || n_values < 1 || n_values > 8 ||
-        max_tries < 1 || max_tries > 65535)
-        return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!values || !probs || !tape || !bits) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)bits | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_demo_gen(S, N, R, shift, n_values, max_tries, values, probs, tape, tape_step_stride, bits); rc != tg::LAUNCH)
+        return rc;
     if (!tg::alphabet_ok(values, probs, n_values, shift)) return TG_E_ARG;
     int odd = -1; // the last odd value: the forced triple of contract v1
     for (int i = 0; i < n_values; i++)
@@ -215,14 +211,7 @@ int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S,
 }
 
 int tg_demo_alias_tables_gf2(const int8_t *values, const double *probs, int n_values, int S, uint16_t *tables_host) {
-    if (!values || !probs || !tables_host || !tg::alias_applies<true>(values, probs, n_values, S)) return TG_E_ARG;
-    tg::AliasParams ap;
-    tg::build_alias<true>(values, probs, n_values, S, 0, 0, ap);
-    // oracle order: [0] plain size 3, [1] plain size 1, [2 + g] tilted table of group g
-    memcpy(tables_host, ap.tab[6], sizeof(ap.tab[6]));
-    memcpy(tables_host + tg::ALIAS_BUCKETS, ap.tab[7], sizeof(ap.tab[7]));
-    memcpy(tables_host + 2 * tg::ALIAS_BUCKETS, ap.tab[0], 6 * sizeof(ap.tab[0]));
-    return TG_OK;
+    return tg::alias_tables_host<true>(values, probs, n_values, S, tables_host);
 }
 
 } // extern "C"

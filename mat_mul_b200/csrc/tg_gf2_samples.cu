@@ -188,7 +188,8 @@ extern "C" {
 
 int tg_demo_sample_gf2(const uint8_t *tape_dm, const uint32_t *targets_bits, int64_t N, int R, int S, int dim_t, int replay_shift,
                        const int64_t *idx, int64_t nb, float *states, float *scalars, int64_t *actions, float *rewards, void *stream) {
-    const int rc = tg::check_demo_sample_gf2(S, N, R, dim_t, replay_shift, nb, tape_dm, targets_bits, idx, states, scalars, actions, rewards);
+    const int rc = tg::check_demo_sample(S, N, R, dim_t, 0, nb, true, replay_shift, tape_dm, targets_bits, idx, states, scalars, actions,
+                                         rewards);
     if (rc != tg::LAUNCH) return rc;
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;

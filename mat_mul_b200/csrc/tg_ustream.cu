@@ -191,12 +191,14 @@ int64_t tg_demo_from_ustream_workspace(int64_t n_u, int S) {
 int tg_demo_from_ustream(const double *u, int64_t n_u, const int8_t *values, const float *probs, int n_values, int R, int S,
                          int shift, int64_t N, uint8_t *tape, int64_t tape_step_stride, int8_t *slab, uint8_t *flags,
                          int64_t *result, void *workspace, int64_t workspace_bytes, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || shift < 1 || shift > 4 || n_values < 1 || n_values > 8 || n_u < 0)
+    if (!tg::supported_S(S) || N < 0 || R < 1 || shift < 1 || shift > 4 || n_values < 1 || n_values > 8 || n_u < 0 ||
+        n_u / (3 * S) >= (1LL << 31))
         return TG_E_ARG;
+    if (N == 0) return TG_OK;
     if (!u || !values || !probs || !tape || !slab || !result || !workspace) return TG_E_ARG;
     if (((uintptr_t)tape | (uintptr_t)slab | (uintptr_t)tape_step_stride | (uintptr_t)workspace) & 15) return TG_E_ARG;
+    if (workspace_bytes < tg_demo_from_ustream_workspace(n_u, S)) return TG_E_ARG;
     const int64_t n_tries = n_u / (3 * S);
-    if (n_tries >= (1LL << 31) || workspace_bytes < tg_demo_from_ustream_workspace(n_u, S)) return TG_E_ARG;
     cudaStream_t st = (cudaStream_t)stream;
     // the CDF exactly as Categorical + the multinomial CPU kernel build it (float32)
     tg::CdfF32 cat;

@@ -142,10 +142,8 @@ extern "C" {
 
 int tg_demo_accumulate_i16(const uint8_t *tape, int64_t tape_step_stride, int64_t N, int R, int S, int shift, int16_t *slab16,
                            uint8_t *flags, void *stream) {
-    if (!tg::supported_S(S) || N < 0 || R < 1 || shift < 0 || shift > 127) return TG_E_ARG;
-    if (N == 0) return TG_OK;
-    if (!tape || !slab16) return TG_E_ARG;
-    if (((uintptr_t)tape | (uintptr_t)slab16 | (uintptr_t)tape_step_stride) & 15) return TG_E_ARG;
+    if (const int rc = tg::check_accumulate(tg::supported_S(S), N, R, shift, 0, 127, tape, tape_step_stride, slab16); rc != tg::LAUNCH)
+        return rc;
     cudaStream_t st = (cudaStream_t)stream;
     const long long cmax = shift > 255 - shift ? shift : 255 - shift;
     if ((long long)R * cmax * cmax * cmax > 0x7FFFFFFFLL) {
