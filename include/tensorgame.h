@@ -80,7 +80,7 @@
 extern "C" {
 #endif
 
-#define TG_VERSION 207
+#define TG_VERSION 208
 
 #define TG_OK 0
 #define TG_E_ARG (-1)     /* bad argument (unsupported S, null pointer, misaligned buffer) */
@@ -405,6 +405,35 @@ int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S,
 /* HOST function: the tables of v2 mod 2 in tg_demo_alias_tables' layout (uint16 [8][128]); TG_E_ARG where v2 mod 2 does
  * not apply (also at S = 25). */
 int tg_demo_alias_tables_gf2(const int8_t *values, const double *probs, int n_values, int S, uint16_t *tables_host);
+
+/* ---- demonstrations in a box: rectangular products <n, m, p> (S in {4, 9, 16, 25}) ---------------------------------- */
+/* <n, m, p> (A n x m, B m x p, C n x p, T[i m + j][j p + k][i p + k] = 1) is a tensor of shape (n m, m p, n p), played
+ * zero-padded in the smallest S that holds its largest mode; every game kernel is exact on the padded tensor.  Its
+ * demonstrations must keep their factors in the box (nu, nv, nw) = (n m, m p, n p): demos drawn over the whole cube are
+ * not demonstrations of <n, m, p>.
+ * Contract box v1: contract v1 at size S with the box applied.  Demo d = first_demo + n, term r, try t draws all 3S
+ * 15-bit values exactly as v1 does at S (same Philox counters, thresholds and tokens); draws outside the box are made and
+ * discarded: the entries u_e (e >= nu), v_e (e >= nv) and w_e (e >= nw) become the coefficient 0 (token = shift).  A try
+ * is accepted iff u[0, nu), v[0, nv) and w[0, nw) each have a non-zero entry (mod 2: an odd entry).  After max_tries
+ * tries the term is u = v = w = x e_0 (e_0 lies inside every box), x the last value (mod 2: the last odd value), and the
+ * demo gets TG_FLAG_EXHAUSTED.  Consequences:
+ *  - with the full box (S, S, S) the output is contract v1's byte for byte: tg_demo_gen_philox's wherever it uses v1
+ *    (every alphabet at 25; at 4, 9 and 16 alphabets of six or more values or with P(0) > 0.999), and mod 2 the v1 of
+ *    tg_demo_gen_gf2;
+ *  - every factor is zero outside the box, so every target entry outside [0, nu) x [0, nv) x [0, nw) is zero.
+ * Contract v2 is not used: its tilted tables depend on the factor length, and a box has three.
+ * Outputs are those of the cubic twins: the step-major tape (tokens = value + shift, padding zero, tape_step_stride as
+ * there); tg_demo_gen_box the int8 slab, which is exactly what tg_demo_accumulate writes for the same tape (entries
+ * modulo 256, TG_FLAG_RANGE outside [-64, 63]; targets beyond int8 come from tg_demo_accumulate_i16 of the tape);
+ * tg_demo_gen_box_gf2 the bit slab, the xor of the terms; flags (may be NULL): TG_FLAG_EXHAUSTED | TG_FLAG_RANGE.
+ * Arguments: tg_demo_gen_philox's rules, and nu, nv, nw in [1, S] checked with the scalars (before the empty batch); then
+ * the cubic twin's alphabet rules (mod 2: an alphabet with no odd value returns TG_E_ARG). */
+int tg_demo_gen_box(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int nu, int nv, int nw, int shift,
+                    const int8_t *values, const double *probs, int n_values, int max_tries, uint8_t *tape,
+                    int64_t tape_step_stride, int8_t *slab, uint8_t *flags, void *stream);
+int tg_demo_gen_box_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int nu, int nv, int nw, int shift,
+                        const int8_t *values, const double *probs, int n_values, int max_tries, uint8_t *tape,
+                        int64_t tape_step_stride, uint32_t *bits, uint8_t *flags, void *stream);
 
 /* ---- K5: change-of-basis augmentation (S in {4, 9, 16}; TG_E_ARG at 25) ------ */
 /* ABSENT from the reference; specified from the AlphaTensor paper (Methods,

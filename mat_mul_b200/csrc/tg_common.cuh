@@ -141,6 +141,13 @@ inline int check_demo_gen(int S, long long N, int R, int shift, int n_values, in
     return LAUNCH;
 }
 
+// tg_demo_gen_box and tg_demo_gen_box_gf2: check_demo_gen's rules with the box (nu, nv, nw) in [1, S]^3, a scalar rule
+inline int check_demo_gen_box(int S, long long N, int R, int nu, int nv, int nw, int shift, int n_values, int max_tries,
+                              const void *values, const void *probs, const void *tape, long long stride, const void *target) {
+    if (nu < 1 || nu > S || nv < 1 || nv > S || nw < 1 || nw > S) return TG_E_ARG;
+    return check_demo_gen(S, N, R, shift, n_values, max_tries, values, probs, tape, stride, target);
+}
+
 // tg_demo_accumulate*: S where size_ok, R >= 1, shift in [shift_lo, shift_hi]; the tape, its step stride and the slab
 // 16-byte aligned (flags may be NULL)
 inline int check_accumulate(bool size_ok, long long N, int R, int shift, int shift_lo, int shift_hi, const void *tape, long long stride,

@@ -137,7 +137,9 @@ __device__ __forceinline__ int coef_byte(uint32_t w) {
 // then sums the targets of its demos on the tensor cores (tg_demo_mma.cuh) -- CTAs of one SM are in different phases, so
 // the sampler's integer work and the MMAs overlap.
 // ALIAS: phase A draws under contract v2 (group alias tables, no rejection loop); the categorical thresholds are unused.
-template <int S, int NT, int NPASS, bool SAMPLE, int NTHR, bool GUARD, int MMA = 0, bool ALIAS = false>
+// OR_FLAGS (replay only): OR the flags into the caller's (the EXHAUSTED flags of a sampler that ran before) instead of
+// overwriting them.
+template <int S, int NT, int NPASS, bool SAMPLE, int NTHR, bool GUARD, int MMA = 0, bool ALIAS = false, bool OR_FLAGS = false>
 __global__ void __launch_bounds__(NT, S == 16 ? (NT <= 128 ? 4 : 2) : (S == 9 ? (NT == 128 ? 8 : NT == 64 ? 16 : 3) : 4))
     demo_kernel(unsigned long long first_demo, long long N, int R, uint32_t magic_r, int shift,
                 const __grid_constant__ Categorical cat, int max_tries, uint8_t *__restrict__ tape,
@@ -145,6 +147,7 @@ __global__ void __launch_bounds__(NT, S == 16 ? (NT <= 128 ? 4 : 2) : (S == 9 ? 
                 const __grid_constant__ AliasDev ap) {
     using C = DemoCfg<S, NT, NPASS>;
     using G = Geo<S>;
+    static_assert(!OR_FLAGS || (!SAMPLE && MMA == 0), "OR_FLAGS: the replay mode");
     extern __shared__ __align__(128) uint8_t smem[];
     // integer variants: per pass of phase B one region, first the accumulate records [GPASS][R][REC] (phases A, B), then the
     // pass's slab tile [GPASS][PITCH] in the same bytes (C::rec_off / C::slab_off); tensor-core variants: records [TG][R][TP]
@@ -555,13 +558,13 @@ __global__ void __launch_bounds__(NT, S == 16 ? (NT <= 128 ? 4 : 2) : (S == 9 ? 
         if (tid < ng) bulk_commit();
     }
     if (flags)
-        for (int gg = tid; gg < ng; gg += NT) flags[g0 + gg] = (uint8_t)s_flag[gg];
+        for (int gg = tid; gg < ng; gg += NT) flags[g0 + gg] = (uint8_t)(OR_FLAGS ? flags[g0 + gg] | s_flag[gg] : s_flag[gg]);
     if constexpr (S != 4) {
         if (tid < ng) bulk_wait<0>();
     }
 }
 
-template <int S, int NT, int NPASS, bool SAMPLE, int NTHR>
+template <int S, int NT, int NPASS, bool SAMPLE, int NTHR, bool OR_FLAGS = false>
 static int launch_demo(unsigned long long first, long long N, int R, int shift, const Categorical &cat, int max_tries,
                        uint8_t *tape, long long stride, int8_t *slab, uint8_t *flags, cudaStream_t st) {
     using C = DemoCfg<S, NT, NPASS>;
@@ -573,11 +576,11 @@ static int launch_demo(unsigned long long first, long long N, int R, int shift, 
     if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
     static const AliasDev no_alias = {};
     if (guard) {
-        auto kern = demo_kernel<S, NT, NPASS, SAMPLE, NTHR, true>;
+        auto kern = demo_kernel<S, NT, NPASS, SAMPLE, NTHR, true, 0, false, OR_FLAGS>;
         TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         kern<<<(int)grid, NT, smem, st>>>(first, N, R, magic, shift, cat, max_tries, tape, stride, slab, flags, no_alias);
     } else {
-        auto kern = demo_kernel<S, NT, NPASS, SAMPLE, NTHR, false>;
+        auto kern = demo_kernel<S, NT, NPASS, SAMPLE, NTHR, false, 0, false, OR_FLAGS>;
         TG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         kern<<<(int)grid, NT, smem, st>>>(first, N, R, magic, shift, cat, max_tries, tape, stride, slab, flags, no_alias);
     }
@@ -636,8 +639,9 @@ static int launch_demo_alias(unsigned long long first, long long N, int R, int s
 // 32 targets of a warp are one contiguous block of the slab: they leave through a warp-private stage so that a store
 // instruction writes 512 contiguous bytes.  Taken when R * shift^3 <= 191 (a final entry outside int8 then always decodes
 // outside [-64, 63]); larger R keeps the guarded tile kernel.
-// SAMPLE = false (tg_demo_accumulate): the records come from the tape instead (any token: the guarded coefficient form).
-template <bool SAMPLE>
+// SAMPLE = false (tg_demo_accumulate): the records come from the tape instead (any token: the guarded coefficient form);
+// OR_FLAGS: OR the RANGE flags into the caller's, as demo_kernel does.
+template <bool SAMPLE, bool OR_FLAGS = false>
 __global__ void __launch_bounds__(128)
     demo4_thread_kernel(unsigned long long first_demo, long long N, int R, int shift, uint8_t *__restrict__ tape, long long tape_step_stride,
                         int8_t *__restrict__ slab, uint8_t *__restrict__ flags, const __grid_constant__ AliasDev ap) {
@@ -694,7 +698,7 @@ __global__ void __launch_bounds__(128)
         }
         mine[i] = make_uint4(acc[4 * i], acc[4 * i + 1], acc[4 * i + 2], acc[4 * i + 3]);
     }
-    if (flags && real) flags[n] = (~ok & H4) ? (uint8_t)TG_FLAG_RANGE : (uint8_t)0;
+    if (flags && real) flags[n] = (uint8_t)((OR_FLAGS ? flags[n] : 0) | ((~ok & H4) ? TG_FLAG_RANGE : 0));
     __syncwarp();
     const int total = (int)min(32LL, N - nw0) * 4;
     uint4 *out = reinterpret_cast<uint4 *>(slab + nw0 * 64);
@@ -903,7 +907,7 @@ static int launch_demo25(unsigned long long first, long long N, int R, int shift
     return launch_demo_acc_cols<25>(tape, stride, N, R, shift, slab, flags, 1, st);
 }
 
-template <bool SAMPLE, int NTHR>
+template <bool SAMPLE, int NTHR, bool OR_FLAGS = false>
 static int dispatch_demo(unsigned long long first, long long N, int R, int S, int shift, const Categorical &cat,
                          int max_tries, uint8_t *tape, long long stride, int8_t *slab, uint8_t *flags, cudaStream_t st) {
     switch (S) {
@@ -911,42 +915,118 @@ static int dispatch_demo(unsigned long long first, long long N, int R, int S, in
 #ifdef TG_TUNING
         static const int variant = tuning_env("TG_DEMO_VARIANT", 0);
         if (variant == 1 && DemoCfg<4, 128, 8>::smem_bytes(R) <= 160 * 1024)
-            return launch_demo<4, 128, 8, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+            return launch_demo<4, 128, 8, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
         if (variant == 2 && DemoCfg<4, 128, 4>::smem_bytes(R) <= 160 * 1024)
-            return launch_demo<4, 128, 4, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+            return launch_demo<4, 128, 4, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
         if (variant == 3 && DemoCfg<4, 512, 2>::smem_bytes(R) <= 160 * 1024)
-            return launch_demo<4, 512, 2, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+            return launch_demo<4, 512, 2, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
 #endif
         if (DemoCfg<4, 256, 4>::smem_bytes(R) <= 160 * 1024)
-            return launch_demo<4, 256, 4, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        return launch_demo<4, 256, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+            return launch_demo<4, 256, 4, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        return launch_demo<4, 256, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
     }
     case 9: {
 #ifdef TG_TUNING
         switch (tuning_env("TG_DEMO_VARIANT", 0)) {
-        case 1: return launch_demo<9, 256, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        case 3: return launch_demo<9, 128, 3, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        case 4: return launch_demo<9, 192, 2, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        case 5: return launch_demo<9, 64, 4, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        case 1: return launch_demo<9, 256, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        case 3: return launch_demo<9, 128, 3, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        case 4: return launch_demo<9, 192, 2, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        case 5: return launch_demo<9, 64, 4, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
         default: break;
         }
 #endif
         // measured best (profiles/README.md): 128-thread CTAs; 28-demo tiles when sampling, 14-demo tiles (slab tile
         // overlaid on the records) when only accumulating
-        if (SAMPLE) return launch_demo<9, 128, 2, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        return launch_demo<9, 128, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        if (SAMPLE) return launch_demo<9, 128, 2, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        return launch_demo<9, 128, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
     }
     case 16: {
 #ifdef TG_TUNING
         static const int variant = tuning_env("TG_DEMO_VARIANT", 0);
-        if (variant == 1) return launch_demo<16, 256, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        if (variant == 2) return launch_demo<16, 64, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
-        if (variant == 3) return launch_demo<16, 128, 2, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        if (variant == 1) return launch_demo<16, 256, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        if (variant == 2) return launch_demo<16, 64, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
+        if (variant == 3) return launch_demo<16, 128, 2, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st);
 #endif
-        return launch_demo<16, 128, 1, SAMPLE, NTHR>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st); // measured best
+        return launch_demo<16, 128, 1, SAMPLE, NTHR, OR_FLAGS>(first, N, R, shift, cat, max_tries, tape, stride, slab, flags, st); // measured best
     }
     }
     return TG_E_ARG;
+}
+
+// tg_demo_accumulate's choice of sum for (S, R, shift).  OR_FLAGS: OR the flags into the caller's (tg_demo_gen_box, after
+// its sampler wrote the EXHAUSTED flags) instead of overwriting them.
+template <bool OR_FLAGS>
+static int accumulate(const uint8_t *tape, long long stride, long long N, int R, int S, int shift, int8_t *slab, uint8_t *flags,
+                      cudaStream_t st) {
+    // 16x16x16: tensor cores (tg_demo_mma.cu); TG_DEMO_MMA=0 keeps the packed-IMAD kernel (A/B timing only)
+#ifdef TG_TUNING
+    static const int use_mma = tuning_env("TG_DEMO_MMA", 1);
+#else
+    constexpr int use_mma = 1;
+#endif
+    if (S == 25) return launch_demo_acc_cols<25>(tape, stride, N, R, shift, slab, flags, OR_FLAGS, st);
+    if (S == 16 && use_mma && demo_acc16_mma_applies(R)) return launch_demo_acc16_mma(tape, stride, N, R, shift, slab, flags, OR_FLAGS, st);
+    if (S == 4 && (long long)R * shift * shift * shift <= 191 && R <= 65535 && N <= 0x7FFFFFFFLL * 128) { // one thread per demo
+        static const AliasDev no_tables = {};
+        demo4_thread_kernel<false, OR_FLAGS><<<(int)((N + 127) / 128), 128, 0, st>>>(0, N, R, shift, const_cast<uint8_t *>(tape), stride,
+                                                                                   slab, flags, no_tables);
+        TG_CUDA(cudaGetLastError());
+        return TG_OK;
+    }
+    Categorical cat = {};
+    // 9x9x9: walk only the terms with a non-zero v_j (the masks are built from the tape itself, so this is exact for any tape;
+    // with the reference's distributions 70 % of the coefficients are zero: 0.62 -> 0.55 ms per 2^20 demos; a tape without zeros
+    // pays ~15 % in the term loop)
+    cat.sparse_terms = S == 9 ? 1u : 0u;
+    return dispatch_demo<false, 2, OR_FLAGS>(0, N, R, S, shift, cat, 1, const_cast<uint8_t *>(tape), stride, slab, flags, st);
+}
+
+// ---- contract box v1 (tg_demo_gen_box): the sampler alone, one thread per demo -- consecutive threads write consecutive
+// records of a step, so a warp stores 32 TP contiguous bytes per term -- then tg_demo_accumulate's sum with the flags OR-ed
+template <int S, int NTHR>
+__global__ void __launch_bounds__(128)
+    demo_box_sample_kernel(unsigned long long first_demo, long long N, int R, int shift, const __grid_constant__ Categorical cat,
+                           int max_tries, const __grid_constant__ BoxMasks box, uint8_t *__restrict__ tape, long long tape_step_stride,
+                           uint8_t *__restrict__ flags) {
+    constexpr int TP = Geo<S>::TP, NW = (3 * S + 3) / 4;
+    const long long n = (long long)blockIdx.x * 128 + threadIdx.x;
+    if (n >= N) return;
+    const unsigned long long d = first_demo + (unsigned long long)n;
+    const uint32_t d_lo = (uint32_t)d, d_hi = (uint32_t)(d >> 32);
+    uint32_t fl = 0;
+#pragma unroll 1
+    for (int r = 0; r < R; r++) {
+        uint32_t words[TP / 4];
+#pragma unroll
+        for (int w = NW; w < TP / 4; w++) words[w] = 0;
+#pragma unroll 1
+        for (int t = 0;; t++) {
+            if (draw_triple_box<S, NTHR>(words, d_lo, d_hi, r, t, cat, box)) break;
+            if (t + 1 >= max_tries) { // forced: u = v = w = x e_0 (e_0 lies inside every box), x the last value
+#pragma unroll
+                for (int w = 0; w < NW; w++) words[w] = 0;
+#pragma unroll
+                for (int q = 0; q < 3 * S; q++)
+                    words[q >> 2] |= (((q % S) == 0 ? cat.top_tok : (uint32_t)shift) & 0xFFu) << (8 * (q & 3));
+                fl = TG_FLAG_EXHAUSTED;
+                break;
+            }
+        }
+        uint4 *dst = reinterpret_cast<uint4 *>(tape + (size_t)r * tape_step_stride + n * TP);
+#pragma unroll
+        for (int w = 0; w < TP / 16; w++) dst[w] = make_uint4(words[4 * w], words[4 * w + 1], words[4 * w + 2], words[4 * w + 3]);
+    }
+    if (flags) flags[n] = (uint8_t)fl;
+}
+
+template <int S, int NTHR>
+static int launch_demo_box_sample(unsigned long long first, long long N, int R, int shift, const Categorical &cat, int max_tries,
+                                  const BoxMasks &box, uint8_t *tape, long long stride, uint8_t *flags, cudaStream_t st) {
+    const long long grid = (N + 127) / 128;
+    if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
+    demo_box_sample_kernel<S, NTHR><<<(unsigned)grid, 128, 0, st>>>(first, N, R, shift, cat, max_tries, box, tape, stride, flags);
+    TG_CUDA(cudaGetLastError());
+    return TG_OK;
 }
 
 } // namespace tg
@@ -1007,29 +1087,27 @@ int tg_demo_accumulate(const uint8_t *tape, int64_t tape_step_stride, int64_t N,
                        uint8_t *flags, void *stream) {
     if (const int rc = tg::check_accumulate(tg::supported_S(S), N, R, shift, 1, 4, tape, tape_step_stride, slab); rc != tg::LAUNCH)
         return rc;
-    // 16x16x16: tensor cores (tg_demo_mma.cu); TG_DEMO_MMA=0 keeps the packed-IMAD kernel (A/B timing only)
-#ifdef TG_TUNING
-    static const int use_mma = tg::tuning_env("TG_DEMO_MMA", 1);
-#else
-    constexpr int use_mma = 1;
-#endif
-    if (S == 25) return tg::launch_demo_acc_cols<25>(tape, tape_step_stride, N, R, shift, slab, flags, 0, (cudaStream_t)stream);
-    if (S == 16 && use_mma && tg::demo_acc16_mma_applies(R))
-        return tg::launch_demo_acc16_mma(tape, tape_step_stride, N, R, shift, slab, flags, 0, (cudaStream_t)stream);
-    if (S == 4 && (long long)R * shift * shift * shift <= 191 && R <= 65535 && N <= 0x7FFFFFFFLL * 128) { // one thread per demo
-        static const tg::AliasDev no_tables = {};
-        tg::demo4_thread_kernel<false><<<(int)((N + 127) / 128), 128, 0, (cudaStream_t)stream>>>(0, N, R, shift, const_cast<uint8_t *>(tape),
-                                                                                              tape_step_stride, slab, flags, no_tables);
-        TG_CUDA(cudaGetLastError());
-        return TG_OK;
-    }
-    tg::Categorical cat = {};
-    // 9x9x9: walk only the terms with a non-zero v_j (the masks are built from the tape itself, so this is exact for any tape;
-    // with the reference's distributions 70 % of the coefficients are zero: 0.62 -> 0.55 ms per 2^20 demos; a tape without zeros
-    // pays ~15 % in the term loop)
-    cat.sparse_terms = S == 9 ? 1u : 0u;
-    return tg::dispatch_demo<false, 2>(0, N, R, S, shift, cat, 1, const_cast<uint8_t *>(tape), tape_step_stride, slab, flags,
-                                       (cudaStream_t)stream);
+    return tg::accumulate<false>(tape, tape_step_stride, N, R, S, shift, slab, flags, (cudaStream_t)stream);
+}
+
+int tg_demo_gen_box(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int nu, int nv, int nw, int shift,
+                    const int8_t *values, const double *probs, int n_values, int max_tries, uint8_t *tape, int64_t tape_step_stride,
+                    int8_t *slab, uint8_t *flags, void *stream) {
+    if (const int rc = tg::check_demo_gen_box(S, N, R, nu, nv, nw, shift, n_values, max_tries, values, probs, tape, tape_step_stride, slab);
+        rc != tg::LAUNCH)
+        return rc;
+    if (!tg::alphabet_ok(values, probs, n_values, shift)) return TG_E_ARG;
+    const tg::Categorical cat = tg::categorical(values, probs, n_values, shift, seed);
+    const tg::BoxMasks box = tg::box_masks(S, nu, nv, nw, shift);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int rc = tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        if (n_values <= 3) return tg::launch_demo_box_sample<kS, 2>(first_demo, N, R, shift, cat, max_tries, box, tape, tape_step_stride, flags, st);
+        if (n_values <= 5) return tg::launch_demo_box_sample<kS, 4>(first_demo, N, R, shift, cat, max_tries, box, tape, tape_step_stride, flags, st);
+        return tg::launch_demo_box_sample<kS, 7>(first_demo, N, R, shift, cat, max_tries, box, tape, tape_step_stride, flags, st);
+    });
+    if (rc != TG_OK) return rc;
+    return tg::accumulate<true>(tape, tape_step_stride, N, R, S, shift, slab, flags, st);
 }
 
 } // extern "C"

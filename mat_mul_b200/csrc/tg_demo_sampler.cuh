@@ -220,6 +220,45 @@ __device__ __forceinline__ bool draw_triple(uint32_t words[(3 * S + 3) / 4], uin
            factor_nonzero<S, GF2>(words, 2, cat.zero_pat);
 }
 
+// ---- contract box v1: contract v1 at size S with the factors confined to a box (nu, nv, nw) (tg_demo_gen_box).  Per token
+// word of the action record (launch constants, uniform across threads): the bytes inside the box, the shift in every
+// byte outside it that is not tape padding, and the bytes of each factor inside the box.
+constexpr int BOX_WORDS = (3 * 25 + 3) / 4;
+struct BoxMasks {
+    uint32_t keep[BOX_WORDS];
+    uint32_t fill[BOX_WORDS];
+    uint32_t fac[3][BOX_WORDS];
+};
+
+inline BoxMasks box_masks(int S, int nu, int nv, int nw, int shift) {
+    BoxMasks b = {};
+    const int len[3] = {nu, nv, nw};
+    for (int q = 0; q < 3 * S; q++) {
+        const int f = q / S, w = q >> 2, sh = 8 * (q & 3);
+        if (q % S < len[f]) b.keep[w] |= 0xFFu << sh, b.fac[f][w] |= 0xFFu << sh;
+        else b.fill[w] |= ((uint32_t)shift & 0xFFu) << sh;
+    }
+    return b;
+}
+
+// try t of contract box v1: the whole v1 draw at size S, then every entry outside the box becomes the coefficient 0;
+// accepted iff u, v and w each have a non-zero (GF2: an odd) entry inside the box
+template <int S, int NTHR, bool GF2 = false>
+__device__ __forceinline__ bool draw_triple_box(uint32_t words[(3 * S + 3) / 4], uint32_t d_lo, uint32_t d_hi, int r, int t,
+                                                const Categorical &cat, const BoxMasks &box) {
+    draw_triple<S, NTHR, GF2>(words, d_lo, d_hi, r, t, cat);
+    uint32_t acc[3] = {0u, 0u, 0u};
+#pragma unroll
+    for (int w = 0; w < (3 * S + 3) / 4; w++) {
+        words[w] = (words[w] & box.keep[w]) | box.fill[w];
+        const uint32_t x = (words[w] ^ cat.zero_pat) & (GF2 ? ONES4 : 0xFFFFFFFFu);
+#pragma unroll
+        for (int f = 0; f < 3; f++)
+            if ((w + 1) * 4 > f * S && w * 4 < (f + 1) * S) acc[f] |= x & box.fac[f][w];
+    }
+    return acc[0] != 0 && acc[1] != 0 && acc[2] != 0;
+}
+
 // ---- host side
 // the alphabet rules of both generators: every probability >= 0 (NaN refused), a positive sum, values in [-shift, shift]
 inline bool alphabet_ok(const int8_t *values, const double *probs, int n, int shift) {

@@ -44,16 +44,18 @@ __device__ __forceinline__ uint32_t v_word(uint32_t v, uint32_t w, int c) {
     return V;
 }
 
-// NTHR = 0: contract v2 mod 2 (alias tables ap); NTHR > 0: contract v1 mod 2 with NTHR thresholds (cat, max_tries)
-template <int S, int NTHR>
+// NTHR = 0: contract v2 mod 2 (alias tables ap); NTHR > 0: contract v1 mod 2 with NTHR thresholds (cat, max_tries);
+// BOX: contract box v1 mod 2 (tg_demo_gen_box_gf2), v1 with the factors confined to the box
+template <int S, int NTHR, bool BOX = false>
 __global__ void __launch_bounds__(128) demo_gen_gf2_kernel(unsigned long long first_demo, long long N, int R, int shift,
                                                            const __grid_constant__ Categorical cat, int max_tries,
                                                            uint8_t *__restrict__ tape, long long tape_step_stride,
                                                            uint32_t *__restrict__ bits, uint8_t *__restrict__ flags,
-                                                           const __grid_constant__ AliasDev ap) {
+                                                           const __grid_constant__ AliasDev ap, const __grid_constant__ BoxMasks box) {
     using B = GeoB<S>;
     constexpr int G = DemoB<S>::G, RW = B::RW, GW = B::GB / 4, TW = B::TP / 4, NW = (3 * S + 3) / 4;
     constexpr bool ALIAS = NTHR == 0;
+    static_assert(!BOX || !ALIAS, "contract box v1 only");
     __shared__ __align__(16) uint32_t s_alias[ALIAS ? AliasGeo<S>::TAB_WORDS : 4];
     __shared__ __align__(16) uint4 s_stage[B::STAGED ? 4 * 32 * (GW / 4) : 1];
     if constexpr (ALIAS) {
@@ -80,7 +82,11 @@ __global__ void __launch_bounds__(128) demo_gen_gf2_kernel(unsigned long long fi
         } else {
 #pragma unroll 1
             for (int t = 0;; t++) {
-                if (draw_triple<S, NTHR, true>(words, d_lo, d_hi, r, t, cat)) break;
+                if constexpr (BOX) {
+                    if (draw_triple_box<S, NTHR, true>(words, d_lo, d_hi, r, t, cat, box)) break;
+                } else {
+                    if (draw_triple<S, NTHR, true>(words, d_lo, d_hi, r, t, cat)) break;
+                }
                 if (t + 1 >= max_tries) { // forced: u = v = w = x e_0, x the last odd value (cat.top_tok is its token)
 #pragma unroll
                     for (int w = 0; w < NW; w++) words[w] = 0;
@@ -157,12 +163,27 @@ __global__ void __launch_bounds__(128) demo_gen_gf2_kernel(unsigned long long fi
     }
 }
 
-template <int S, int NTHR>
+// contract v1 mod 2's launch constants: a factor is "zero" when every entry is even, and the forced triple is the last odd
+// value's.  false for an alphabet the generator refuses (alphabet_ok, or no odd value: no factor could be odd)
+inline bool categorical_gf2(const int8_t *values, const double *probs, int n, int shift, uint64_t seed, Categorical &cat) {
+    if (!alphabet_ok(values, probs, n, shift)) return false;
+    int odd = -1;
+    for (int i = 0; i < n; i++)
+        if (values[i] & 1) odd = i;
+    if (odd < 0) return false;
+    cat = categorical(values, probs, n, shift, seed);
+    cat.zero_pat = (uint32_t)shift * ONES4;
+    cat.top_tok = (uint32_t)(values[odd] + shift) & 0xFFu;
+    return true;
+}
+
+template <int S, int NTHR, bool BOX = false>
 int launch_demo_gen_gf2(unsigned long long first, long long N, int R, int shift, const Categorical &cat, int max_tries, const AliasDev &ap,
-                        uint8_t *tape, long long stride, uint32_t *bits, uint8_t *flags, cudaStream_t st) {
+                        const BoxMasks &box, uint8_t *tape, long long stride, uint32_t *bits, uint8_t *flags, cudaStream_t st) {
     const long long grid = (N + DemoB<S>::DPC - 1) / DemoB<S>::DPC;
     if (grid > 0x7FFFFFFFLL) return TG_E_ARG;
-    demo_gen_gf2_kernel<S, NTHR><<<(unsigned)grid, DemoB<S>::NT, 0, st>>>(first, N, R, shift, cat, max_tries, tape, stride, bits, flags, ap);
+    demo_gen_gf2_kernel<S, NTHR, BOX><<<(unsigned)grid, DemoB<S>::NT, 0, st>>>(first, N, R, shift, cat, max_tries, tape, stride, bits, flags,
+                                                                              ap, box);
     TG_CUDA(cudaGetLastError());
     return TG_OK;
 }
@@ -177,14 +198,9 @@ int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S,
                     uint32_t *bits, uint8_t *flags, void *stream) {
     if (const int rc = tg::check_demo_gen(S, N, R, shift, n_values, max_tries, values, probs, tape, tape_step_stride, bits); rc != tg::LAUNCH)
         return rc;
-    if (!tg::alphabet_ok(values, probs, n_values, shift)) return TG_E_ARG;
-    int odd = -1; // the last odd value: the forced triple of contract v1
-    for (int i = 0; i < n_values; i++)
-        if (values[i] & 1) odd = i;
-    if (odd < 0) return TG_E_ARG; // no factor can be odd
-    tg::Categorical cat = tg::categorical(values, probs, n_values, shift, seed);
-    cat.zero_pat = (uint32_t)shift * tg::ONES4;
-    cat.top_tok = (uint32_t)(values[odd] + shift) & 0xFFu;
+    tg::Categorical cat;
+    if (!tg::categorical_gf2(values, probs, n_values, shift, seed, cat)) return TG_E_ARG;
+    static const tg::BoxMasks no_box = {};
     cudaStream_t st = (cudaStream_t)stream;
     tg::AliasDev dev = {};
     const bool alias = tg::alias_applies<true>(values, probs, n_values, S);
@@ -199,11 +215,33 @@ int tg_demo_gen_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S,
     return tg::with_S(S, [&](auto s) {
         constexpr int kS = decltype(s)::value;
         auto go = [&](auto nthr) {
-            return tg::launch_demo_gen_gf2<kS, decltype(nthr)::value>(first_demo, N, R, shift, cat, max_tries, dev, tape,
+            return tg::launch_demo_gen_gf2<kS, decltype(nthr)::value>(first_demo, N, R, shift, cat, max_tries, dev, no_box, tape,
                                                                       tape_step_stride, bits, flags, st);
         };
         if constexpr (kS != 25) // contract v2 needs at most six groups per factor
             if (alias) return go(std::integral_constant<int, 0>{});
+        if (n_values <= 3) return go(std::integral_constant<int, 2>{});
+        if (n_values <= 5) return go(std::integral_constant<int, 4>{});
+        return go(std::integral_constant<int, 7>{});
+    });
+}
+
+int tg_demo_gen_box_gf2(uint64_t seed, uint64_t first_demo, int64_t N, int R, int S, int nu, int nv, int nw, int shift,
+                        const int8_t *values, const double *probs, int n_values, int max_tries, uint8_t *tape,
+                        int64_t tape_step_stride, uint32_t *bits, uint8_t *flags, void *stream) {
+    if (const int rc = tg::check_demo_gen_box(S, N, R, nu, nv, nw, shift, n_values, max_tries, values, probs, tape, tape_step_stride, bits);
+        rc != tg::LAUNCH)
+        return rc;
+    tg::Categorical cat;
+    if (!tg::categorical_gf2(values, probs, n_values, shift, seed, cat)) return TG_E_ARG;
+    const tg::BoxMasks box = tg::box_masks(S, nu, nv, nw, shift);
+    static const tg::AliasDev no_alias = {};
+    return tg::with_S(S, [&](auto s) {
+        constexpr int kS = decltype(s)::value;
+        auto go = [&](auto nthr) {
+            return tg::launch_demo_gen_gf2<kS, decltype(nthr)::value, true>(first_demo, N, R, shift, cat, max_tries, no_alias, box, tape,
+                                                                            tape_step_stride, bits, flags, (cudaStream_t)stream);
+        };
         if (n_values <= 3) return go(std::integral_constant<int, 2>{});
         if (n_values <= 5) return go(std::integral_constant<int, 4>{});
         return go(std::integral_constant<int, 7>{});

@@ -389,6 +389,137 @@ def make_synthetic_demos_gf2(n_demos: int, max_actions: int, S: int, values=(-1,
     return tape, bits, flags
 
 
+# ---------------------------------------------------------------- rectangular products <n, m, p>
+_SIZES = (4, 9, 16, 25)
+
+
+def matmul_box(n: int, m: int, p: int) -> tuple[int, tuple[int, int, int]]:
+    """<n, m, p> (A n x m, B m x p, C n x p) is a tensor of shape box = (n m, m p, n p).  Returns (S, box): the smallest
+    game size S in {4, 9, 16, 25} that holds every mode of the box.  Raises for a box with a mode beyond 25."""
+    if min(n, m, p) < 1:
+        raise TensorGameError(f"<{n}, {m}, {p}>: sizes must be >= 1")
+    box = (n * m, m * p, n * p)
+    for S in _SIZES:
+        if max(box) <= S:
+            return S, box
+    raise TensorGameError(f"<{n}, {m}, {p}>: its box {box} does not fit the largest game size 25")
+
+
+def matmul_tensor(n: int, m: int, p: int, S: int | None = None) -> torch.Tensor:
+    """The matrix multiplication tensor of <n, m, p> zero-padded to (S, S, S), int8 on the host (S defaults to
+    matmul_box's): T[i m + j][j p + k][i p + k] = 1 for i < n, j < m, k < p, the reference's convention with the C index
+    not transposed.  At n = m = p it is utils.build_matmul_tensor(1, n, n, n)[0].  pack_states, pack_states16 and
+    pack_gf2 turn it into any slab format; its float() is a start_tensor for TensorGameDataset.  Every factorization of
+    the padded tensor, truncated to the box (project_to_box), is one of <n, m, p> with at most as many non-null terms."""
+    S0, box = matmul_box(n, m, p)
+    S = S0 if S is None else S
+    if S not in _SIZES or S < S0:
+        raise TensorGameError(f"<{n}, {m}, {p}> needs S in {tuple(s for s in _SIZES if s >= S0)}, got {S}")
+    T = torch.zeros((S, S, S), dtype=torch.int8)
+    i, j, k = torch.meshgrid(torch.arange(n), torch.arange(m), torch.arange(p), indexing="ij")
+    T[i * m + j, j * p + k, i * p + k] = 1
+    return T
+
+
+def _box_args(S: int, box) -> tuple[int, int, int]:
+    nu, nv, nw = (int(x) for x in box)
+    if not all(1 <= x <= S for x in (nu, nv, nw)):
+        raise TensorGameError(f"box {tuple(box)} must lie in [1, {S}]^3")
+    return nu, nv, nw
+
+
+def make_synthetic_demos_box(n_demos: int, max_actions: int, S: int, box, values=(-1, 0, 1), probs=(0.15, 0.7, 0.15),
+                             shift: int = 1, seed: int = 0, first_demo: int = 0, device="cuda", max_tries: int = 64,
+                             tape: torch.Tensor | None = None, slab: torch.Tensor | None = None):
+    """make_synthetic_demos with every factor confined to box = (nu, nv, nw) (tg_demo_gen_box, contract box v1): the
+    demonstrations of a rectangular product played at size S (matmul_box).  Every entry of u beyond nu, of v beyond nv and
+    of w beyond nw is 0, and each factor has a non-zero entry inside the box.  With the full box (S, S, S) it is contract
+    v1 at S.  The targets are what accumulate_demos writes for the tape; beyond int8 re-sum with accumulate_demos16.
+
+    Returns (tape uint8 (R, N, TP) step-major, slab int8 (N, GP), flags uint8 (N,): FLAG_EXHAUSTED | FLAG_RANGE).  tape
+    and slab may be views into larger stores (several shapes in one S = 25 store: one call per shape into slices, with
+    disjoint first_demo ranges)."""
+    lay = layout(S)
+    nu, nv, nw = _box_args(S, box)
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise TensorGameError("make_synthetic_demos_box needs a CUDA device (there is no CPU path)")
+    v, p = _cat_arrays(values, probs)
+    if tape is None:
+        tape = torch.empty((max_actions, n_demos, lay.token_pitch), dtype=torch.uint8, device=dev)
+    if slab is None:
+        slab = torch.empty((n_demos, lay.game_pitch), dtype=torch.int8, device=dev)
+    flags = torch.empty(n_demos, dtype=torch.uint8, device=dev)
+    stride = tape.stride(0) if max_actions > 1 else n_demos * lay.token_pitch
+    with torch.cuda.device(dev):
+        _call("tg_demo_gen_box", (tape, slab, flags), seed, first_demo, n_demos, max_actions, S, nu, nv, nw, shift, v.ctypes.data,
+              p.ctypes.data, len(v), max_tries, _p(tape), stride, _p(slab), _p(flags))
+    return tape, slab, flags
+
+
+def make_synthetic_demos_box_gf2(n_demos: int, max_actions: int, S: int, box, values=(-1, 0, 1), probs=(0.15, 0.7, 0.15),
+                                 shift: int = 1, seed: int = 0, first_demo: int = 0, device="cuda", max_tries: int = 64,
+                                 tape: torch.Tensor | None = None, bits: torch.Tensor | None = None):
+    """make_synthetic_demos_gf2 with every factor confined to box = (nu, nv, nw) (tg_demo_gen_box_gf2, contract box v1
+    mod 2: each factor has an odd entry inside the box).  Returns (tape uint8 (R, N, TP), bits int32 (N, GB/4), flags
+    uint8 (N,): FLAG_EXHAUSTED or 0)."""
+    lay, lb = layout(S), layout_gf2(S)
+    nu, nv, nw = _box_args(S, box)
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise TensorGameError("make_synthetic_demos_box_gf2 needs a CUDA device (there is no CPU path)")
+    v, p = _cat_arrays(values, probs)
+    if tape is None:
+        tape = torch.empty((max_actions, n_demos, lay.token_pitch), dtype=torch.uint8, device=dev)
+    if bits is None:
+        bits = torch.empty((n_demos, lb.game_words), dtype=torch.int32, device=dev)
+    flags = torch.empty(n_demos, dtype=torch.uint8, device=dev)
+    stride = tape.stride(0) if max_actions > 1 else n_demos * lay.token_pitch
+    with torch.cuda.device(dev):
+        _call("tg_demo_gen_box_gf2", (tape, bits, flags), seed, first_demo, n_demos, max_actions, S, nu, nv, nw, shift,
+              v.ctypes.data, p.ctypes.data, len(v), max_tries, _p(tape), stride, _p(bits), _p(flags))
+    return tape, bits, flags
+
+
+def box_bases(mats: torch.Tensor, box) -> torch.Tensor:
+    """Change-of-basis triples that keep the box: matrix f keeps its leading box[f] x box[f] block and is the identity
+    elsewhere, so entries outside the box stay zero and factors inside it stay inside.  mats int8 (N, 3, S, S)
+    (sample_unimodular, S <= 16) or GF(2) bit matrices int32 (N, 3, S) (sample_invertible_gf2; word r = row r, bit c =
+    entry (r, c)).  Both samplers draw M = L U (L unit lower, U upper triangular): the leading k x k block is L11 U11,
+    unimodular (invertible over GF(2)) and distributed as the sampler's own draw at size k, so the results are unimodular
+    (invertible) and their inverses are the block-diagonal inverses invert_bases(_gf2) return."""
+    bits = mats.dtype == torch.int32
+    S = mats.shape[-1]
+    m = mats.reshape((-1, 3, S) if bits else (-1, 3, S, S)).clone()
+    dev = mats.device
+    r = torch.arange(S, device=dev)
+    for f in range(3):
+        k = _box_args(S, box)[f]
+        if bits:
+            # rows < k keep their bits < k; rows >= k are unit rows
+            keep = torch.where(r < k, (1 << k) - 1, 0).to(torch.int32)
+            unit = torch.where(r < k, 0, torch.bitwise_left_shift(torch.ones_like(r), r)).to(torch.int32)
+            m[:, f] = (m[:, f] & keep) | unit
+        else:
+            inside = (r[:, None] < k) & (r[None, :] < k)
+            eye = torch.eye(S, dtype=torch.int8, device=dev)
+            m[:, f] = torch.where(inside, m[:, f], eye)
+    return m
+
+
+def project_to_box(tape: torch.Tensor, S: int, box, shift: int) -> torch.Tensor:
+    """The projection onto the box of every action of a tape (..., TP): tokens of u beyond box[0], of v beyond box[1]
+    and of w beyond box[2] become `shift` (the coefficient 0).  The projection is linear and fixes every tensor that is
+    zero outside the box, so a tape that sums to such a target still sums to it afterwards.  Returns a new tape."""
+    _need_cuda(tape, "tape", torch.uint8)
+    nu, nv, nw = _box_args(S, box)
+    e = torch.arange(S, device=tape.device)
+    out = torch.cat([(e >= n) for n in (nu, nv, nw)])
+    res = tape.clone()
+    res[..., : 3 * S][..., out] = shift
+    return res
+
+
 def accumulate_demos(tape: torch.Tensor, S: int, shift: int, slab: torch.Tensor | None = None):
     """slab[n] = sum_r rank1(tape[r, n]) (tg_demo_accumulate).  Returns (slab, flags)."""
     _need_cuda(tape, "tape", torch.uint8)
