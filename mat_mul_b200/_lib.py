@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import re
 import subprocess
 from pathlib import Path
 
@@ -62,8 +63,6 @@ def _stale() -> bool:
 
 
 def header_version() -> int:
-    import re
-
     return int(re.search(r"#define\s+TG_VERSION\s+(\d+)", HEADER.read_text()).group(1))
 
 
@@ -88,112 +87,58 @@ def build(force: bool = False, verbose: bool = False) -> Path:
 
 _lib = None
 
-_i8p = C.c_void_p
-_vp = C.c_void_p
+# ctypes of the header's scalar types; pointers are mapped in _ctype
+_SCALARS = {"int": C.c_int, "int64_t": C.c_int64, "uint64_t": C.c_uint64, "uint32_t": C.c_uint32, "double": C.c_double}
 
-_SIGNATURES = {
-    "tg_version": (C.c_int, []),
-    "tg_last_cuda_error": (C.c_int, []),
-    "tg_error_string": (C.c_char_p, [C.c_int]),
-    "tg_layout": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
-    "tg_pack_f32": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, _vp, _vp]),
-    "tg_expand_f32": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
-    "tg_pack_actions_i64": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp]),
-    "tg_unpack_actions_i64": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_expand_children": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_rollout": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_replay": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_demo_gen_philox": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
-                                     _vp, C.c_int64, _vp, _vp, _vp]),
-    "tg_demo_alias_tables": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
-    "tg_demo_accumulate": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
-    "tg_demo_accumulate_tc": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
-    "tg_demo_sample": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp,
-                                 _vp, _vp]),
-    "tg_demo_sample_dm": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int64, _vp,
-                                    _vp, _vp, _vp, _vp]),
-    "tg_tape_to_demo_major": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_slice_rank": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_state_key": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_change_of_basis": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_change_of_basis_i16": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_demo_accumulate_i16": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp]),
-    "tg_pack_f32_i16": (C.c_int, [_vp, C.c_int64, _vp, C.c_int64, C.c_int, _vp, _vp]),
-    "tg_expand_f32_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
-    "tg_step_i16": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_expand_children_i16": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_rollout_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_replay_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_state_key_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_slice_rank_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_layout_gf2": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
-    "tg_pack_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_pack_gf2_i16": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_unpack_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_step_gf2": (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_expand_children_gf2": (C.c_int, [_vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_rollout_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_replay_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp]),
-    "tg_state_key_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_slice_rank_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_change_of_basis_gf2": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_change_of_basis_factors_gf2": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, C.c_int64, C.c_int,
-                                                 C.c_int, _vp]),
-    "tg_sample_invertible_gf2": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),
-    "tg_invert_bases_gf2": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_demo_sample_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp, _vp,
-                                     _vp]),
-    "tg_expand_f32_gf2": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp]),
-    "tg_demo_gen_gf2": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
-                                  _vp, C.c_int64, _vp, _vp, _vp]),
-    "tg_demo_alias_tables_gf2": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp]),
-    "tg_demo_gen_box": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp,
-                                  C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp]),
-    "tg_demo_gen_box_gf2": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp,
-                                      _vp, C.c_int, C.c_int, _vp, C.c_int64, _vp, _vp, _vp]),
-    "tg_change_of_basis_factors": (C.c_int, [_vp, C.c_int64, C.c_int, _vp, C.c_int, _vp, C.c_int64, C.c_int, _vp, C.c_int64,
-                                             C.c_int, C.c_int, _vp]),
-    "tg_sample_unimodular": (C.c_int, [C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_double, _vp, _vp]),
-    "tg_invert_bases": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp]),
-    "tg_mt19937_fill_f64": (C.c_int, [C.c_uint32, C.c_int64, C.c_int64, _vp]),
-    "tg_mt19937_fill_f64_state": (C.c_int, [_vp, C.c_int, C.c_int64, C.c_int64, _vp]),
-    "tg_demo_from_ustream_workspace": (C.c_int64, [C.c_int64, C.c_int]),
-    "tg_demo_from_ustream": (C.c_int, [_vp, C.c_int64, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _vp, C.c_int64,
-                                       _vp, _vp, _vp, _vp, C.c_int64, _vp]),
-    "tg_host_ctx_create": (C.c_int, [C.POINTER(_vp), C.c_int, C.c_int, C.c_int64]),
-    "tg_host_ctx_destroy": (C.c_int, [_vp]),
-    "tg_step_host": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_rollout_host": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_demo_gen_host": (C.c_int, [_vp, C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
-                                   _vp, _vp, _vp]),
-    "tg_step_host_i16": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_rollout_host_i16": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_step_host_gf2": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_rollout_host_gf2": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int]),
-    "tg_demo_gen_host_gf2": (C.c_int, [_vp, C.c_uint64, C.c_uint64, C.c_int64, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_int,
-                                       _vp, _vp, _vp]),
-}
-if TUNING:  # sweep build only (declared under TG_TUNING in include/tensorgame.h)
-    _SIGNATURES["tg_tune_step_ctas_per_sm"] = (C.c_int, [C.c_int])
-    _SIGNATURES["tg_tune_step_variant"] = (C.c_int, [C.c_int])
+
+def _ctype(decl: str, ret: bool = False):
+    """The ctypes type of a C type as include/tensorgame.h writes it (a return type, or a parameter without its name).
+    Raises for a type it does not know: a guessed type would pass wrong arguments without any error."""
+    words = [w for w in decl.replace("*", " * ").split() if w != "const"]
+    stars, base = words.count("*"), " ".join(w for w in words if w != "*")
+    if not stars and base in _SCALARS:
+        return _SCALARS[base]
+    if (base, stars) == ("char", 1) and ret:
+        return C.c_char_p
+    if (base, stars) == ("int", 1):
+        return C.POINTER(C.c_int)
+    if (base, stars) == ("tg_host_ctx", 2):
+        return C.POINTER(C.c_void_p)
+    if stars and not ret:
+        return C.c_void_p
+    raise TensorGameError(f"{HEADER.name}: no ctypes type for {decl.strip()!r}")
+
+
+def _parse_prototypes(text: str) -> dict:
+    """name -> (restype, argtypes) of every tg_* function a C header declares; the TG_TUNING block counts only in the
+    sweep build, as there the library exports it."""
+    text = re.sub(r"/\*.*?\*/", " ", text, flags=re.S)
+    if not TUNING:
+        text = re.sub(r"#ifdef TG_TUNING.*?#endif", "", text, flags=re.S)
+    text = re.sub(r"^\s*#.*$", "", text, flags=re.M)
+    sigs = {}
+    for ret, name, params in re.findall(r"([^;{}()]*?)\b(tg_\w+)\s*\(([^()]*)\)\s*;", text):
+        params = [p.strip() for p in params.split(",")]
+        if params == ["void"]:
+            params = []
+        # every parameter is named in the header: the type is what precedes the name
+        sigs[name] = (_ctype(ret, ret=True), [_ctype(re.fullmatch(r"(.*?)\w+", p, flags=re.S).group(1)) for p in params])
+    return sigs
+
+
+_SIGNATURES = _parse_prototypes(HEADER.read_text())
 
 
 def exported_symbols() -> list[str]:
     """Every function include/tensorgame.h declares (used by the symbol test)."""
-    import re
-
-    text = HEADER.read_text()
-    if not TUNING:  # the sweep-only entry points exist in the -DTG_TUNING build alone
-        text = re.sub(r"#ifdef TG_TUNING.*?#endif", "", text, flags=re.S)
-    return sorted(set(re.findall(r"\b(tg_[a-z0-9_]+)\s*\(", text)))
+    return sorted(_SIGNATURES)
 
 
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
         if _stale():
-            # never load a library built from other sources: the ctypes signatures below describe THIS tree
+            # never load a library built from other sources: the ctypes signatures come from THIS tree's header
             try:
                 build()
             except (TensorGameError, FileNotFoundError) as e:

@@ -162,3 +162,18 @@ def test_python_surface_and_the_store(S):
     assert np.array_equal(st.cpu().numpy(), want.astype(np.float32))
     assert np.array_equal(sc.cpu().numpy().ravel(), np.asarray(wsc, dtype=np.float32).ravel())
     assert np.array_equal(ac.cpu().numpy(), wac) and np.array_equal(rw.cpu().numpy().ravel(), np.asarray(wrw, dtype=np.float32).ravel())
+
+
+@pytest.mark.parametrize("S", SIZES)
+def test_into_views_of_a_larger_store(S):
+    """Both mod-2 generators write a shard of demos through tape[:, a:b] / bits[a:b] views of a larger store: the same
+    bytes as a call on a store of their own, and nothing outside the shard."""
+    N, R, shift = 40, 6, 2
+    tp, gw = env.layout(S).token_pitch, env.layout_gf2(S).game_words
+    for gen, box in ((env.make_synthetic_demos_gf2, ()), (env.make_synthetic_demos_box_gf2, ((S, S - 2, 2),))):
+        want = gen(N, R, S, *box, V5, P5, shift, seed=S, first_demo=N, device=DEV)
+        wide = torch.zeros((R, 3 * N, tp), dtype=torch.uint8, device=DEV)
+        store = torch.zeros((3 * N, gw), dtype=torch.int32, device=DEV)
+        got = gen(N, R, S, *box, V5, P5, shift, seed=S, first_demo=N, device=DEV, tape=wide[:, N:2 * N], bits=store[N:2 * N])
+        assert torch.equal(wide[:, N:2 * N], want[0]) and torch.equal(store[N:2 * N], want[1]) and torch.equal(got[2], want[2])
+        assert not wide[:, :N].any() and not wide[:, 2 * N:].any() and not store[:N].any() and not store[2 * N:].any()
